@@ -7,6 +7,7 @@ input stage (mask / normalise, fused) -> SqueezeSegV2 -> softmax/argmax/mask hea
 
     python bench.py --gpus N --steps K --warmup W            # this implementation (CUDA, one rank per GPU)
     python bench.py --impl reference --steps K --warmup W    # CPU restatement of the reference graph (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + what the last timed step returned, as DIR/*.npy
 
 Prints ONE JSON line on rank 0.  `value` = whole-job frames/s with inputs resident in HBM; `e2e` = the same metric
 through the reference-facing call `model([lidar, mask])` with HOST (pinned) buffers, H2D + D2H inside the timed
@@ -251,6 +252,28 @@ def timed_steps(rk, step, steps, warmup):
   lat = [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)]
   clocks = sampler.stop() if rk.rank == 0 else None
   return rk.max_over_ranks(total_ms), lat, clocks
+
+
+DUMP_BYTES = 60 * 10 ** 6   # --dump-outputs writes at most this many bytes
+
+
+def dump_outputs(out_dir, res):
+  """--dump-outputs: writes what one forward returned (`res`: predictions [B,H,W] int32, probabilities [B,H,W,NC]
+  float32) as out_dir/<name>.npy.  The pixels are a fixed seeded sample (every pixel when they all fit in DUMP_BYTES),
+  the same for every build of the project, so that two builds can be compared file by file:
+    pixel_index.npy    float64 [n]     flat index of the pixel into [B,H,W], ascending
+    predictions.npy    float32 [n]     class label
+    probabilities.npy  float32 [n,NC]"""
+  import torch
+  preds = res["predictions"].reshape(-1)
+  probs = res["probabilities"].reshape(preds.numel(), -1)
+  n = min(preds.numel(), (DUMP_BYTES - 3 * 128) // (8 + 4 + 4 * probs.shape[1]))   # 128: .npy header
+  idx = np.sort(np.random.default_rng(0).choice(preds.numel(), n, replace=False))
+  sel = torch.from_numpy(idx).to(preds.device)
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+  np.save(os.path.join(out_dir, "predictions.npy"), preds[sel].cpu().numpy().astype(np.float32))
+  np.save(os.path.join(out_dir, "probabilities.npy"), probs[sel].cpu().numpy().astype(np.float32))
 
 
 def op_roofline(lib, model, mc, sub, pb, outs, peaks, step_ms, B, op_table_path=None, workload=""):
@@ -530,6 +553,8 @@ def run_ours(args):
   # ---- timed region: K steps, CUDA events on the launching stream, max over ranks ----
   total_ms, lat, clocks = timed_steps(rk, step, args.steps, args.warmup)
   value = world * B * args.steps / (total_ms / 1e3)
+  if args.dump_outputs and rank == 0:   # before the roofline pass below overwrites outs[0]
+    dump_outputs(args.dump_outputs, outs[(args.steps - 1) % 2])
 
   # ---- e2e: the reference-facing call with HOST buffers (pinned), H2D + forward + D2H of the predictions ----
   # host inputs in the reference's contract (normalised [B,H,W,6] float32 + bool mask), produced untimed by the
@@ -813,7 +838,13 @@ def main():
   ap.add_argument("--no-eval", action="store_true", help="skip the config-5 eval leg (sharded eval + NCCL all-reduce)")
   ap.add_argument("--eval-frames", type=int, default=1024, help="eval leg: synthetic val frames per rank")
   ap.add_argument("--ref-frames", type=int, default=2, help="--impl reference: frames per step (bounded sample)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write the predictions and probabilities of the last timed step (rank 0) to DIR/*.npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and (args.impl == "reference" or args.workload in PROJECTION_WORKLOADS):
+    ap.error("--dump-outputs is implemented for the network workloads of --impl ours")
   if args.workload in PROJECTION_WORKLOADS:
     run_projection(args)
   elif args.impl == "reference":
