@@ -294,6 +294,9 @@ int64_t pcls_net_workspace_bytes(const pcls_net* net);
  *   "fuse_head"  1 = softmax / argmax / mask in the epilogue of the final convolution (default), 0 = separate kernel
  *   "keep_tensors" (before finalize) 1 = no workspace reuse: every intermediate tensor of the last forward stays readable
  *                with pcls_net_read_tensor (per-layer parity tests); default 0 = liveness-planned arena
+ *   "fuse_skip"  (before finalize) 1 = a 1x1 convolution of the network input with no activation whose only reader adds it
+ *                as a skip after its ReLU (SqueezeSegV2's conv1_skip -> fire13 expand) is computed in that reader's epilogue
+ *                and never written (default; off with keep_tensors or conv_impl = 1), 0 = its own launch and tensor
  * planning switches of the tcgen05 path, process-wide, to be set BEFORE pcls_net_finalize (all default 1):
  *   "tc_halo" (one 130-pixel tile serves three horizontal taps), "tc_resident" (weights stay in smem), "tc_group"
  *   (pixel-group view for 16 / 32-channel inputs), "tc_tma_store" (TMA-store epilogue), "tc_res_tma" (residual blocks
@@ -304,6 +307,7 @@ int64_t pcls_net_workspace_bytes(const pcls_net* net);
  * launch-time switches (any time; cached CUDA graphs are dropped):
  *   "tc_rtma"  bit 0: compile-time specialised residual kernel (one TMA-loaded skip tensor, TMA store, ReLU / LeakyReLU),
  *              bit 1: specialised plain kernel (no residual, TMA store); default 3, 0 = the generic kernel everywhere
+ *              (a layer planned with a fused skip always runs its own specialised kernel)
  *   "cam_px"   pixels per thread of the CAM kernel: 0 = default (2), 1, 2
  * "tc_debug" (wait-cycle counters) needs a library built with PCLS_NVCC_FLAGS=-DPCLS_TC_DEBUG=1. */
 int pcls_net_set_option(pcls_net* net, const char* name, int value);

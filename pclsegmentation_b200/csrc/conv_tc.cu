@@ -112,6 +112,11 @@ struct TcParams {
   const void* res1;
   int res0_channels, res1_channels;
   const float* bias;
+  // skip computed in the epilogue (RM = 3): the skip tensor is a 1x1 conv (no activation) of the 8-channel network input
+  // (6 channels + 2 zero pads), map_r is that input.  skip_w = [64][8] 16-bit: the folded weights of channels 0-5, and
+  // the bias split in two 16-bit parts (hi, lo = bias - hi) in columns 6 and 7, which the kernel multiplies by 1
+  int skip;
+  const void* skip_w;
   // fused segmentation head (final conv only): softmax -> argmax -> mask; any of logits/probs may be NULL
   int head, none_index;
   const uint8_t* mask;
@@ -150,6 +155,38 @@ template <> __device__ __forceinline__ uint32_t add2_16<__nv_bfloat16>(uint32_t 
 #ifndef PCLS_TC_PACKED_SKIP
 #define PCLS_TC_PACKED_SKIP 1
 #endif
+
+// Skip computed in the epilogue (RM = 3): warp-level m16n8k8 MMAs (fp32 accumulation), the 16-bit results go through
+// stmatrix into the output staging buffer, where the packed skip add reads them like a TMA-loaded residual block.
+template <typename T> __device__ __forceinline__ uint32_t pack2_rn(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack2_rn<__half>(float lo, float hi) {
+  uint32_t d;
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+  return d;
+}
+template <> __device__ __forceinline__ uint32_t pack2_rn<__nv_bfloat16>(float lo, float hi) {
+  uint32_t d;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+  return d;
+}
+// d = a (16 x 8, row-major) * b (8 x 8, column-major), fp32 accumulators starting from zero
+template <typename T> __device__ __forceinline__ void mma_16x8x8(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t b);
+template <> __device__ __forceinline__ void mma_16x8x8<__half>(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t b) {
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5}, {%6}, {%7, %7, %7, %7};"
+               : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3]) : "r"(a0), "r"(a1), "r"(b), "f"(0.0f));
+}
+template <> __device__ __forceinline__ void mma_16x8x8<__nv_bfloat16>(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t b) {
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5}, {%6}, {%7, %7, %7, %7};"
+               : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3]) : "r"(a0), "r"(a1), "r"(b), "f"(0.0f));
+}
+__device__ __forceinline__ void ldmatrix_x4(uint32_t addr, uint32_t (&r)[4]) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr) : "memory");
+}
+__device__ __forceinline__ void stmatrix_x4(uint32_t addr, uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
+  asm volatile("stmatrix.sync.aligned.m8n8.x4.shared.b16 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(r0), "r"(r1), "r"(r2), "r"(r3)
+               : "memory");
+}
 
 // 8 accumulator columns (the bias is already in them: the epilogue pre-loads every TMEM accumulator with the bias row
 // before its MMAs run, see preload_bias) -> activation, +residuals -> one 16-byte vector of 16-bit outputs.
@@ -245,6 +282,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   constexpr int TC_NG = tc_ng(RES);
   constexpr bool RTMA = RES && RM == 1;
   constexpr bool PTMA = !RES && RM == 2;   // no residual, 16-bit outputs through the TMA-store epilogue (known at compile time)
+  // RM = 3: as RM = 1, but the skip is computed from the network input (TcParams::skip) instead of loaded, G = 4, ReLU
+  constexpr bool SKIP = RES && RM == 3;
+  static_assert(!SKIP || (G == 4 && !LEAKY), "the computed skip exists for the pixel-group view G = 4 with ReLU");
+  constexpr bool FIXED = RTMA || SKIP;      // one skip tensor, TMA-store epilogue, known at compile time
   extern __shared__ uint8_t smem_raw[];
   // carve: [stages x (A tile | B tiles)] 1024-aligned, resident weights, barriers, TMEM base slot, bias
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -256,13 +297,15 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   const uint32_t bres_base = smem_base + (uint32_t)S * stage_bytes;   // resident weights (1024-aligned)
   const uint32_t cstage_base = bres_base + (uint32_t)p.bres_bytes;  // output staging: [group][n_cbuf] x c_stage_bytes
   const uint32_t rstage_base = cstage_base + (p.tma_store ? (uint32_t)(p.n_cbuf * TC_NG) * (uint32_t)p.c_stage_bytes : 0u);  // residual0 staging (RES)
-  const uint32_t bar_base = rstage_base + ((RES && p.res_smem) ? (uint32_t)TC_NG * 16384u : 0u);
+  // (SKIP: the same space holds two 8 KB network-input tiles per group)
+  const uint32_t bar_base = rstage_base + ((RES && (SKIP || p.res_smem)) ? (uint32_t)TC_NG * 16384u : 0u);
 #define FULL_BAR(s) (bar_base + 8u * (uint32_t)(s))
 #define EMPTY_BAR(s) (bar_base + 8u * (uint32_t)(S + (s)))
 #define TFULL_BAR(a) (bar_base + 8u * (uint32_t)(2 * S + (a)))
 #define TEMPTY_BAR(a) (bar_base + 8u * (uint32_t)(2 * S + 8 + (a)))
 #define BRES_BAR (bar_base + 8u * (uint32_t)(2 * S + 16))
 #define RFULL_BAR(i) (bar_base + 8u * (uint32_t)(2 * S + 17 + (i)))   // [group][3]: residual block landed in staging buffer
+                                                                       // (SKIP: [group][2] network-input tile landed)
   const uint32_t tmem_slot = bar_base + 8u * (uint32_t)(2 * S + 17 + 3 * TC_NG);
   volatile uint32_t* tmem_slot_ptr =
       reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - smem_u32(smem_raw)));
@@ -282,7 +325,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b) : "memory");
     if (p.n1 > 0) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b2) : "memory");
     if (p.tma_store) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c) : "memory");
-    if (RES && p.res_tma) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_r) : "memory");
+    if (RES && (SKIP || p.res_tma)) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_r) : "memory");
     for (int i = 0; i < 3 * TC_NG; ++i) mbar_init(RFULL_BAR(i), 1);
     for (int s = 0; s < S; ++s) { mbar_init(FULL_BAR(s), 1); mbar_init(EMPTY_BAR(s), 1); }
     for (int a = 0; a < 8; ++a) { mbar_init(TFULL_BAR(a), 1); mbar_init(TEMPTY_BAR(a), 4); }
@@ -532,12 +575,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const int blk_shift = p.cout_blk_shift;              // pixel-group view: column n -> pixel n >> blk_shift
     const int blk_mask = G > 1 ? (1 << blk_shift) - 1 : -1;
     const float slope = p.act == PCLS_ACT_RELU ? 0.0f : (p.act == PCLS_ACT_LEAKY ? 0.1f : 1.0f);   // (float32 logits path)
-    const float act_lo = (RTMA || p.act == PCLS_ACT_RELU) ? 0.0f : -INFINITY;
+    const float act_lo = (FIXED || p.act == PCLS_ACT_RELU) ? 0.0f : -INFINITY;
     const uint16_t* res0 = reinterpret_cast<const uint16_t*>(p.res0);
     const uint16_t* res1 = reinterpret_cast<const uint16_t*>(p.res1);
     const int res0_channels = p.res0_channels, res1_channels = p.res1_channels;
-    const bool has_r0 = RTMA || res0 != nullptr, has_r1 = !RTMA && res1 != nullptr;
-    const bool tma_store = RTMA || PTMA || p.tma_store != 0, out_f32 = !RTMA && !PTMA && p.out_f32 != 0, c_is_5d = p.c_is_5d != 0;
+    const bool has_r0 = FIXED || res0 != nullptr, has_r1 = !FIXED && res1 != nullptr;
+    const bool tma_store = FIXED || PTMA || p.tma_store != 0, out_f32 = !FIXED && !PTMA && p.out_f32 != 0, c_is_5d = p.c_is_5d != 0;
     const uint32_t c_stage_bytes = (uint32_t)p.c_stage_bytes;
     T* const outp = reinterpret_cast<T*>(p.out);
     const bool issuer = (q == 2) && lane == 0;            // first warp of the group (warp 2 or 6) issues the TMA stores
@@ -577,8 +620,53 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       const int uwt = unit % n_wt, hseg = (unit / n_wt) % vs_hseg, ub = unit / (n_wt * vs_hseg);
       return (ub * n_ht + hseg * vs_R + i) * n_wt + uwt;   // n_nt = n_phase = 1 in this mode
     };
-    if (RES && p.res_tma != 0 && has_r0 && issuer && (uint32_t)grp < ng && tile_at((uint32_t)grp) >= 0)
+    if (RES && !SKIP && p.res_tma != 0 && has_r0 && issuer && (uint32_t)grp < ng && tile_at((uint32_t)grp) >= 0)
       issue_res(tile_at((uint32_t)grp), 0, 0u);
+    // ---- SKIP: skip = 1x1 conv (6 -> 64, folded BN, no activation) of the 8-channel network input, computed here ----
+    // A tile is 512 consecutive pixels of one image row, i.e. 8 KB of the input: ONE TMA load of 128 rows x 64 bytes (four
+    // pixels per row, SWIZZLE_64B) per tile, a tile ahead, into one of two buffers per group.  For the 64-channel block of
+    // pixel pp the warp's 32 rows m take pixel 4m + pp: two 16-row MMA tiles x eight 8-channel N tiles of m16n8k8, A by
+    // ldmatrix (the 64-byte swizzle puts the 8 rows of a matrix in distinct banks), B = the weights in registers, C = the
+    // bias; the results are rounded to 16 bits and written by stmatrix into the swizzled staging rows that the packed
+    // skip add reads.  Each warp reads back only its own 32 rows.
+    uint32_t skw[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    const uint32_t in_base = rstage_base + (uint32_t)grp * 16384u;   // [2] x 8 KB
+    // the bias rides in the MMA: lanes holding input channels 6 and 7 (the zero pads) put 1 there instead
+    const bool ones_lane = (lane & 3) == 3;
+    const uint32_t one2 = std::is_same<T, __half>::value ? 0x3C003C00u : 0x3F803F80u;
+    if constexpr (SKIP) {
+      const uint32_t* w32 = reinterpret_cast<const uint32_t*>(p.skip_w);   // [64][8] 16-bit: row n, channels 2 t, 2 t + 1
+#pragma unroll
+      for (int j = 0; j < 8; ++j) skw[j] = __ldg(w32 + (8 * j + (lane >> 2)) * 4 + (lane & 3));
+    }
+    auto issue_in = [&](int rtile, uint32_t bi) {
+      const int wt2 = (rtile / n_nt / n_phase) % n_wt;
+      const int ht2 = (rtile / n_nt / n_phase / n_wt) % n_ht;
+      const int b2 = rtile / n_nt / n_phase / n_wt / n_ht;
+      const uint32_t bar = RFULL_BAR(grp * 3 + (int)bi);
+      mbar_arrive_expect_tx(bar, 8192u);
+      tma_load_4d(in_base + bi * 8192u, &map_r, bar, 0, wt2 * BW, ht2 * BH, b2);
+    };
+    auto compute_skip = [&](uint32_t buf, int pp, uint32_t in_buf) {
+      uint32_t a[4];
+      ldmatrix_x4(in_buf + (uint32_t)(m * 64) + (uint32_t)((pp ^ ((m >> 1) & 3)) << 4), a);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) a[k] = ones_lane ? one2 : a[k];
+      const int sr = (q * 32 + ((lane >> 3) & 1) * 8 + (lane & 7));   // stmatrix row of this lane (M tile 0)
+#pragma unroll
+      for (int i = 0; i < 2; ++i)
+#pragma unroll
+        for (int jp = 0; jp < 4; ++jp) {
+          float d0[4], d1[4];
+          mma_16x8x8<T>(d0, a[2 * i], a[2 * i + 1], skw[2 * jp]);
+          mma_16x8x8<T>(d1, a[2 * i], a[2 * i + 1], skw[2 * jp + 1]);
+          const uint32_t chunk = (uint32_t)((2 * jp + (lane >> 4)) ^ (lane & 7));
+          stmatrix_x4(buf + (uint32_t)((sr + 16 * i) * 128) + (chunk << 4), pack2_rn<T>(d0[0], d0[1]), pack2_rn<T>(d0[2], d0[3]),
+                      pack2_rn<T>(d1[0], d1[1]), pack2_rn<T>(d1[2], d1[3]));
+        }
+      __syncwarp();
+    };
+    if (SKIP && issuer && (uint32_t)grp < ng && tile_at((uint32_t)grp) >= 0) issue_in(tile_at((uint32_t)grp), 0u);
     // Bias through the accumulator (kernels without residuals): before an accumulator's MMAs start, its rows are pre-loaded with the bias row of
     // the tile that will use it (tcgen05.st, 4x the TMEM read rate; every MMA then accumulates).  This takes the bias
     // add - one FADD per output element plus the shared-memory reads of the bias - out of the epilogue's inner loop.
@@ -644,8 +732,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       // The second residual (Darknet decoder only, compute-bound layers) is fetched one chunk ahead.
       const uint32_t rslot = rstage_base + (uint32_t)grp * 16384u + (uint32_t)(m & 127) * 16u;  // + i * 2048 per vector
       int4 r0[4], r1[4];
-      const bool res_smem = !RTMA && RES && p.res_smem != 0 && has_r0;
-      const bool res_tma = RTMA || (RES && p.res_tma != 0 && has_r0);
+      const bool res_smem = !FIXED && RES && p.res_smem != 0 && has_r0;
+      const bool res_tma = RTMA || (RES && !SKIP && p.res_tma != 0 && has_r0);
+      const bool res_stage = res_tma || SKIP;   // residual0 block sits in the output staging buffer (row res_row)
       uint32_t res_row = 0;     // res_tma: this thread's row of the staging buffer that holds the residual block
       auto prefetch_r0 = [&](int cs) {
         if constexpr (RES) {
@@ -665,14 +754,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           for (int g = 0; g < 4; ++g) {
             const int64_t o = has_r1 ? elem_off(n0 + c + g * 8, res1_channels) : (int64_t)-1;
             r1[g] = o >= 0 ? __ldg(reinterpret_cast<const int4*>(res1 + o)) : make_int4(0, 0, 0, 0);
-            if (has_r0 && !res_smem && !res_tma) {
+            if (has_r0 && !res_smem && !res_stage) {
               const int64_t o0 = elem_off(n0 + c + g * 8, res0_channels);
               r0[g] = o0 >= 0 ? __ldg(reinterpret_cast<const int4*>(res0 + o0)) : make_int4(0, 0, 0, 0);
             }
           }
         }
       };
-      const bool reg_res = RES && (has_r1 || (has_r0 && !res_smem && !res_tma));
+      const bool reg_res = RES && (has_r1 || (has_r0 && !res_smem && !res_stage));
       prefetch_r0(0);
       if (reg_res) load_r1(0);
       uint8_t head_mask = 1;                                       // fused head: the mask byte travels during the MMAs
@@ -690,7 +779,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         for (int g = 0; g < 4; ++g) {
           int4 r0v = make_int4(0, 0, 0, 0);
           if constexpr (RES) {
-            r0v = res_tma ? ld_shared_v4(res_row + (uint32_t)(((((cc & 63) >> 3) + g) ^ (m & 7)) << 4))
+            r0v = res_stage ? ld_shared_v4(res_row + (uint32_t)(((((cc & 63) >> 3) + g) ^ (m & 7)) << 4))
                 : res_smem ? ld_shared_v4(rslot + (uint32_t)(((cc & 63) >> 3) + g) * 2048u) : r0[g];
           }
           sink(g, epilogue_vec8<T, LEAKY, !PRELOAD>(v + g * 8, bias_s + n0 + cc + g * 8, act_lo, RES && has_r0, r0v, RES && has_r1, r1[g]));
@@ -851,6 +940,16 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           } else {
             // two staging buffers per group: block k is written while the TMA store of block k-1 drains the other one
             buf = cstage_base + (uint32_t)(grp * 2 + (int)(blk & 1u)) * c_stage_bytes;
+            if constexpr (SKIP) {
+              const uint32_t tg = tl / ng;   // this group's tile count: input buffer tg & 1
+              if (cb == 0) {
+                // the other input buffer was last read by the previous tile, before its last group barrier
+                if (issuer && tile_at(tl + ng) >= 0) issue_in(tile_at(tl + ng), (tg + 1u) & 1u);
+                DBG_T0; mbar_wait(RFULL_BAR(grp * 3 + (int)(tg & 1u)), (tg >> 1) & 1u); DBG_ADD(4);
+              }
+              // buffer blk & 1 was last read by the store of block k-2, finished before block k-1's group barrier
+              compute_skip(buf, cb >> 6, in_base + (tg & 1u) * 8192u);
+            }
           }
           // a 32-channel tail block (N tile = 64 k + 32, kernels without residuals): 64-byte rows, SWIZZLE_64B, map_c2
           const bool narrow = !RES && BN - cb < 64;
@@ -1047,6 +1146,8 @@ static TcKernelFn tc_rtma_kernel_for(int G) {
   return conv_tc_kernel<T, 64, 3, 1, true, LEAKY, 4, 1>;
 }
 static TcKernelFn tc_kernel_for(int KC, int SUB, int G, int is_bf16, int res, int leaky, int ks = 0, int rtma = 0) {
+  if (rtma == 3)   // the skip computed from the network input (Net::tc_skip_fusable)
+    return is_bf16 ? conv_tc_kernel<__nv_bfloat16, 64, 3, 4, true, false, 4, 3> : conv_tc_kernel<__half, 64, 3, 4, true, false, 4, 3>;
   if (rtma == 2 && !res) {
     if (is_bf16) return leaky ? tc_ptma_kernel_for<__nv_bfloat16, true>(KC, SUB, G, ks) : tc_ptma_kernel_for<__nv_bfloat16, false>(KC, SUB, G, ks);
     return leaky ? tc_ptma_kernel_for<__half, true>(KC, SUB, G, ks) : tc_ptma_kernel_for<__half, false>(KC, SUB, G, ks);
@@ -1119,6 +1220,37 @@ static bool tc_eligible(const ConvParams& p) {
   return true;
 }
 
+// Pixel-group view for narrow inputs (Cin = 16 / 32): TMA moves about one box row per ~8 cycles whatever its
+// width, so G adjacent pixels are viewed as ONE row of G*Cin channels (<= 128 bytes) and the MMAs are issued
+// banded (kernel comment).  Needs the whole tensor row to be contiguous (Cin == tensor channels).
+static int tc_group_size(const ConvParams& cp) {
+  if (tc_group_mode && tc_resident_mode && (cp.mode == MODE_1x1 || cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) &&
+      (cp.cin_pad == 16 || cp.cin_pad == 32) && cp.in_channels == cp.cin_pad && cp.cout == cp.cout_pad && !cp.out_f32 &&
+      cp.Wout == cp.Win) {
+    for (int g = 64 / cp.cin_pad; g >= 2; g /= 2)
+      if (cp.Win % g == 0 && cp.Win / g >= 128 && g * cp.cout_pad <= 256 && (cp.cout_pad & (cp.cout_pad - 1)) == 0) return g;
+  }
+  return 1;
+}
+
+// Skip fusion (Net::finalize): P = 1x1 conv of the network input (<= 6 channels, no activation, no residual) whose output
+// E adds as its only residual.  E computes P in its epilogue (RM = 3 kernel) when E is planned on the RM = 1 path with the
+// G = 4 pixel-group view: 3x3 stride 1, 16 -> 64 channels, ReLU, TMA-store epilogue with 64-channel blocks.  Decided here,
+// before the arena is planned (P's output is then never allocated); tc_plan_layer checks that the plan agrees.
+bool Net::tc_skip_fusable(const ConvLayer& P, const ConvLayer& E) const {
+  const ConvParams &pp = P.p, &e = E.p;
+  if (P.in != 0 || pp.mode != MODE_1x1 || pp.act != PCLS_ACT_NONE || P.res0 >= 0 || P.res1 >= 0 ||
+      pp.out_f32 || pp.out_coff != 0 || P.cin_logical > 6 || pp.cout != 64 || pp.out_channels != 64)
+    return false;
+  if (E.res0 != P.out || E.res1 >= 0 || E.in == P.out || E.pair_view || e.mode != MODE_3x3_S1 || e.act != PCLS_ACT_RELU ||
+      e.out_f32 || e.cout != 64 || e.res0_channels != 64)
+    return false;
+  if (!tc_eligible(e) || tc_group_size(e) != 4 || !tc_halo_mode || !tc_tma_store_mode || !tc_res_tma_mode || !tc_rtma_mode ||
+      (e.out_channels * 2) % 16 != 0)
+    return false;
+  return true;
+}
+
 int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
   const int max_smem = 227 * 1024;
     ConvParams& cp = L.pair_view ? L.ptc : L.p;
@@ -1136,16 +1268,8 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     q.ksteps = q.KC / 16;
     q.BN = cp.cout_pad <= 256 ? cp.cout_pad : 256;
     q.n_nt = cp.cout_pad / q.BN;
-    // Pixel-group view for narrow inputs (Cin = 16 / 32): TMA moves about one box row per ~8 cycles whatever its
-    // width, so G adjacent pixels are viewed as ONE row of G*Cin channels (<= 128 bytes) and the MMAs are issued
-    // banded (kernel comment).  Needs the whole tensor row to be contiguous (Cin == tensor channels).
-    int G = 1;
-    if (allow_group && tc_group_mode && tc_resident_mode && (cp.mode == MODE_1x1 || cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) &&
-        (cp.cin_pad == 16 || cp.cin_pad == 32) && cp.in_channels == cp.cin_pad && cp.cout == cp.cout_pad && !cp.out_f32 &&
-        cp.Wout == cp.Win) {
-      for (int g = 64 / cp.cin_pad; g >= 2; g /= 2)
-        if (cp.Win % g == 0 && cp.Win / g >= 128 && g * cp.cout_pad <= 256 && (cp.cout_pad & (cp.cout_pad - 1)) == 0) { G = g; break; }
-    }
+    const int G = allow_group ? tc_group_size(cp) : 1;
+    const bool skip = L.skip_src >= 0;   // residual0 computed from the network input (RM = 3 kernel)
     const int cin_blk = cp.cin_pad;
     q.G = G; q.cout_blk = G > 1 ? cp.cout_pad : (1 << 30);
     q.cout_blk_shift = 0;
@@ -1305,10 +1429,15 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     q.bres_bytes = q.b_resident ? (all_w + 1023) / 1024 * 1024 : 0;
     // residual0 of the memory-bound layers (resident weights) with the TMA-store epilogue: TMA-loaded into a third
     // staging buffer and added in place (no per-thread address arithmetic, a whole block of latency hiding)
-    q.res_tma = (tc_res_tma_mode && L.res0 >= 0 && q.tma_store && q.cbw == 64 && q.b_resident && (cp.res0_channels * 2) % 16 == 0) ? 1 : 0;
+    q.res_tma = (!skip && tc_res_tma_mode && L.res0 >= 0 && q.tma_store && q.cbw == 64 && q.b_resident && (cp.res0_channels * 2) % 16 == 0) ? 1 : 0;
     q.n_cbuf = (q.res_tma && !q.nsplit) ? 3 : 2;
-    q.res_smem = (!q.res_tma && L.res0 >= 0 && q.BN <= 128) ? 1 : 0;
-    const int cstage_total = (q.tma_store ? q.n_cbuf * TC_NG * q.c_stage_bytes : 0) + (q.res_smem ? TC_NG * 16384 : 0);
+    q.res_smem = (!skip && !q.res_tma && L.res0 >= 0 && q.BN <= 128) ? 1 : 0;
+    // (skip: two 8 KB network-input tiles per group in place of the third staging buffer)
+    const int cstage_total = (q.tma_store ? q.n_cbuf * TC_NG * q.c_stage_bytes : 0) + ((q.res_smem || skip) ? TC_NG * 16384 : 0);
+    if (skip && !(G == 4 && q.tma_store && q.cbw == 64 && q.b_resident && q.BN == 256 && q.BW == 128 && q.BH == 1)) {
+      set_error("tc plan: the layer that computes the fused skip is not planned on the G = 4 TMA-store path");
+      delete plan; return PCLS_ERR_STATE;
+    }
     if (G > 1 && !q.b_resident) { delete plan; *retry = true; return PCLS_OK; }
     const int stage_bytes = q.a_bytes + (q.b_resident ? 0 : q.sub * q.b_tile_bytes);
     int stages = (max_smem - 2048 - cp.cout_pad * 4 - q.bres_bytes - cstage_total - (cp.out_f32 ? 4 * TC_NG * 32 * 33 * 4 : 0)) / stage_bytes;
@@ -1427,6 +1556,33 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
       plan->map_c2 = plan->map_a;
     }
     plan->map_r = plan->map_c;
+    if (skip) {
+      // R: the network input viewed as rows of four pixels x 8 channels (64 bytes); a tile is 128 such rows.
+      // Skip weights [64][8]: channels 0-5 of the source conv, its bias split into hi + lo (= bias - hi) in 6 and 7.
+      const ConvLayer& P = convs[L.skip_src];
+      const uint64_t dims[4] = {32, (uint64_t)W / 4, Hh, F};
+      const uint64_t str[3] = {64, (uint64_t)W / 4 * 64, Hh * (uint64_t)W / 4 * 64};
+      const uint32_t box[4] = {32, (uint32_t)q.BW, 1, 1};
+      rc = make_map(&plan->map_r, bf16, tensor_ptr(P.in, frames_per_pass), 4, dims, str, box, 64);
+      if (rc) { delete plan; return rc; }
+      std::vector<float> ws(64 * 8, 0.0f);
+      for (int n = 0; n < 64; ++n) {
+        for (int ci = 0; ci < P.cin_logical; ++ci) ws[n * 8 + ci] = P.w_f32[(size_t)n * P.p.cin_pad + ci];
+        const float b = P.bias_f32[n];
+        const float hi = bf16 ? __bfloat162float(__float2bfloat16_rn(b)) : __half2float(__float2half_rn(b));
+        ws[n * 8 + 6] = hi; ws[n * 8 + 7] = b - hi;
+      }
+      std::vector<uint16_t> hw(ws.size());
+      for (size_t i = 0; i < ws.size(); ++i) {
+        if (bf16) { __nv_bfloat16 hv = __float2bfloat16_rn(ws[i]); memcpy(&hw[i], &hv, 2); }
+        else { __half hv = __float2half_rn(ws[i]); memcpy(&hw[i], &hv, 2); }
+      }
+      if (cudaMalloc(&plan->w_dev, hw.size() * 2) != cudaSuccess ||
+          cudaMemcpy(plan->w_dev, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice) != cudaSuccess) {
+        set_error("tc plan: upload of the skip weights failed"); delete plan; return PCLS_ERR_CUDA;
+      }
+      q.skip = 1; q.skip_w = plan->w_dev;
+    }
     if (q.res_tma) {  // R: the residual tensor, same view as C
       char* r_base = (char*)tensor_ptr(L.res0, frames_per_pass);
       const uint64_t Co = (uint64_t)cp.res0_channels, Wo = (uint64_t)cp.Wout;
@@ -1457,6 +1613,7 @@ int Net::tc_prepare() {
   bool& attr_set = attr_set_dev[dev & 63];
   for (auto& L : convs) {
     bool retry = false;
+    if (L.skip_into >= 0) continue;   // computed by the layer that reads it (no launch of its own)
     int rc = head_plan_layer(L);   // the logits layer has its own kernel (conv_head.cu); falls through when it does not qualify
     if (rc) return rc;
     if (L.hp) { L.tc_ok = true; continue; }
@@ -1487,6 +1644,7 @@ int Net::tc_prepare() {
               PCLS_CHECK_CUDA(cudaFuncSetAttribute(tc_kernel_for(kc, sub, g, bf, 0, lk, 0, 2), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
           }
       PCLS_CHECK_CUDA(cudaFuncSetAttribute(tc_kernel_for(64, 3, 1, bf, 0, 0, 3, 2), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+      PCLS_CHECK_CUDA(cudaFuncSetAttribute(tc_kernel_for(64, 3, 4, bf, 1, 0, 0, 3), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
     }
     attr_set = true;
   }
@@ -1517,11 +1675,12 @@ int Net::tc_launch(ConvLayer& L, const ConvParams& p, int nb, cudaStream_t s) {
   int grid = work < sm_count() ? work : sm_count();
   if (prm.nsplit) grid -= grid % prm.n_nt;   // every CTA sees one N tile only (tile % n_nt == blockIdx.x % n_nt)
   // one skip tensor, TMA-loaded into the staging buffers, TMA-store epilogue, ReLU: the specialised residual kernel
-  const int rtma = (tc_rtma_mode && prm.res_tma && prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 &&
+  const int rtma = prm.skip ? 3 : (tc_rtma_mode && prm.res_tma && prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 &&
                     (prm.act == PCLS_ACT_RELU || prm.act == PCLS_ACT_LEAKY) && !(PCLS_TC_VSTREAM && prm.vstream)) ? 1
                  : ((tc_rtma_mode & 2) && !prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 && !(PCLS_TC_VSTREAM && prm.vstream)) ? 2 : 0;
-  PCLS_CHECK_CUDA(launch_pdl(tc_kernel_for(prm.KC, prm.sub, prm.G, prm.is_bf16, (prm.res0 || prm.res1) ? 1 : 0, prm.act == PCLS_ACT_LEAKY ? 1 : 0, prm.ksteps, rtma),
-                             dim3(grid), dim3(tc_threads(prm.res0 || prm.res1)), plan->smem_bytes, s,
+  const bool res = prm.res0 || prm.res1 || prm.skip;
+  PCLS_CHECK_CUDA(launch_pdl(tc_kernel_for(prm.KC, prm.sub, prm.G, prm.is_bf16, res ? 1 : 0, prm.act == PCLS_ACT_LEAKY ? 1 : 0, prm.ksteps, rtma),
+                             dim3(grid), dim3(tc_threads(res)), plan->smem_bytes, s,
                              plan->map_a, plan->map_b, plan->map_c, plan->map_r, plan->map_b2, plan->map_c2, prm, num_tiles));
   return check_launch("conv_tc_kernel");
 }

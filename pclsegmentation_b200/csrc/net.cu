@@ -316,10 +316,12 @@ void Net::op_tensors(const OpRef& op, std::vector<int>& reads, std::vector<int>&
   reads.clear(); writes.clear();
   if (op.type == OP_CONV) {
     const ConvLayer& L = convs[op.index];
+    if (L.skip_into >= 0) return;   // computed by the conv that reads its output: neither reads nor writes
     reads.push_back(L.in);
     if (L.pool_src >= 0) reads.push_back(L.pool_src);   // (fused max-pool: the un-pooled tensor is what the kernel reads)
     if (L.up_squeeze >= 0) reads.push_back(convs[L.up_squeeze].in);   // (fused squeeze conv: its input is what the kernel reads)
-    if (L.res0 >= 0) reads.push_back(L.res0);
+    if (L.skip_src >= 0) reads.push_back(convs[L.skip_src].in);      // (fused skip: computed from the network input)
+    else if (L.res0 >= 0) reads.push_back(L.res0);
     if (L.res1 >= 0) reads.push_back(L.res1);
     writes.push_back(L.out);
   } else if (op.type == OP_POOL) {
@@ -387,6 +389,29 @@ int Net::finalize(int logits_tensor_, int num_classes_, int none_index_) {
       U.up_squeeze = ops[i].index;
       Q.fused_into_up = ops[i + 1].index;
     }
+  // skip fusion (conv_tc.cu, RM = 3): a 1x1 conv of the network input with no activation (SqueezeSegV2's conv1_skip) whose
+  // output has ONE reader, a conv that adds it as its residual after the ReLU (fire13's expand), is computed in that
+  // conv's epilogue from the 16 bytes per pixel of the input instead of crossing HBM twice at 128 bytes per pixel.  Not
+  // with keep_tensors (the skip tensor is then never written) nor with the CUDA-core path.
+  if (fuse_skip && !keep_tensors && conv_impl == 0)
+    for (int i = 0; i < n_ops; ++i) {
+      if (ops[i].type != OP_CONV) continue;
+      ConvLayer& P = convs[ops[i].index];
+      if (P.in != 0 || P.out == logits_tensor || P.fused_into_up >= 0) continue;
+      int reader = -1, n_use = 0;
+      std::vector<int> rd, wr;
+      for (int k = 0; k < n_ops; ++k) {
+        if (k == i) continue;
+        op_tensors(ops[k], rd, wr);
+        for (int r : rd) if (r == P.out) { ++n_use; reader = k; }
+        for (int w : wr) if (w == P.out) n_use += 2;   // a second writer (channel slices) rules it out
+      }
+      if (n_use != 1 || ops[reader].type != OP_CONV) continue;
+      ConvLayer& E = convs[ops[reader].index];
+      if (E.pool_src >= 0 || E.up_squeeze >= 0 || !tc_skip_fusable(P, E)) continue;
+      E.skip_src = ops[i].index;
+      P.skip_into = ops[reader].index;
+    }
   // liveness: first write .. last read (op order); the logits tensor lives to the end (head reads it)
   std::vector<int> reads, writes;
   for (auto& t : tensors) { t.first = -1; t.last = -1; }
@@ -446,8 +471,11 @@ int Net::finalize(int logits_tensor_, int num_classes_, int none_index_) {
         release(tensors[t].offset, tensor_frame_bytes(tensors[t]));
   }
   frame_bytes = align_up(peak, 1024);
-  for (size_t t = 0; t < tensors.size(); ++t)
-    PCLS_REQUIRE(t == 0 || tensors[t].first >= 0, "pcls_net_finalize: tensor %d is never written", (int)t);
+  for (size_t t = 0; t < tensors.size(); ++t) {
+    bool fused_skip = false;   // (the output of a conv computed by its reader is never materialised)
+    for (const auto& L : convs) fused_skip = fused_skip || (L.skip_into >= 0 && L.out == (int)t);
+    PCLS_REQUIRE(t == 0 || tensors[t].first >= 0 || fused_skip, "pcls_net_finalize: tensor %d is never written", (int)t);
+  }
 
   frames_per_pass = (micro_batch > 0 && micro_batch < max_batch) ? micro_batch : max_batch;
   PCLS_CHECK_CUDA(cudaMalloc(&arena, frame_bytes * (size_t)frames_per_pass));
@@ -521,9 +549,10 @@ int Net::run_pass(const float* lidar, int channels, const uint8_t* mask, bool ra
       ConvParams p = L.p;
       p.in = tensor_ptr(L.in, nb);
       p.out = (L.out == logits_tensor) ? (void*)logits_buf : tensor_ptr(L.out, nb);
-      p.res0 = L.res0 >= 0 ? tensor_ptr(L.res0, nb) : nullptr;
+      p.res0 = (L.res0 >= 0 && L.skip_src < 0) ? tensor_ptr(L.res0, nb) : nullptr;   // (fused skip: see TcParams::skip)
       p.res1 = L.res1 >= 0 ? tensor_ptr(L.res1, nb) : nullptr;
       if (conv_impl == 0 && L.fused_into_up >= 0) continue;   // computed by the transposed conv behind it
+      if (L.skip_into >= 0) continue;                          // computed in the epilogue of the conv that reads it
       if (conv_impl == 0 && L.up_squeeze >= 0) {
         const ConvLayer& Q = convs[L.up_squeeze];
         SqueezeUpconvParams su;
@@ -746,9 +775,19 @@ int Net::op_info(int i, char* name, int* family, int64_t* flops, int64_t* bytes)
         by += (int64_t)H * (tensors[L.pool_src].width - p.Win) * cin * 2;
         snprintf(buf, sizeof(buf), "pool+%s_%dx%d_w%d", mode, (int)cin, (int)cout, p.Wout);
       }
-      if (L.res0 >= 0) by += (int64_t)H * p.Wout * cout * 2;
+      if (L.skip_src >= 0) {   // the skip is computed from the network input: 16 bytes per pixel instead of the 64-channel tensor
+        const ConvLayer& P = convs[L.skip_src];
+        by += (int64_t)H * W * tensors[P.in].stride * 2 + (int64_t)P.cin_logical * P.cout_logical * 2;
+        fl += 2 * (int64_t)H * W * P.cin_logical * P.cout_logical;
+      } else if (L.res0 >= 0) {
+        by += (int64_t)H * p.Wout * cout * 2;
+      }
       if (L.res1 >= 0) by += (int64_t)H * p.Wout * cout * 2;
       fam = (conv_impl == 0 && L.tc_ok) ? 1 : 0;
+      if (L.skip_into >= 0) {                                 // runs inside the conv that reads its output
+        snprintf(buf, sizeof(buf), "%s_%dx%d_w%d(fused)", mode, (int)cin, (int)cout, p.Wout);
+        fl = 0; by = 0; fam = 0;
+      }
       if (conv_impl == 0 && L.fused_into_up >= 0) {          // runs inside the transposed conv behind it
         snprintf(buf, sizeof(buf), "%s_%dx%d_w%d(fused)", mode, (int)cin, (int)cout, p.Wout);
         fl = 0; by = 0; fam = 0;
@@ -783,6 +822,8 @@ int Net::op_info(int i, char* name, int* family, int64_t* flops, int64_t* bytes)
 int Net::read_tensor(int t, int B, float* out, cudaStream_t s) {
   PCLS_REQUIRE(finalized && t >= 0 && t < (int)tensors.size(), "pcls_net_read_tensor: bad tensor id %d", t);
   PCLS_REQUIRE(B >= 0 && B <= frames_per_pass, "pcls_net_read_tensor: B exceeds the frames of one pass");
+  PCLS_REQUIRE(t == 0 || tensors[t].first >= 0, "pcls_net_read_tensor: tensor %d is computed inside the conv that reads it "
+               "(set keep_tensors or fuse_skip = 0 before finalize)", t);
   const TensorInfo& ti = tensors[t];
   const int64_t n = (int64_t)B * H * ti.width * ti.channels;
   if (ti.logits) { PCLS_CHECK_CUDA(cudaMemcpyAsync(out, tensor_ptr(t, B), n * 4, cudaMemcpyDeviceToDevice, s)); return PCLS_OK; }
@@ -907,6 +948,7 @@ extern "C" int pcls_net_launches_per_forward(const pcls_net* net) {
   int launches = 1;
   for (const OpRef& op : n->ops) {
     if (op.type == OP_CONV && n->conv_impl == 0 && n->convs[op.index].fused_into_up >= 0) continue;
+    if (op.type == OP_CONV && n->convs[op.index].skip_into >= 0) continue;
     if (op.type == OP_POOL && n->conv_impl == 0 && n->pools[op.index].fused_conv >= 0) continue;
     ++launches;
   }
@@ -921,7 +963,13 @@ extern "C" int64_t pcls_net_workspace_bytes(const pcls_net* net) {
 extern "C" int pcls_net_set_option(pcls_net* net, const char* name, int value) {
   Net* n = reinterpret_cast<Net*>(net);
   PCLS_REQUIRE(n != nullptr && name != nullptr, "pcls_net_set_option: NULL argument");
-  if (!strcmp(name, "conv_impl")) { PCLS_REQUIRE(value == 0 || value == 1, "conv_impl must be 0 or 1"); n->conv_impl = value; return PCLS_OK; }
+  if (!strcmp(name, "conv_impl")) {
+    PCLS_REQUIRE(value == 0 || value == 1, "conv_impl must be 0 or 1");
+    bool skip_fused = false;   // (the fused skip tensor is never allocated: the CUDA-core path could not write it)
+    for (const auto& L : n->convs) skip_fused = skip_fused || L.skip_into >= 0;
+    PCLS_REQUIRE(value == 0 || !skip_fused, "conv_impl = 1 needs a net finalized with fuse_skip = 0 (or conv_impl = 1 set before)");
+    n->conv_impl = value; return PCLS_OK;
+  }
   if (!strcmp(name, "use_graph")) { n->use_graph = value != 0; if (!n->use_graph) n->drop_graphs(); return PCLS_OK; }
   if (!strcmp(name, "micro_batch")) {
     PCLS_REQUIRE(!n->finalized, "micro_batch must be set before pcls_net_finalize");
@@ -957,6 +1005,10 @@ extern "C" int pcls_net_set_option(pcls_net* net, const char* name, int value) {
   if (!strcmp(name, "fuse_pool")) {
     PCLS_REQUIRE(!n->finalized, "fuse_pool must be set before pcls_net_finalize");
     n->fuse_pool = value != 0; return PCLS_OK;
+  }
+  if (!strcmp(name, "fuse_skip")) {
+    PCLS_REQUIRE(!n->finalized, "fuse_skip must be set before pcls_net_finalize");
+    n->fuse_skip = value != 0; return PCLS_OK;
   }
   if (!strcmp(name, "fuse_head")) { n->fuse_head = value != 0; n->drop_graphs(); return PCLS_OK; }
   if (!strcmp(name, "tc_debug")) {  // per-role wait-cycle counters of conv_tc_kernel (development aid)

@@ -34,6 +34,8 @@ struct ConvLayer {
   int pool_src = -1, pool_pad_left = 0;   // >= 0: this 1x1 conv reads tensor pool_src through a fused 3x3/s2 max-pool
   int up_squeeze = -1;     // transposed conv: index of the squeeze 1x1 conv computed in front of it by the same kernel (squeeze_upconv.cu)
   int fused_into_up = -1;  // that squeeze conv: index of the transposed conv that runs it (no launch of its own)
+  int skip_src = -1;       // >= 0: residual0 is that conv's output, computed in this conv's epilogue from its input (conv_tc.cu, RM = 3)
+  int skip_into = -1;      // that conv: index of the conv that computes it (no launch, its output tensor is never allocated)
   // Pixel-pair view for the convolutions that read the 8-channel network input (tensor-core path only):
   // [B,H,W,8] is viewed as [B,H,W/2,16]; `ptc` / `w_tc` / `bias_tc` describe the equivalent convolution on pairs.
   bool pair_view = false;
@@ -78,6 +80,7 @@ struct Net {
   bool fuse_up = true;     // FireDeconv squeeze 1x1 + transposed conv as one kernel (squeeze_upconv.cu)
   bool fuse_pool = true;   // max-pool + the squeeze 1x1 conv that consumes it as one kernel (pool_conv.cu)
   bool fuse_head = true;   // run softmax/argmax/mask in the epilogue of the final convolution (tcgen05 path)
+  bool fuse_skip = true;   // a 1x1 conv of the network input whose only reader adds it as a skip: computed by that reader
   struct HeadArgs { int head = 0, none_index = 0; const uint8_t* mask = nullptr; float* probs = nullptr; int32_t* preds = nullptr; float* logits = nullptr; } head_args;
   int micro_batch = 0;
   int cam_px = 0;             // CAM pixels per thread: 0 = default (2), 1 = cam_kernel, 2 = cam2_kernel
@@ -123,6 +126,7 @@ struct Net {
   // tcgen05 implicit-GEMM path (conv_tc.cu)
   int tc_prepare();
   int tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry);
+  bool tc_skip_fusable(const ConvLayer& P, const ConvLayer& E) const;
   int tc_launch(ConvLayer& L, const ConvParams& p, int nb, cudaStream_t s);
   void tc_release();
   // logits layer + fused head (conv_head.cu)
