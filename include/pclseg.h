@@ -297,19 +297,13 @@ int64_t pcls_net_workspace_bytes(const pcls_net* net);
  *   "fuse_skip"  (before finalize) 1 = a 1x1 convolution of the network input with no activation whose only reader adds it
  *                as a skip after its ReLU (SqueezeSegV2's conv1_skip -> fire13 expand) is computed in that reader's epilogue
  *                and never written (default; off with keep_tensors or conv_impl = 1), 0 = its own launch and tensor
- * planning switches of the tcgen05 path, process-wide, to be set BEFORE pcls_net_finalize (all default 1):
- *   "tc_halo" (one 130-pixel tile serves three horizontal taps), "tc_resident" (weights stay in smem), "tc_group"
- *   (pixel-group view for 16 / 32-channel inputs), "tc_tma_store" (TMA-store epilogue), "tc_res_tma" (residual blocks
- *   TMA-loaded into the output staging buffers), "tc_split" (outer taps skip the expand1x1 half of merged Fire expands)
- *   "tc_nsplit" (N-split across CTAs with resident weight halves), "tc_head" (logits layer on its own kernel),
- *   "pad48" / "pair_s2" (before the first pcls_net_conv: 48-channel tensors stored with a 64-channel stride; 3x3 stride-2
- *   convolutions with 32 input channels on the pixel-pair view)
- * launch-time switches (any time; cached CUDA graphs are dropped):
- *   "tc_rtma"  bit 0: compile-time specialised residual kernel (one TMA-loaded skip tensor, TMA store, ReLU / LeakyReLU),
- *              bit 1: specialised plain kernel (no residual, TMA store); default 3, 0 = the generic kernel everywhere
- *              (a layer planned with a fused skip always runs its own specialised kernel)
- *   "cam_px"   pixels per thread of the CAM kernel: 0 = default (2), 1, 2
- * "tc_debug" (wait-cycle counters) needs a library built with PCLS_NVCC_FLAGS=-DPCLS_TC_DEBUG=1. */
+ *   "fuse_up"    (before finalize) 1 = each FireDeconv squeeze 1x1 runs inside the transposed convolution behind it
+ *                (default), 0 = two launches
+ *   "fuse_pool"  (before finalize) 1 = each 3x3 / stride-2 max-pool runs inside the 1x1 convolution that reads it
+ *                (default), 0 = its own launch and tensor
+ *   "tc_debug"   1 = per-role wait-cycle counters of the tcgen05 kernel, printed per convolution by pcls_net_profile_ops;
+ *                needs a library built with PCLS_NVCC_FLAGS=-DPCLS_TC_DEBUG=1
+ * Any other name fails with PCLS_ERR_INVALID. */
 int pcls_net_set_option(pcls_net* net, const char* name, int value);
 
 #ifdef __cplusplus

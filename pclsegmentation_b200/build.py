@@ -23,7 +23,7 @@ SOURCES = [("conv_tc.cu", k) for k in range(TC_PARTS)] + ["conv_head.cu", "net.c
            "projection.cu", "head.cu", "input_stage.cu", "confusion.cu", "validation.cu", "error.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr"]
-# development builds, e.g. PCLS_NVCC_FLAGS="-DPCLS_TC_DEBUG=1" (wait-cycle counters) or "-DPCLS_TC_VSTREAM=1"
+# development builds, e.g. PCLS_NVCC_FLAGS="-DPCLS_TC_DEBUG=1" (wait-cycle counters)
 NVCC_FLAGS += os.environ.get("PCLS_NVCC_FLAGS", "").split()
 
 

@@ -411,14 +411,12 @@ static HeadKernelFn head_kernel_for(int KC, int CS, int bf16) {
   return bf16 ? head_kernel_for_t<__nv_bfloat16>(KC, CS) : head_kernel_for_t<__half>(KC, CS);
 }
 
-int tc_head_mode = 1;   // A/B switch (pcls_net_set_option "tc_head" before finalize): 0 = the generic kernel runs the logits layer
-
 // Plans the logits layer for conv_head_kernel when its shape allows: 3x3 stride-1 conv from a tensor with 32 k channels
 // to <= 20 float32 logits, no residuals.  Returns PCLS_OK with L.hp == nullptr when the layer does not qualify.
 int Net::head_plan_layer(ConvLayer& L) {
   L.hp = nullptr;
   const ConvParams& cp = L.p;
-  if (!tc_head_mode || !cp.out_f32 || cp.mode != MODE_3x3_S1 || L.pair_view || L.res0 >= 0 || L.res1 >= 0) return PCLS_OK;
+  if (!cp.out_f32 || cp.mode != MODE_3x3_S1 || L.pair_view || L.res0 >= 0 || L.res1 >= 0) return PCLS_OK;
   if (cp.cin_pad % 32 != 0 || cp.cin_pad > cp.in_channels || cp.cout > 20 || cp.out_coff != 0 || cp.out_channels != cp.cout) return PCLS_OK;
   if (cp.Win != cp.Wout || cp.Wout < 64) return PCLS_OK;
   const bool bf16 = precision == PCLS_BF16;

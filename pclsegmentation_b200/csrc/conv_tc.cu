@@ -38,21 +38,12 @@ namespace pcls {
 // kernel parameters
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int TC_MAX_TAPS = 9;
-// Vertical streaming of input rows (see TcParams::vstream) is compiled out by default: measured -0.7 % on SqueezeSegV2
-// (the 3x3 layers it applies to are bound by the epilogue or by the tensor pipe's A-operand reads, not by TMA), and its
-// code in the issuer loop costs the tensor-bound Darknet layers instruction-cache room.  -DPCLS_TC_VSTREAM=1 enables it.
-#ifndef PCLS_TC_VSTREAM
-#define PCLS_TC_VSTREAM 0
-#endif
 // Epilogue warp-groups (4 warps each; tiles are dealt round-robin).  Kernels with residual adds need ~166 registers per
 // thread: two groups (320 threads).  Kernels without (bias pre-loaded, ReLU in the conversion) need ~125 and could run
-// three (448 threads, -DPCLS_TC_NG_NORES=3) - measured slower on SqueezeSegV2 (3.83 vs 3.71 ms): the third group's
-// staging buffers cost the layers with resident weights their pipeline stages.
-#ifndef PCLS_TC_NG_NORES
-#define PCLS_TC_NG_NORES 2
-#endif
-constexpr int tc_ng(bool res) { return res ? 2 : PCLS_TC_NG_NORES; }
-constexpr int tc_threads(bool res) { return 64 + 128 * tc_ng(res); }   // warp 0 TMA producer, warp 1 MMA issuer, then the groups
+// three (448 threads) - measured slower on SqueezeSegV2 (3.83 vs 3.71 ms): the third group's staging buffers cost the
+// layers with resident weights their pipeline stages.
+constexpr int TC_NG = 2;
+constexpr int TC_THREADS = 64 + 128 * TC_NG;   // warp 0 TMA producer, warp 1 MMA issuer, then the groups
 
 struct TcParams {
   int pdl_early;              // trigger the dependent grid at the start (common.cuh)
@@ -74,8 +65,6 @@ struct TcParams {
   int a_is_5d;
   int a_rows;                 // rows of the A box: 128, or 130 with the one-pixel halo on both sides
   int b_resident;             // 1: every weight tile of the layer is loaded into smem once per CTA
-  int ntaps_total;
-  int use_base_offset;
   // pipeline
   int stages, a_bytes, b_tile_bytes, bres_bytes;
   uint32_t idesc, desc_hi;    // instruction descriptor; high 32 bits of the smem matrix descriptors
@@ -100,10 +89,6 @@ struct TcParams {
   // weight / bias rows were permuted so that every N tile holds a slice of both halves of a merged Fire expand
   // (centre-tap-only channels first, split-N applies per tile); cblk_off[i] = output channel of 64-column block i.
   int nsplit, perm, cblk_off[8];
-  // vertical streaming (3x3 stride-1 layers with the halo tile and resident weights): a CTA walks R consecutive output
-  // rows of one 128-pixel column strip; every input row travels to smem ONCE per strip and serves the three output rows
-  // around it (R + 2 row loads per R tiles instead of 3 R).  R is chosen per launch (R = 1: plain tiles).
-  int vstream, R, n_hseg;
   uint32_t desc_hi_b, idesc_blk;
   // epilogue
   int cout, out_channels, out_coff, act, out_f32, is_bf16;
@@ -151,10 +136,6 @@ template <> __device__ __forceinline__ uint32_t add2_16<__nv_bfloat16>(uint32_t 
   asm("add.rn.bf16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
   return d;
 }
-
-#ifndef PCLS_TC_PACKED_SKIP
-#define PCLS_TC_PACKED_SKIP 1
-#endif
 
 // Skip computed in the epilogue (RM = 3): warp-level m16n8k8 MMAs (fp32 accumulation), the 16-bit results go through
 // stmatrix into the output staging buffer, where the packed skip add reads them like a TMA-loaded residual block.
@@ -212,7 +193,7 @@ __device__ __forceinline__ int4 epilogue_vec8(const uint32_t* acc, const float* 
       return o;
     }
   }
-  if constexpr (PCLS_TC_PACKED_SKIP && !LEAKY) {
+  if constexpr (!LEAKY) {
     // ReLU + ONE skip tensor (the FireDeconv expands of SqueezeSegV2: x = relu(bn(conv)) + skip): the activation value is
     // rounded to 16 bits by the converting ReLU and the skip is added with packed 16-bit adds - 8 + 4 + 4 instructions per
     // 8 outputs instead of 8 + 8 + 8 (unpack) + 8 + 4; one more 16-bit rounding than the float32 add.  ncu source view of
@@ -273,13 +254,12 @@ __device__ __forceinline__ int4 epilogue_vec8(const uint32_t* acc, const float* 
 // code of every residual mode (cp.async staging, per-chunk LDG, second residual) behind run-time flags that are tested per
 // 8 outputs; the epilogue's instruction chain is what bounds these layers (DESIGN.md section 6, step 22).
 template <typename T, int KC, int SUB, int G, bool RES, bool LEAKY, int KS = KC / 16, int RM = 0>
-__global__ void __launch_bounds__(tc_threads(RES), 1)
+__global__ void __launch_bounds__(TC_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                const __grid_constant__ CUtensorMap map_c, const __grid_constant__ CUtensorMap map_r,
                const __grid_constant__ CUtensorMap map_b2, const __grid_constant__ CUtensorMap map_c2,
                const __grid_constant__ TcParams p, const int num_tiles) {
   constexpr bool PRELOAD = !RES;   // bias pre-loaded into the TMEM accumulators (see preload_bias)
-  constexpr int TC_NG = tc_ng(RES);
   constexpr bool RTMA = RES && RM == 1;
   constexpr bool PTMA = !RES && RM == 2;   // no residual, 16-bit outputs through the TMA-store epilogue (known at compile time)
   // RM = 3: as RM = 1, but the skip is computed from the network input (TcParams::skip) instead of loaded, G = 4, ReLU
@@ -380,21 +360,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       const bool is5d = p.a_is_5d != 0;
       int stage = 0;
       uint32_t phase = 0;
-      if (PCLS_TC_VSTREAM && p.vstream) {
-        const int R = p.R, n_hseg = p.n_hseg, num_units = num_tiles / R;
-        for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
-          const int wt = unit % n_wt, hseg = (unit / n_wt) % n_hseg, b = unit / (n_wt * n_hseg);
-          const int ww = wt * BW - 1;
-          for (int hh = hseg * R - 1; hh <= hseg * R + R; ++hh)   // rows outside the image are zero-filled by TMA
-            for (int kc = 0; kc < kchunks; ++kc) {
-              { DBG_T0; mbar_wait(EMPTY_BAR(stage), phase ^ 1u); DBG_ADD(0); }
-              const uint32_t fb = FULL_BAR(stage);
-              mbar_arrive_expect_tx_elect(fb, a_tx_bytes);
-              tma_load_4d_elect(smem_base + (uint32_t)stage * stage_bytes, &map_a, fb, kc * KC, ww, hh, b);
-              if (++stage == S) { stage = 0; phase ^= 1u; }
-            }
-        }
-      } else
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         int r = tile;
         const int nt = r % n_nt; r /= n_nt;
@@ -447,23 +412,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       int stage = 0;
       uint32_t phase = 0, acc = 0, acc_phase = 0;
       if (b_resident) mbar_wait(BRES_BAR, 0u);
-      // vertical streaming: ring position of load (input row h - 1, K chunk 0) of the current output row h; loads are
-      // numbered in the producer's order, [0, vs_waited) have been waited for
-      const bool vs = PCLS_TC_VSTREAM && p.vstream != 0;
-      const int vs_R = vs ? p.R : 1;
-      const int my_tiles = vs ? ((num_tiles / vs_R - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x) * vs_R
-                              : (num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-      uint32_t vs_slot = 0, vs_phase = 0, vs_idx = 0, vs_waited = 0;
-      int vs_row = 0;
-      auto vs_release = [&](int n) {   // the n oldest loads are no longer needed once the MMAs issued so far have completed
-        for (int i = 0; i < n; ++i) {
-          umma_commit_elect(EMPTY_BAR(vs_slot));
-          if (++vs_slot == (uint32_t)S) { vs_slot = 0; vs_phase ^= 1u; }
-        }
-        vs_idx += (uint32_t)n;
-      };
+      const int my_tiles = (num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
       for (int seq = 0; seq < my_tiles; ++seq) {
-        const int tile = blockIdx.x + seq * gridDim.x;   // (only the transposed-conv phase below reads it; not vstream)
+        const int tile = blockIdx.x + seq * gridDim.x;   // (only the transposed-conv phase below reads it)
         { DBG_T0; mbar_wait(TEMPTY_BAR(acc), PRELOAD ? acc_phase : (acc_phase ^ 1u)); DBG_ADD(1); }  // the epilogue has drained this accumulator and pre-loaded the bias row
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * (uint32_t)BN;
@@ -471,19 +422,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         uint32_t accumulate = PRELOAD ? 1u : 0u, acc_lo = accumulate;   // PRELOAD: the accumulator starts from the bias row
         int kc_i = 0, g_i = 0;   // K chunk and A-load group of iteration k
         for (int k = 0; k < k_iters; ++k) {
-          uint32_t a_addr;
-          if (vs) {
-            uint32_t sl = vs_slot + (uint32_t)k, par = vs_phase;
-            if (sl >= (uint32_t)S) { sl -= (uint32_t)S; par ^= 1u; }
-            if (vs_idx + (uint32_t)k >= vs_waited) {
-              { DBG_T0; mbar_wait(FULL_BAR(sl), par); DBG_ADD(2); }
-              vs_waited = vs_idx + (uint32_t)k + 1u;
-            }
-            a_addr = smem_base + sl * stage_bytes;
-          } else {
-            { DBG_T0; mbar_wait(FULL_BAR(stage), phase); DBG_ADD(2); }
-            a_addr = smem_base + (uint32_t)stage * stage_bytes;
-          }
+          { DBG_T0; mbar_wait(FULL_BAR(stage), phase); DBG_ADD(2); }
+          const uint32_t a_addr = smem_base + (uint32_t)stage * stage_bytes;
           tc_fence_after();
           if constexpr (G == 1) {
             uint32_t b_addr = b_resident ? b_res : a_addr + a_bytes;
@@ -550,14 +490,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           }
           if constexpr (G > 1) b_res += (uint32_t)SUB * b_tile_bytes;
           if (++kc_i == kchunks) { kc_i = 0; ++g_i; }
-          if (!vs) {
-            umma_commit_elect(EMPTY_BAR(stage));  // smem slot free once these MMAs have read it
-            if (++stage == S) { stage = 0; phase ^= 1u; }
-          }
-        }
-        if (vs) {  // input row h - 1 is done; the last output row of the strip also retires rows h and h + 1
-          if (++vs_row == vs_R) { vs_row = 0; vs_release(3 * kchunks); }
-          else vs_release(kchunks);
+          umma_commit_elect(EMPTY_BAR(stage));  // smem slot free once these MMAs have read it
+          if (++stage == S) { stage = 0; phase ^= 1u; }
         }
         umma_commit_elect(TFULL_BAR(acc));  // accumulator complete
         if (++acc == n_acc) { acc = 0; acc_phase ^= 1u; }
@@ -606,19 +540,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       if (c_is_5d) tma_load_5d(dst, &map_r, bar, c02, G > 1 ? pp2 : ph2, wt2 * BW, ht2 * BH, b2);
       else tma_load_4d(dst, &map_r, bar, c02, wt2 * BW, ht2 * BH, b2);
     };
-    // the CTA's seq-th tile as a flat index of the plain (nt, phase, wt, ht, b) encoding, or -1 past the end
-    const bool vs = PCLS_TC_VSTREAM && p.vstream != 0;
-    const int vs_R = vs ? p.R : 1, vs_hseg = p.n_hseg;
+    // the CTA's seq-th tile as a flat index of the (nt, phase, wt, ht, b) encoding, or -1 past the end
     auto tile_at = [&](uint32_t seq) -> int {
-      if (!vs) {
-        const long long t = (long long)blockIdx.x + (long long)seq * gridDim.x;
-        return t < num_tiles ? (int)t : -1;
-      }
-      const int unit = (int)blockIdx.x + (int)(seq / (uint32_t)vs_R) * (int)gridDim.x;
-      if (unit >= num_tiles / vs_R) return -1;
-      const int i = (int)(seq % (uint32_t)vs_R);
-      const int uwt = unit % n_wt, hseg = (unit / n_wt) % vs_hseg, ub = unit / (n_wt * vs_hseg);
-      return (ub * n_ht + hseg * vs_R + i) * n_wt + uwt;   // n_nt = n_phase = 1 in this mode
+      const long long t = (long long)blockIdx.x + (long long)seq * gridDim.x;
+      return t < num_tiles ? (int)t : -1;
     };
     if (RES && !SKIP && p.res_tma != 0 && has_r0 && issuer && (uint32_t)grp < ng && tile_at((uint32_t)grp) >= 0)
       issue_res(tile_at((uint32_t)grp), 0, 0u);
@@ -1204,12 +1129,8 @@ int make_map(CUtensorMap* map, bool bf16, void* base, int rank, const uint64_t* 
   return PCLS_OK;
 }
 
-// A/B switches for measurement (pcls_net_set_option before finalize): halo reuse, resident weights, base offset
-int tc_rtma_mode = 3;   // A/B switch "tc_rtma"
-int tc_tma_store_mode = 1, tc_group_mode = 1, tc_res_tma_mode = 1, tc_split_mode = 1, tc_vstream_mode = 0, tc_nsplit_mode = 1;
 const int tc_debug_compiled = PCLS_TC_DEBUG;
 unsigned long long* tc_debug_buf = nullptr;  // [148][24] counters of the most recent launch when enabled
-int tc_halo_mode = 1, tc_resident_mode = 1, tc_base_offset_mode = 0;  // measured: UMMA swizzles on absolute smem address bits, a row-shifted start needs NO base offset
 
 // Which layers run on tensor cores: the input tensor must carry >= 16 real channels (the 6-channel network input
 // goes through the CUDA-core kernel), and a stride-2 conv needs an even input width (pair view).
@@ -1224,7 +1145,7 @@ static bool tc_eligible(const ConvParams& p) {
 // width, so G adjacent pixels are viewed as ONE row of G*Cin channels (<= 128 bytes) and the MMAs are issued
 // banded (kernel comment).  Needs the whole tensor row to be contiguous (Cin == tensor channels).
 static int tc_group_size(const ConvParams& cp) {
-  if (tc_group_mode && tc_resident_mode && (cp.mode == MODE_1x1 || cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) &&
+  if ((cp.mode == MODE_1x1 || cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) &&
       (cp.cin_pad == 16 || cp.cin_pad == 32) && cp.in_channels == cp.cin_pad && cp.cout == cp.cout_pad && !cp.out_f32 &&
       cp.Wout == cp.Win) {
     for (int g = 64 / cp.cin_pad; g >= 2; g /= 2)
@@ -1245,8 +1166,7 @@ bool Net::tc_skip_fusable(const ConvLayer& P, const ConvLayer& E) const {
   if (E.res0 != P.out || E.res1 >= 0 || E.in == P.out || E.pair_view || e.mode != MODE_3x3_S1 || e.act != PCLS_ACT_RELU ||
       e.out_f32 || e.cout != 64 || e.res0_channels != 64)
     return false;
-  if (!tc_eligible(e) || tc_group_size(e) != 4 || !tc_halo_mode || !tc_tma_store_mode || !tc_res_tma_mode || !tc_rtma_mode ||
-      (e.out_channels * 2) % 16 != 0)
+  if (!tc_eligible(e) || tc_group_size(e) != 4 || (e.out_channels * 2) % 16 != 0)
     return false;
   return true;
 }
@@ -1260,7 +1180,6 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     TcPlan* plan = new TcPlan();
     memset(plan, 0, sizeof(TcPlan));
     TcParams& q = plan->prm;
-    const int TC_NG = tc_ng(L.res0 >= 0 || L.res1 >= 0);   // epilogue groups of the kernel this layer will run
     const bool bf16 = precision == PCLS_BF16;
     // K chunk / swizzle: the widest of 64/32/16 channels that divides cin_pad
     q.KC = (cp.cin_pad % 64 == 0) ? 64 : (cp.cin_pad % 32 == 0) ? 32 : 16;
@@ -1280,7 +1199,7 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     // split-N: leading output channels whose kernel is zero outside the centre tap (the expand1x1 half of a merged Fire
     // expand layer).  Multiples of 16 channels on both sides (UMMA N granularity at M = 128).
     q.n1 = 0;
-    if (tc_split_mode && G == 1 && cp.mode == MODE_3x3_S1 && q.n_nt == 1 && !L.pair_view) {
+    if (G == 1 && cp.mode == MODE_3x3_S1 && q.n_nt == 1 && !L.pair_view) {
       int z = 0;
       for (; z < cp.cout_pad; ++z) {
         bool zero = true;
@@ -1294,11 +1213,8 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
       z = z / 16 * 16;
       if (z >= 16 && q.BN - z >= 16) q.n1 = z;
     }
-#ifndef PCLS_TC_KSKIP
-#define PCLS_TC_KSKIP 1
-#endif
     // zero-padded K tail (48 logical channels in a 64-channel chunk): the MMAs of the all-zero K steps are not issued
-    if (PCLS_TC_KSKIP && G == 1 && q.kchunks == 1 && q.n1 == 0) q.ksteps = std::min(q.KC / 16, (cp.cin + 15) / 16);
+    if (G == 1 && q.kchunks == 1 && q.n1 == 0) q.ksteps = std::min(q.KC / 16, (cp.cin + 15) / 16);
     // N-split across CTAs: a 3x3 layer whose weights do not fit in smem next to the pipeline (fire10's merged expand: 160 KB;
     // fire6 / fire7's 64(48) -> 192 expand3x3: 216 KB) streams them from L2 for every tile - 10 x the bytes of the A tile,
     // L2 -> smem bound (wait-cycle counters: issuer 50 % on FULL).  Cutting N in two and giving every CTA one half keeps the
@@ -1307,13 +1223,13 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     q.nsplit = 0; q.perm = 0;
     for (int i = 0; i < 8; ++i) q.cblk_off[i] = i * 64;
     std::vector<int> row_perm;   // new weight row -> old weight row, when permuted
-    if (tc_nsplit_mode && tc_resident_mode && tc_halo_mode && G == 1 && cp.mode == MODE_3x3_S1 && q.n_nt == 1 && !L.pair_view &&
+    if (G == 1 && cp.mode == MODE_3x3_S1 && q.n_nt == 1 && !L.pair_view &&
         q.KC == 64 && !cp.out_f32 && cp.cout == cp.cout_pad && cp.Wout >= 128 && L.res1 < 0) {
       const int btile1 = q.BN * q.KC * 2, bsmall1 = (q.BN - q.n1) * q.KC * 2;
       const int all_w1 = q.n1 > 0 ? q.kchunks * (btile1 + 8 * bsmall1) : 9 * q.kchunks * btile1;
       const int half = q.BN / 2;
       if (all_w1 > 112 * 1024) {
-        if (q.n1 > 0 && q.n1 % 128 == 0 && (q.BN - q.n1) % 128 == 0 && tc_tma_store_mode && (L.res0 < 0 || tc_res_tma_mode)) {
+        if (q.n1 > 0 && q.n1 % 128 == 0 && (q.BN - q.n1) % 128 == 0) {
           const int h1 = q.n1 / 2, h3 = (q.BN - q.n1) / 2;
           if (q.kchunks * ((h1 + h3) * q.KC * 2 + 8 * h3 * q.KC * 2) <= 112 * 1024) {
             row_perm.resize(q.BN);
@@ -1349,14 +1265,13 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     q.num_tiles = q.n_nt * q.n_phase * q.n_wt * q.n_ht;  // per frame
     // K walk
     q.a_is_5d = cp.mode == MODE_3x3_S2 ? 1 : 0;
-    q.sub = 1; q.a_rows = 128; q.ntaps_total = cp.ntaps;
-    q.use_base_offset = tc_base_offset_mode;
+    q.sub = 1; q.a_rows = 128;
     // halo reuse needs the three weight tiles of a row next to the A tile: only when >= 4 stages still fit
-    bool halo = (cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) && q.BW == 128 && tc_halo_mode;
+    bool halo = (cp.mode == MODE_3x3_S1 || cp.mode == MODE_ROW3) && q.BW == 128;
     if (halo) {
       const int btile_ = G > 1 ? cp.cout_pad * cin_blk * 2 : q.BN * q.KC * 2;
       const int all_w_ = q.n1 > 0 ? q.kchunks * (btile_ + (cp.ntaps - 1) * q.b_small_bytes) : cp.ntaps * q.kchunks * btile_;
-      const bool resident_ = tc_resident_mode && (q.n_nt == 1 || q.nsplit) && all_w_ <= 112 * 1024;
+      const bool resident_ = (q.n_nt == 1 || q.nsplit) && all_w_ <= 112 * 1024;
       const int st_ = (130 * q.KC * 2 + 1023) / 1024 * 1024 + (resident_ ? 0 : 3 * btile_);
       // (N-split layers hold half of a big weight set: they take two staging buffers per group instead of three)
       const int staging_ = 2 * TC_NG * 16384 + ((L.res0 >= 0 && (q.BN <= 128 || resident_) && !q.nsplit) ? TC_NG * 16384 : 0);
@@ -1409,7 +1324,7 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     // (N tile = 64 k + 32, e.g. the halves of fire6 / fire7's 192-channel expand3x3: the tail block is stored through a
     // second map with 64-byte rows - with per-thread stores that epilogue took 50 cycles per column instead of 24)
     const bool narrow_tail = q.BN % 64 == 32 && q.BN > 64 && G == 1 && !deconv && L.res0 < 0 && L.res1 < 0;
-    if (tc_tma_store_mode && !cp.out_f32 && cp.cout == cp.cout_pad && (q.BN % 64 == 0 || narrow_tail) &&
+    if (!cp.out_f32 && cp.cout == cp.cout_pad && (q.BN % 64 == 0 || narrow_tail) &&
         (G == 1 || cp.cout_pad % 64 == 0) &&
         (cp.out_channels * 2) % 16 == 0) {
       q.tma_store = 1;
@@ -1424,12 +1339,12 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     const int all_w = q.n1 > 0 ? q.kchunks * (q.b_tile_bytes + 8 * q.b_small_bytes)
                                : q.n_phase * q.n_groups * q.kchunks * q.sub * q.b_tile_bytes;
     q.bres_tx = all_w;
-    q.b_resident = (tc_resident_mode && (q.n_nt == 1 || q.nsplit) && all_w <= 112 * 1024) ? 1 : 0;
+    q.b_resident = ((q.n_nt == 1 || q.nsplit) && all_w <= 112 * 1024) ? 1 : 0;
     if (q.nsplit && !q.b_resident) { set_error("tc plan: N-split layer lost its resident weights"); delete plan; return PCLS_ERR_STATE; }
     q.bres_bytes = q.b_resident ? (all_w + 1023) / 1024 * 1024 : 0;
     // residual0 of the memory-bound layers (resident weights) with the TMA-store epilogue: TMA-loaded into a third
     // staging buffer and added in place (no per-thread address arithmetic, a whole block of latency hiding)
-    q.res_tma = (!skip && tc_res_tma_mode && L.res0 >= 0 && q.tma_store && q.cbw == 64 && q.b_resident && (cp.res0_channels * 2) % 16 == 0) ? 1 : 0;
+    q.res_tma = (!skip && L.res0 >= 0 && q.tma_store && q.cbw == 64 && q.b_resident && (cp.res0_channels * 2) % 16 == 0) ? 1 : 0;
     q.n_cbuf = (q.res_tma && !q.nsplit) ? 3 : 2;
     q.res_smem = (!skip && !q.res_tma && L.res0 >= 0 && q.BN <= 128) ? 1 : 0;
     // (skip: two 8 KB network-input tiles per group in place of the third staging buffer)
@@ -1444,8 +1359,6 @@ int Net::tc_plan_layer(ConvLayer& L, bool allow_group, bool* retry) {
     if (stages > 12) stages = 12;
     if (stages < 2) { delete plan; *retry = G > 1; return PCLS_OK; }
     q.stages = stages;
-    q.vstream = (PCLS_TC_VSTREAM && tc_vstream_mode && halo && cp.mode == MODE_3x3_S1 && q.b_resident && stages >= 3 * q.kchunks + 1) ? 1 : 0;
-    q.R = 1; q.n_hseg = q.Hgrid;
     plan->smem_bytes = (size_t)stages * stage_bytes + q.bres_bytes + cstage_total + 1024 /*alignment slack*/ +
                        (size_t)(2 * stages + 17 + 3 * TC_NG) * 8 + 48 + (cp.out_f32 ? 4 * TC_NG * 32 * 33 * 4 : 0) + (size_t)cp.cout_pad * 4 /*bias*/;
     // descriptors
@@ -1663,24 +1576,15 @@ int Net::tc_launch(ConvLayer& L, const ConvParams& p, int nb, cudaStream_t s) {
   prm.probs = head_args.probs; prm.preds = head_args.preds; prm.logits = head_args.logits;
   const int num_tiles = prm.num_tiles * nb;
   if (num_tiles == 0) return PCLS_OK;
-  int work = num_tiles;
-  if (prm.vstream) {
-    // rows per strip: the longest run that still leaves >= 6 strips per SM (wave quantisation), R | H
-    int R = 1;
-    for (int r = 32; r > 1; r /= 2)
-      if (prm.Hgrid % r == 0 && (long long)nb * prm.n_wt * (prm.Hgrid / r) >= 6LL * sm_count()) { R = r; break; }
-    prm.R = R; prm.n_hseg = prm.Hgrid / R;
-    work = num_tiles / R;
-  }
-  int grid = work < sm_count() ? work : sm_count();
+  int grid = num_tiles < sm_count() ? num_tiles : sm_count();
   if (prm.nsplit) grid -= grid % prm.n_nt;   // every CTA sees one N tile only (tile % n_nt == blockIdx.x % n_nt)
   // one skip tensor, TMA-loaded into the staging buffers, TMA-store epilogue, ReLU: the specialised residual kernel
-  const int rtma = prm.skip ? 3 : (tc_rtma_mode && prm.res_tma && prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 &&
-                    (prm.act == PCLS_ACT_RELU || prm.act == PCLS_ACT_LEAKY) && !(PCLS_TC_VSTREAM && prm.vstream)) ? 1
-                 : ((tc_rtma_mode & 2) && !prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 && !(PCLS_TC_VSTREAM && prm.vstream)) ? 2 : 0;
+  const int rtma = prm.skip ? 3 : (prm.res_tma && prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32 &&
+                                   (prm.act == PCLS_ACT_RELU || prm.act == PCLS_ACT_LEAKY)) ? 1
+                 : (!prm.res0 && !prm.res1 && prm.tma_store && !prm.out_f32) ? 2 : 0;
   const bool res = prm.res0 || prm.res1 || prm.skip;
   PCLS_CHECK_CUDA(launch_pdl(tc_kernel_for(prm.KC, prm.sub, prm.G, prm.is_bf16, res ? 1 : 0, prm.act == PCLS_ACT_LEAKY ? 1 : 0, prm.ksteps, rtma),
-                             dim3(grid), dim3(tc_threads(res)), plan->smem_bytes, s,
+                             dim3(grid), dim3(TC_THREADS), plan->smem_bytes, s,
                              plan->map_a, plan->map_b, plan->map_c, plan->map_r, plan->map_b2, plan->map_c2, prm, num_tiles));
   return check_launch("conv_tc_kernel");
 }

@@ -13,9 +13,6 @@
 
 namespace pcls {
 
-int pad48_mode = 1;   // A/B switch (pcls_net_set_option "pad48", before the ops are added)
-int pair_s2_mode = 1; // A/B switch "pair_s2": stride-2 convs with Cin = 32 run on the pixel-pair view (build_pair_view)
-
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 template <typename T>
@@ -85,7 +82,7 @@ int Net::add_conv(const pcls_conv_desc& d) {
   // expand); stored with a 64-channel pixel stride the tensor takes the 128-byte-row path like every other layer.  The
   // producing conv writes all 64 channels (zero weights and bias beyond 48: act(0) = 0), consumers contract 64 input
   // channels against zero-padded kernels.  Only for tensors that ONE convolution writes completely.
-  if (pad48_mode && !tensors[d.out_tensor].logits && tensors[d.out_tensor].channels == 48 && tensors[d.out_tensor].stride == 48 &&
+  if (!tensors[d.out_tensor].logits && tensors[d.out_tensor].channels == 48 && tensors[d.out_tensor].stride == 48 &&
       d.out_channel_offset == 0 && d.cout == 48 && d.residual0 < 0 && d.residual1 < 0 && d.kind == PCLS_CONV)
     tensors[d.out_tensor].stride = 64;
   const TensorInfo& ti = tensors[d.in_tensor];
@@ -197,7 +194,7 @@ void Net::build_pair_view(ConvLayer& L) {
   // 130-pair halo tiles with 128-byte rows per tile: enc1.down 0.328 -> 0.202 ms at batch 32.  A third of the MMAs multiply
   // zeros and the zero taps' weights are loaded like any others: for Cin = 64 (enc2.down, 295 KB of pair-view weights
   // streamed per tile) the same change measured 0.219 -> 0.343 ms, so Cin = 32 only.
-  if (L.in != 0 && pair_s2_mode && p.mode == MODE_3x3_S2 && p.pad_left == 0 && p.Win % 2 == 0 && !p.out_f32 && L.res0 < 0 &&
+  if (L.in != 0 && p.mode == MODE_3x3_S2 && p.pad_left == 0 && p.Win % 2 == 0 && !p.out_f32 && L.res0 < 0 &&
       L.res1 < 0 && p.cin == p.cin_pad && p.in_channels == p.cin_pad && p.cin_pad == 32 && p.Wout == p.Win / 2) {
     ConvParams q = p;
     const int cp2 = 2 * p.cin_pad;
@@ -594,7 +591,7 @@ int Net::run_pass(const float* lidar, int channels, const uint8_t* mask, bool ra
                                    tensors[L.out].width, tensors[L.in].stride, L.pad_left, s);
     } else {
       const CamLayer& L = cams[op.index];
-      rc = launch_cam<T>((const T*)tensor_ptr(L.in, nb), (T*)tensor_ptr(L.out, nb), L.p, nb, H, tensors[L.in].width, cam_px, s);
+      rc = launch_cam<T>((const T*)tensor_ptr(L.in, nb), (T*)tensor_ptr(L.out, nb), L.p, nb, H, tensors[L.in].width, s);
     }
     if (rc) return rc;
     if (tc_debug_buf && ev && op.type == OP_CONV) {  // development aid: print the counters of this launch
@@ -980,24 +977,6 @@ extern "C" int pcls_net_set_option(pcls_net* net, const char* name, int value) {
     PCLS_REQUIRE(!n->finalized, "keep_tensors must be set before pcls_net_finalize");
     n->keep_tensors = value != 0; return PCLS_OK;
   }
-  if (!strcmp(name, "tc_head")) { tc_head_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "cam_px")) { PCLS_REQUIRE(value >= 0 && value <= 2, "cam_px must be 0 (default), 1 or 2"); n->cam_px = value; n->drop_graphs(); return PCLS_OK; }
-  if (!strcmp(name, "tc_nsplit")) { tc_nsplit_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "pad48")) {
-    PCLS_REQUIRE(n->convs.empty(), "pad48 must be set before the first pcls_net_conv");
-    pad48_mode = value; return PCLS_OK;
-  }
-  if (!strcmp(name, "pair_s2")) {
-    PCLS_REQUIRE(n->convs.empty(), "pair_s2 must be set before the first pcls_net_conv");
-    pair_s2_mode = value; return PCLS_OK;
-  }
-  if (!strcmp(name, "tc_halo")) { tc_halo_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_rtma")) { tc_rtma_mode = value; n->drop_graphs(); return PCLS_OK; }
-  if (!strcmp(name, "tc_tma_store")) { tc_tma_store_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_group")) { tc_group_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_res_tma")) { tc_res_tma_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_split")) { tc_split_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_vstream")) { tc_vstream_mode = value; return PCLS_OK; }
   if (!strcmp(name, "fuse_up")) {
     PCLS_REQUIRE(!n->finalized, "fuse_up must be set before pcls_net_finalize");
     n->fuse_up = value != 0; return PCLS_OK;
@@ -1017,8 +996,6 @@ extern "C" int pcls_net_set_option(pcls_net* net, const char* name, int value) {
     if (!value && tc_debug_buf) { cudaFree(tc_debug_buf); tc_debug_buf = nullptr; }
     return PCLS_OK;
   }
-  if (!strcmp(name, "tc_resident")) { tc_resident_mode = value; return PCLS_OK; }
-  if (!strcmp(name, "tc_base_offset")) { tc_base_offset_mode = value; return PCLS_OK; }
   set_error("pcls_net_set_option: unknown option '%s'", name);
   return PCLS_ERR_INVALID;
 }

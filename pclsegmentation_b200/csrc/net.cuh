@@ -16,11 +16,8 @@ struct TensorInfo {
 
 struct TcPlan;    // tcgen05 launch plan of one conv layer (conv_tc.cu)
 struct HeadPlan;  // launch plan of the logits layer + fused segmentation head (conv_head.cu)
-extern int tc_head_mode;
-extern int tc_rtma_mode, tc_halo_mode, tc_resident_mode, tc_base_offset_mode, tc_tma_store_mode, tc_group_mode, tc_res_tma_mode, tc_split_mode, tc_vstream_mode, tc_nsplit_mode;
-extern int pad48_mode;  // 48-channel tensors written by one conv are stored with a 64-channel pixel stride (zero pads)
 extern const int tc_debug_compiled;
-extern unsigned long long* tc_debug_buf;  // A/B measurement switches (process-wide)
+extern unsigned long long* tc_debug_buf;  // wait-cycle counters of the most recent conv_tc_kernel launch ("tc_debug")
 
 struct ConvLayer {
   ConvParams p;
@@ -83,7 +80,6 @@ struct Net {
   bool fuse_skip = true;   // a 1x1 conv of the network input whose only reader adds it as a skip: computed by that reader
   struct HeadArgs { int head = 0, none_index = 0; const uint8_t* mask = nullptr; float* probs = nullptr; int32_t* preds = nullptr; float* logits = nullptr; } head_args;
   int micro_batch = 0;
-  int cam_px = 0;             // CAM pixels per thread: 0 = default (2), 1 = cam_kernel, 2 = cam2_kernel
   bool keep_tensors = false;  // test aid: no arena reuse, every intermediate stays readable after the forward
   // device state
   int frames_per_pass = 0;

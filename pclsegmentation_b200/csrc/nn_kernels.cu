@@ -307,18 +307,23 @@ template int launch_maxpool3x3_s2<__nv_bfloat16>(const __nv_bfloat16*, __nv_bflo
 // --------------------------------------------------------------------------------------------------
 // CAM (nets/SqueezeSegV2.py:66-70), one row-streaming kernel:
 //   pool = maxpool7x7_SAME(x); s = relu(W1^T pool + b1); e = sigmoid(W2^T s + b2); out = x * e
-// A CTA owns a strip of TW columns of one frame and walks down the H rows; a thread owns one pixel x 8 channels of the
-// strip.  Per iteration, ONE __syncthreads:
+// A CTA (128 threads) owns a strip of TW columns of one frame and walks down the H rows; a thread owns two horizontally
+// adjacent pixels x 8 channels of the strip.  Per iteration, ONE __syncthreads:
 //   stage   input row r+3 travels global -> smem ring with cp.async (TW + 6 columns; -inf outside the image)
-//   phase A horizontal 7-max of row r from the ring; the last seven horizontal maxima stay in registers -> vertical
-//           7-max = pooled row r-3, still in registers.  They ARE the A fragment of the squeeze MMA (mma.sync m16n8k16,
-//           fp32 accumulate; the K order is a free permutation of the channels, chosen so that lane (g, t) holds pixel g,
-//           channels 8 cv .. 8 cv + 7, cv = 4 cvg + t; fragment rows 8-15 are unused).  A warp covers 8 pixels x 32
-//           channels and leaves its partial sums in its own [TW][8] fp32 tile.
+//   phase A horizontal 7-max of row r from the ring for both pixels (their windows share six of their seven columns: 8
+//           loads for the pair); the last seven horizontal maxima stay in registers -> vertical 7-max = pooled row r-3,
+//           still in registers.  They ARE the A fragment of the squeeze MMA (mma.sync m16n8k16, fp32 accumulate; the K
+//           order is a free permutation of the channels, chosen so that lane (g, t) holds channels 8 cv .. 8 cv + 7,
+//           cv = 4 cvg + t, of its first pixel in fragment row g and of its second in row g + 8).  A warp covers 16 pixels x
+//           32 channels and leaves its partial sums in its own [TW][8] fp32 tile.
 //   phase B (row r-4) sum of the C/32 partial tiles -> bias + ReLU -> A fragment of the excitation MMAs, whose N order is
 //           permuted so that lane (g, t) receives exactly its own 8 channels (b2 rides along as two extra K rows, split
-//           hi + lo); sigmoid on the SFU, gate x (16 bytes from the ring), one coalesced 16-byte global store.
+//           hi + lo); sigmoid on the SFU, gate x (16 bytes per pixel from the ring), two coalesced 16-byte global stores.
 // HBM traffic: (TW + 6) / TW reads + 1 write of the tensor.  Weights live in registers as MMA B fragments.
+// Two pixels per thread because the one-pixel form's busiest unit was the LSU data pipe (shared-memory wavefronts, 64 %),
+// 7 of its LDS.128 per pixel going to the horizontal 7-max; the pair also carries its second pixel in fragment rows 8-15
+// that were idle there: half the MMAs, address arithmetic and loop overhead per pixel.  Measured at batch 32: C = 64
+// 0.138 vs 0.185 ms, C = 128 0.143 vs 0.189 ms (the one-pixel kernel has since been removed).
 // --------------------------------------------------------------------------------------------------
 template <typename T> __device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]);
 template <> __device__ __forceinline__ void mma16816<__half>(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
@@ -339,56 +344,40 @@ template <typename T> __device__ __forceinline__ float2 unpack2(uint32_t v) {
   const T* h = reinterpret_cast<const T*>(&v);
   return make_float2(to_f32<T>(h[0]), to_f32<T>(h[1]));
 }
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-// PCLS_CAM_TANH=1: sigmoid(e) = 0.5 + 0.5 tanh(e / 2) with ONE SFU op (tanh.approx.f32, max relative error 2^-11) instead
-// of ex2 + rcp; the factor 1/2 is folded into W2 / b2.  x * sigmoid = fma(x/2, t, x/2).
-#ifndef PCLS_CAM_TANH
-#define PCLS_CAM_TANH 1
-#endif
+// sigmoid(e) = 0.5 + 0.5 tanh(e / 2) with ONE SFU op (tanh.approx.f32, max relative error 2^-11) instead of ex2 + rcp
+// (0.137 -> 0.127 ms at C = 64, 0.143 -> 0.132 ms at C = 128); the factor 1/2 is folded into W2 / b2.  x * sigmoid =
+// fma(x/2, t, x/2).
 __device__ __forceinline__ float tanh_approx(float x) {
   float y;
   asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-__device__ __forceinline__ float rcp_approx(float x) {
-  float y;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 
-#ifndef PCLS_CAM_DIST
-#define PCLS_CAM_DIST 3
-#endif
-template <int C, int PX = 1> struct CamGeom {     // PX = pixels per thread (cam_kernel 1, cam2_kernel 2)
+constexpr int CAM_DIST = 3;   // rows of loads in flight (5 measured no faster: the per-row dependency chain bounds CAM)
+constexpr int CAM_CTAS = 3;   // resident CTAs per SM the register allocation targets (4: 128 registers, spills, 0.137 -> 0.256 ms)
+template <int C> struct CamGeom {
   static constexpr int CV = C / 8;              // 16-byte vectors per pixel (8 or 16)
   static constexpr int TW = 256 / CV;           // columns per CTA (32 or 16)
-  static constexpr int PITCH = C * 2 + 64 / PX; // bytes per ring pixel; PX * PITCH = 64 mod 128: the (pixel, 4 vectors) reads
+  static constexpr int PITCH = C * 2 + 32;      // bytes per ring pixel; 2 PITCH = 64 mod 128: the (pixel, 4 vectors) reads
                                                 // of a quarter warp (2 threads' pixels x 64 bytes) fall on disjoint banks.
-                                                // (cam2 with the 1-pixel pitch: every LDS.128 took two wavefronts, ncu
+                                                // (with a pitch of C * 2 + 64 every LDS.128 took two wavefronts, ncu
                                                 // l1tex shared wavefronts 70 M vs 36 M ideal)
   static constexpr int ROWB = (TW + 6) * PITCH; // bytes per ring slot
-  static constexpr int DIST = PCLS_CAM_DIST, NB = DIST + 6;   // ring: rows r-5 .. r+DIST resident (DIST rows of loads in flight)
+  static constexpr int DIST = CAM_DIST, NB = DIST + 6;   // ring: rows r-5 .. r+DIST resident (DIST rows of loads in flight)
   static constexpr int SMEM = NB * ROWB + (2 * (CV / 4) + 1) * TW * 8 * 4;
 };
 
-#ifndef PCLS_CAM_CTAS
-#define PCLS_CAM_CTAS 2   // resident CTAs per SM the register allocation targets (3 needs <= 85 registers: spills, measured slower)
-#endif
 template <typename T, int C>
-__global__ void __launch_bounds__(256, PCLS_CAM_CTAS)
-cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int H, int W, int rows_per_seg) {
+__global__ void __launch_bounds__(128, CAM_CTAS)
+cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int H, int W, int rows_per_seg) {
   using G = CamGeom<C>;
   constexpr int CV = G::CV, TW = G::TW, PITCH = G::PITCH, ROWB = G::ROWB, NB = G::NB, DIST = G::DIST;
   constexpr int R = C / 16;                // reduced channels (4 or 8)
   constexpr int NSTG = (TW + 6) * CV;      // 16-byte copies per staged row
-  constexpr int LPT = (NSTG + 255) / 256;
+  constexpr int LPT = (NSTG + 127) / 128;
   constexpr int CVG = CV / 4;              // warps per pixel group (2 or 4)
   constexpr int STILE = TW * 8 * 4;        // bytes of one partial squeeze tile [TW][8] fp32
-  extern __shared__ int4 cam_smem[];       // ring [NB][ROWB] | squeeze tiles [2][CVG][TW][8] fp32 | b1 tile [TW][8] fp32
+  extern __shared__ int4 cam_smem[];       // ring [NB][ROWB] | squeeze tiles [2][CVG][TW][8] fp32
   unsigned char* const ring = reinterpret_cast<unsigned char*>(cam_smem);
   unsigned char* const St = ring + NB * ROWB;
 
@@ -396,9 +385,9 @@ cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int
   const int64_t b = blockIdx.y;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int cvg = warp % CVG, pg = warp / CVG;
-  const int c = pg * 8 + g, cv = cvg * 4 + t;              // this thread's pixel (column in the strip) and channel vector
+  const int c0 = pg * 16 + 2 * g, cv = cvg * 4 + t;      // this thread's pixels c0, c0 + 1 (columns of the strip) and channel vector
   const int4 NEG = neg_inf8<T>();
-  const int64_t rowv = (int64_t)W * CV;                    // vectors per image row
+  const int64_t rowv = (int64_t)W * CV;                  // vectors per image row
 
   // ---- squeeze weights: B fragments of the two k-steps.  K slot (2t', 2t'+1 | +8) <-> channels 8 cv(t') + 4u + {0,1 | 2,3}
   uint32_t w1f[2][2];
@@ -410,9 +399,8 @@ cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int
     w1f[u][1] = pack2<T>(w1(2), w1(3));
   }
   // ---- excitation weights: N slot n of tile q <-> channel 8 (4 cvg + n / 2) + 2q + n % 2, so that the accumulator of
-  // lane (g, t) (columns 2t, 2t+1) is channel pair q of its own vector.  sigmoid(e) = 1 / (1 + 2^(-log2(e) e)): the factor
-  // is folded into W2 and b2.
-  constexpr float NL2E = -1.4426950408889634f;
+  // lane (g, t) (columns 2t, 2t+1) is channel pair q of its own vector.  The tanh form's 1/2 is folded into W2 and b2.
+  constexpr float NL2E = 0.5f;
   uint32_t w2f[4];
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
@@ -433,21 +421,19 @@ cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int
   // ---- staging: this thread's copies of a row (fixed columns, the source advances one image row per call) ----
   const int4* const fin = in + b * H * rowv;                 // this frame (CTA-uniform); per-thread offsets stay 32-bit
   int4* const fout = out + b * H * rowv;
-  static_assert(LPT == 2, "two copies per thread and row");
-  // copy k = 0: column w0 - 3 + tid / CV, vector tid % CV; copy k = 1: 256 / CV columns further right
+  // copy k: column w0 - 3 + (tid + 128 k) / CV, vector tid % CV
   unsigned sptr = (unsigned)((w0 - 3 + (int)threadIdx.x / CV) * CV + threadIdx.x % CV);
   const unsigned soff = (unsigned)__cvta_generic_to_shared(ring) + (threadIdx.x / CV) * PITCH + (threadIdx.x % CV) * 16;
   bool sok[LPT];
 #pragma unroll
   for (int k = 0; k < LPT; ++k) {
-    const int i = threadIdx.x + k * 256;
+    const int i = threadIdx.x + k * 128;
     const int col = w0 - 3 + i / CV;
     sok[k] = i < NSTG && col >= 0 && col < W;
     if (i < NSTG && !sok[k])                                               // columns outside the image: -inf, written once
       for (int sl = 0; sl < NB; ++sl) *reinterpret_cast<int4*>(ring + sl * ROWB + (i / CV) * PITCH + (i % CV) * 16) = NEG;
   }
-  for (int i = threadIdx.x; i < TW * 8; i += 256)                          // b1, replicated per pixel (zero beyond R)
-    reinterpret_cast<float*>(St + 2 * CVG * STILE)[i] = (i % 8) < R ? p.b1[i % 8] : 0.0f;
+  const float b1x = 2 * t < R ? p.b1[2 * t] : 0.0f, b1y = 2 * t + 1 < R ? p.b1[2 * t + 1] : 0.0f;
   // blockIdx.z = row segment [h0, h1) of the strip (small batches: more CTAs than SMs; a segment re-reads three rows
   // above and below).  The walk starts at input row a0 = max(h0 - 3, 0).
   pdl_trigger(p.pdl_early);   // PDL (common.cuh): the weight fragments above are independent of the producing layer
@@ -460,25 +446,26 @@ cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int
 #pragma unroll
       for (int k = 0; k < LPT; ++k)
         if (sok[k])
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(soff + k * (256 / CV) * PITCH + slot * ROWB),
-                       "l"(fin + (unsigned)(sptr + k * 256)) : "memory");   // 32-bit wrap: sptr is "negative" left of the image
+          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(soff + k * (128 / CV) * PITCH + slot * ROWB),
+                       "l"(fin + (unsigned)(sptr + k * 128)) : "memory");   // 32-bit wrap: sptr is "negative" left of the image
       sptr += (unsigned)rowv;
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
 
   // ---- per-thread offsets ----
-  const unsigned a_off = c * PITCH + cv * 16;                              // ring: pixel c - 3 (+ d * PITCH), this vector
-  const unsigned s_off = (c * 8 + 2 * t) * 4;                              // squeeze tile: pixel c, columns 2t, 2t+1
-  const bool col_ok = (w0 + c) < W;
-  unsigned optr = (unsigned)((w0 + c) * CV + cv) + (unsigned)h0 * (unsigned)rowv;
+  const unsigned a_off = c0 * PITCH + cv * 16;            // ring: pixel c0 - 3 (+ d * PITCH), this vector
+  const unsigned s_off = ((pg * 8 + g) * 4 + t) * 16;     // squeeze tile [pixel pair][t]: {c0: columns 2t, 2t+1 | c0 + 1: same} = one
+                                                          // conflict-free 16-byte access per lane
+  const bool ok0 = (w0 + c0) < W, ok1 = (w0 + c0 + 1) < W;
+  unsigned optr = (unsigned)((w0 + c0) * CV + cv) + (unsigned)h0 * (unsigned)rowv;
 
-  int4 win[7];   // horizontal maxima of the last seven input rows (slot = row mod 7)
+  int4 win0[7], win1[7];   // horizontal maxima of the last seven input rows (slot = row mod 7)
 #pragma unroll
-  for (int k = 0; k < 7; ++k) win[k] = NEG;
+  for (int k = 0; k < 7; ++k) { win0[k] = NEG; win1[k] = NEG; }
 
   for (int r = 0; r < DIST; ++r) stage_row(a0 + r, r);
-  int sc = 0;                                                              // ring slot of row r ((r - a0) mod NB)
+  int sc = 0;                                             // ring slot of row r ((r - a0) mod NB)
   for (int r0 = a0; r0 < h1 + 4; r0 += 7) {
 #pragma unroll
     for (int j = 0; j < 7; ++j) {
@@ -488,173 +475,9 @@ cam_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int
       asm volatile("cp.async.wait_group %0;" ::"n"(DIST) : "memory");    // row r has landed (this thread's copies)
       __syncthreads();
 
-      // ---------------- phase A: pooled row r - 3, squeeze partial sums -> tiles [r & 1] ----------------
-      if (r < h1 + 3) {
-        int4 hm = NEG;                                                     // rows below the image pad with -inf
-        if (r < H) {
-          const unsigned char* src = ring + sc * ROWB + a_off;
-          hm = *reinterpret_cast<const int4*>(src);
-#pragma unroll
-          for (int d = 1; d < 4; ++d) hm = max8<T>(hm, *reinterpret_cast<const int4*>(src + d * PITCH));
-          __syncwarp();   // two batches of loads: seven 16-byte values in flight at once cost 12 more registers (spills)
-#pragma unroll
-          for (int d = 4; d < 7; ++d) hm = max8<T>(hm, *reinterpret_cast<const int4*>(src + d * PITCH));
-        }
-        win[j] = hm;
-        if (r >= h0 + 3) {
-          int4 vm = win[0];
-#pragma unroll
-          for (int k = 1; k < 7; ++k) vm = max8<T>(vm, win[k]);
-          float sq[4] = {0.0f, 0.0f, 0.0f, 0.0f};   // (columns right of the image carry -inf: their rows are never stored)
-          const uint32_t a0[4] = {(uint32_t)vm.x, 0u, (uint32_t)vm.y, 0u};
-          const uint32_t a1[4] = {(uint32_t)vm.z, 0u, (uint32_t)vm.w, 0u};
-          mma16816<T>(sq, a0, w1f[0]);
-          mma16816<T>(sq, a1, w1f[1]);
-          *reinterpret_cast<float2*>(St + ((r & 1) * CVG + cvg) * STILE + s_off) = make_float2(sq[0], sq[1]);
-        }
-      }
-
-      // ---------------- phase B: gate and store row r - 4 (tiles [(r - 1) & 1]) ----------------
-      if (r >= h0 + 4) {
-        float2 sv = *reinterpret_cast<const float2*>(St + 2 * CVG * STILE + s_off);   // b1
-#pragma unroll
-        for (int k = 0; k < CVG; ++k) {
-          const float2 part = *reinterpret_cast<const float2*>(St + (((r - 1) & 1) * CVG + k) * STILE + s_off);
-          sv.x += part.x; sv.y += part.y;
-        }
-        uint32_t sa[4] = {pack2<T>(fmaxf(sv.x, 0.0f), fmaxf(sv.y, 0.0f)), 0u, 0u, 0u};
-        const int sb = sc + NB - 4 >= NB ? sc - 4 : sc + NB - 4;           // ring slot of input row r - 4
-        const int4 xv = *reinterpret_cast<const int4*>(ring + sb * ROWB + a_off + 3 * PITCH);
-        const uint32_t xw[4] = {(uint32_t)xv.x, (uint32_t)xv.y, (uint32_t)xv.z, (uint32_t)xv.w};
-        uint32_t o[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float e[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-          const uint32_t bq[2] = {w2f[q], w2b};
-          sa[2] = t == q ? one2 : 0u;
-          mma16816<T>(e, sa, bq);
-          const float2 x = unpack2<T>(xw[q]);
-          o[q] = pack2<T>(x.x * rcp_approx(1.0f + ex2_approx(e[0])), x.y * rcp_approx(1.0f + ex2_approx(e[1])));
-        }
-        if (col_ok) fout[optr] = make_int4((int)o[0], (int)o[1], (int)o[2], (int)o[3]);
-        optr += (unsigned)rowv;
-      }
-      sc = sc + 1 == NB ? 0 : sc + 1;
-    }
-  }
-}
-
-// ---- two pixels per thread --------------------------------------------------------------------------------------------
-// Same algorithm and shared-memory layout as cam_kernel, but a thread owns TWO horizontally adjacent pixels x 8 channels
-// (CTA = 128 threads over the same TW-column strip).  ncu on cam_kernel: the LSU data pipe (shared-memory wavefronts) is
-// the busiest unit (64 %), 7 of its LDS.128 per pixel go to the horizontal 7-max; adjacent pixels share six of their seven
-// columns, so the pair needs 8 loads instead of 14, and the squeeze / excitation MMAs (m16n8k16) carry the second pixel in
-// fragment rows 8-15 that were idle: half the MMAs, address arithmetic and loop overhead per pixel.  Needs ~150 registers:
-// three 128-thread CTAs per SM.
-#ifndef PCLS_CAM2_CTAS
-#define PCLS_CAM2_CTAS 3   // resident CTAs per SM the two-pixel kernel's register allocation targets
-#endif
-template <typename T, int C>
-__global__ void __launch_bounds__(128, PCLS_CAM2_CTAS)
-cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, int H, int W, int rows_per_seg) {
-  using G = CamGeom<C, 2>;
-  constexpr int CV = G::CV, TW = G::TW, PITCH = G::PITCH, ROWB = G::ROWB, NB = G::NB, DIST = G::DIST;
-  constexpr int R = C / 16;
-  constexpr int NSTG = (TW + 6) * CV;
-  constexpr int LPT = (NSTG + 127) / 128;
-  constexpr int CVG = CV / 4;
-  constexpr int STILE = TW * 8 * 4;
-  extern __shared__ int4 cam_smem[];
-  unsigned char* const ring = reinterpret_cast<unsigned char*>(cam_smem);
-  unsigned char* const St = ring + NB * ROWB;
-
-  const int w0 = blockIdx.x * TW;
-  const int64_t b = blockIdx.y;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int cvg = warp % CVG, pg = warp / CVG;
-  const int c0 = pg * 16 + 2 * g, cv = cvg * 4 + t;      // this thread's pixels c0, c0 + 1 (columns of the strip) and channel vector
-  const int4 NEG = neg_inf8<T>();
-  const int64_t rowv = (int64_t)W * CV;
-
-  uint32_t w1f[2][2];
-#pragma unroll
-  for (int u = 0; u < 2; ++u) {
-    const int ch = cv * 8 + 4 * u;
-    auto w1 = [&](int k) { return g < R ? p.w1[(ch + k) * R + g] : 0.0f; };
-    w1f[u][0] = pack2<T>(w1(0), w1(1));
-    w1f[u][1] = pack2<T>(w1(2), w1(3));
-  }
-  constexpr float NL2E = PCLS_CAM_TANH ? 0.5f : -1.4426950408889634f;   // (PCLS_CAM_TANH: the tanh form's 1/2)
-  uint32_t w2f[4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const int chn = (cvg * 4 + (g >> 1)) * 8 + 2 * q + (g & 1);
-    auto w2 = [&](int j) { return j < R ? NL2E * p.w2[j * C + chn] : 0.0f; };
-    w2f[q] = pack2<T>(w2(2 * t), w2(2 * t + 1));
-  }
-  uint32_t w2b;
-  {
-    const float bias = NL2E * p.b2[(cvg * 4 + (g >> 1)) * 8 + 2 * t + (g & 1)];
-    const float hi = to_f32<T>(from_f32<T>(bias));
-    w2b = pack2<T>(hi, bias - hi);
-  }
-  const uint32_t one2 = pack2<T>(1.0f, 1.0f);
-
-  const int4* const fin = in + b * H * rowv;
-  int4* const fout = out + b * H * rowv;
-  unsigned sptr = (unsigned)((w0 - 3 + (int)threadIdx.x / CV) * CV + threadIdx.x % CV);
-  const unsigned soff = (unsigned)__cvta_generic_to_shared(ring) + (threadIdx.x / CV) * PITCH + (threadIdx.x % CV) * 16;
-  bool sok[LPT];
-#pragma unroll
-  for (int k = 0; k < LPT; ++k) {
-    const int i = threadIdx.x + k * 128;
-    const int col = w0 - 3 + i / CV;
-    sok[k] = i < NSTG && col >= 0 && col < W;
-    if (i < NSTG && !sok[k])
-      for (int sl = 0; sl < NB; ++sl) *reinterpret_cast<int4*>(ring + sl * ROWB + (i / CV) * PITCH + (i % CV) * 16) = NEG;
-  }
-  const float b1x = 2 * t < R ? p.b1[2 * t] : 0.0f, b1y = 2 * t + 1 < R ? p.b1[2 * t + 1] : 0.0f;
-  pdl_trigger(p.pdl_early);   // PDL (common.cuh): the weight fragments above are independent of the producing layer
-  pdl_wait();
-  const int h0 = blockIdx.z * rows_per_seg, h1 = min(H, h0 + rows_per_seg);
-  const int a0 = h0 - 3 < 0 ? 0 : h0 - 3;
-  sptr += (unsigned)a0 * (unsigned)rowv;
-  auto stage_row = [&](int r, int slot) {
-    if (r < H && r <= h1 + 2) {
-#pragma unroll
-      for (int k = 0; k < LPT; ++k)
-        if (sok[k])
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(soff + k * (128 / CV) * PITCH + slot * ROWB),
-                       "l"(fin + (unsigned)(sptr + k * 128)) : "memory");
-      sptr += (unsigned)rowv;
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-
-  const unsigned a_off = c0 * PITCH + cv * 16;            // ring: pixel c0 - 3 (+ d * PITCH), this vector
-  const unsigned s_off = ((pg * 8 + g) * 4 + t) * 16;     // squeeze tile [pixel pair][t]: {c0: columns 2t, 2t+1 | c0 + 1: same} = one
-                                                          // conflict-free 16-byte access per lane
-  const bool ok0 = (w0 + c0) < W, ok1 = (w0 + c0 + 1) < W;
-  unsigned optr = (unsigned)((w0 + c0) * CV + cv) + (unsigned)h0 * (unsigned)rowv;
-
-  int4 win0[7], win1[7];
-#pragma unroll
-  for (int k = 0; k < 7; ++k) { win0[k] = NEG; win1[k] = NEG; }
-
-  for (int r = 0; r < DIST; ++r) stage_row(a0 + r, r);
-  int sc = 0;
-  for (int r0 = a0; r0 < h1 + 4; r0 += 7) {
-#pragma unroll
-    for (int j = 0; j < 7; ++j) {
-      const int r = r0 + j;
-      if (r >= h1 + 4) break;
-      stage_row(r + DIST, sc + DIST >= NB ? sc + DIST - NB : sc + DIST);
-      asm volatile("cp.async.wait_group %0;" ::"n"(DIST) : "memory");
-      __syncthreads();
-
       // ---------------- phase A: pooled row r - 3 of both pixels, squeeze partial sums -> tiles [r & 1] ----------------
       if (r < h1 + 3) {
-        int4 hm0 = NEG, hm1 = NEG;
+        int4 hm0 = NEG, hm1 = NEG;                                         // rows below the image pad with -inf
         if (r < H) {
           const unsigned char* src = ring + sc * ROWB + a_off;
           int4 m6 = *reinterpret_cast<const int4*>(src + PITCH);                     // columns shared by both windows
@@ -668,7 +491,8 @@ cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, in
           int4 vm0 = win0[0], vm1 = win1[0];
 #pragma unroll
           for (int k = 1; k < 7; ++k) { vm0 = max8<T>(vm0, win0[k]); vm1 = max8<T>(vm1, win1[k]); }
-          float sq[4] = {0.0f, 0.0f, 0.0f, 0.0f};   // rows g / g + 8 of the fragment = pixels c0 / c0 + 1
+          // rows g / g + 8 of the fragment = pixels c0 / c0 + 1 (columns right of the image carry -inf: never stored)
+          float sq[4] = {0.0f, 0.0f, 0.0f, 0.0f};
           const uint32_t fa0[4] = {(uint32_t)vm0.x, (uint32_t)vm1.x, (uint32_t)vm0.y, (uint32_t)vm1.y};
           const uint32_t fa1[4] = {(uint32_t)vm0.z, (uint32_t)vm1.z, (uint32_t)vm0.w, (uint32_t)vm1.w};
           mma16816<T>(sq, fa0, w1f[0]);
@@ -686,7 +510,7 @@ cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, in
           sv0.x += pa.x; sv0.y += pa.y; sv1.x += pa.z; sv1.y += pa.w;
         }
         uint32_t sa[4] = {pack2<T>(fmaxf(sv0.x, 0.0f), fmaxf(sv0.y, 0.0f)), pack2<T>(fmaxf(sv1.x, 0.0f), fmaxf(sv1.y, 0.0f)), 0u, 0u};
-        const int sb = sc + NB - 4 >= NB ? sc - 4 : sc + NB - 4;
+        const int sb = sc + NB - 4 >= NB ? sc - 4 : sc + NB - 4;           // ring slot of input row r - 4
         const int4 xv0 = *reinterpret_cast<const int4*>(ring + sb * ROWB + a_off + 3 * PITCH);
         const int4 xv1 = *reinterpret_cast<const int4*>(ring + sb * ROWB + a_off + 4 * PITCH);
         const uint32_t xw0[4] = {(uint32_t)xv0.x, (uint32_t)xv0.y, (uint32_t)xv0.z, (uint32_t)xv0.w};
@@ -700,14 +524,9 @@ cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, in
           sa[3] = sa[2];
           mma16816<T>(e, sa, bq);
           const float2 x0 = unpack2<T>(xw0[q]), x1 = unpack2<T>(xw1[q]);
-          if constexpr (PCLS_CAM_TANH) {
-            const float h0 = 0.5f * x0.x, h1 = 0.5f * x0.y, h2 = 0.5f * x1.x, h3 = 0.5f * x1.y;
-            o0[q] = pack2<T>(fmaf(h0, tanh_approx(e[0]), h0), fmaf(h1, tanh_approx(e[1]), h1));
-            o1[q] = pack2<T>(fmaf(h2, tanh_approx(e[2]), h2), fmaf(h3, tanh_approx(e[3]), h3));
-          } else {
-          o0[q] = pack2<T>(x0.x * rcp_approx(1.0f + ex2_approx(e[0])), x0.y * rcp_approx(1.0f + ex2_approx(e[1])));
-          o1[q] = pack2<T>(x1.x * rcp_approx(1.0f + ex2_approx(e[2])), x1.y * rcp_approx(1.0f + ex2_approx(e[3])));
-          }
+          const float h0 = 0.5f * x0.x, h1 = 0.5f * x0.y, h2 = 0.5f * x1.x, h3 = 0.5f * x1.y;
+          o0[q] = pack2<T>(fmaf(h0, tanh_approx(e[0]), h0), fmaf(h1, tanh_approx(e[1]), h1));
+          o1[q] = pack2<T>(fmaf(h2, tanh_approx(e[2]), h2), fmaf(h3, tanh_approx(e[3]), h3));
         }
         if (ok0) fout[optr] = make_int4((int)o0[0], (int)o0[1], (int)o0[2], (int)o0[3]);
         if (ok1) fout[optr + CV] = make_int4((int)o1[0], (int)o1[1], (int)o1[2], (int)o1[3]);
@@ -718,18 +537,15 @@ cam2_kernel(const int4* __restrict__ in, int4* __restrict__ out, CamParams p, in
   }
 }
 
-// px: pixels per thread (pcls_net_set_option "cam_px"): 1 = cam_kernel, 2 = cam2_kernel, 0 = default = 2 (measured at batch 32:
-// C = 64 0.138 vs 0.185 ms, C = 128 0.143 vs 0.189 ms)
 template <typename T>
-int launch_cam(const T* in, T* out, const CamParams& p, int B, int H, int W, int px, cudaStream_t s) {
+int launch_cam(const T* in, T* out, const CamParams& p, int B, int H, int W, cudaStream_t s) {
   if (B == 0) return PCLS_OK;
   PCLS_REQUIRE(p.C == 64 || p.C == 128, "CAM: channels must be 64 or 128, got %d", p.C);
   PCLS_REQUIRE(p.R == p.C / 16, "CAM: reduced channels must be C/16");
   const int TW = 256 / (p.C / 8);
-  // row segments (>= 8 rows each): minimise  waves x iterations per CTA  with two CTAs resident per SM; a segment of n
-  // rows runs n + 7 iterations (three rows of halo above / below and the pipeline drain)
-  const bool two = px != 1;
-  const int64_t strips = ceil_div(W, TW) * (int64_t)B, slots = (int64_t)sm_count() * (two ? PCLS_CAM2_CTAS : PCLS_CAM_CTAS);
+  // row segments (>= 8 rows each): minimise  waves x iterations per CTA  with CAM_CTAS CTAs resident per SM; a segment of
+  // n rows runs n + 7 iterations (three rows of halo above / below and the pipeline drain)
+  const int64_t strips = ceil_div(W, TW) * (int64_t)B, slots = (int64_t)sm_count() * CAM_CTAS;
   int segs = 1;
   int64_t best = -1;
   for (int sgs = 1; sgs <= (H >= 8 ? H / 8 : 1); ++sgs) {
@@ -739,25 +555,24 @@ int launch_cam(const T* in, T* out, const CamParams& p, int B, int H, int W, int
   const int rows_per_seg = (int)ceil_div(H, segs);
   segs = (int)ceil_div(H, rows_per_seg);
   dim3 grid((unsigned)ceil_div(W, TW), (unsigned)B, (unsigned)segs);
-  const int smem = two ? (p.C == 64 ? CamGeom<64, 2>::SMEM : CamGeom<128, 2>::SMEM)
-                       : (p.C == 64 ? CamGeom<64>::SMEM : CamGeom<128>::SMEM);   // ring + squeeze tiles, see cam_kernel
-  auto kern = two ? (p.C == 64 ? cam2_kernel<T, 64> : cam2_kernel<T, 128>) : (p.C == 64 ? cam_kernel<T, 64> : cam_kernel<T, 128>);
-  static bool configured[64][2][2] = {};   // function attributes are per device
+  const int smem = p.C == 64 ? CamGeom<64>::SMEM : CamGeom<128>::SMEM;
+  auto kern = p.C == 64 ? cam2_kernel<T, 64> : cam2_kernel<T, 128>;
+  static bool configured[64][2] = {};   // function attributes are per device
   int dev = 0;
   cudaGetDevice(&dev);
-  if (!configured[dev & 63][two][p.C == 128]) {
+  if (!configured[dev & 63][p.C == 128]) {
     PCLS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     PCLS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    configured[dev & 63][two][p.C == 128] = true;
+    configured[dev & 63][p.C == 128] = true;
   }
   CamParams q = p;
   q.pdl_early = pdl_early_now;
-  PCLS_CHECK_CUDA(launch_pdl(kern, grid, dim3(two ? 128 : 256), (size_t)smem, s, reinterpret_cast<const int4*>(in),
+  PCLS_CHECK_CUDA(launch_pdl(kern, grid, dim3(128), (size_t)smem, s, reinterpret_cast<const int4*>(in),
                              reinterpret_cast<int4*>(out), q, H, W, rows_per_seg));
-  return check_launch("cam_kernel");
+  return check_launch("cam2_kernel");
 }
-template int launch_cam<__half>(const __half*, __half*, const CamParams&, int, int, int, int, cudaStream_t);
-template int launch_cam<__nv_bfloat16>(const __nv_bfloat16*, __nv_bfloat16*, const CamParams&, int, int, int, int, cudaStream_t);
+template int launch_cam<__half>(const __half*, __half*, const CamParams&, int, int, int, cudaStream_t);
+template int launch_cam<__nv_bfloat16>(const __nv_bfloat16*, __nv_bfloat16*, const CamParams&, int, int, int, cudaStream_t);
 
 // --------------------------------------------------------------------------------------------------
 // n dense output elements [pixels][channels]; the input holds `stride` >= channels values per pixel (padded tensors)

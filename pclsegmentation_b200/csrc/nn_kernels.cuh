@@ -80,7 +80,7 @@ struct CamParams {
   const float* b2;     // [C]
   int pdl_early;       // filled by the launcher (common.cuh)
 };
-template <typename T> int launch_cam(const T* in, T* out, const CamParams& p, int B, int H, int W, int px, cudaStream_t s);
+template <typename T> int launch_cam(const T* in, T* out, const CamParams& p, int B, int H, int W, cudaStream_t s);
 template <typename T> int launch_tensor_to_f32(const T* in, float* out, int64_t n, int channels, int stride, cudaStream_t s);
 
 int launch_head(const float* logits, const uint8_t* mask, int64_t n_pixels, int nc, int none_index, float* probs,

@@ -6,7 +6,7 @@ from .SegmentationNetwork import PCLSegmentationNetwork
 
 
 class CAM(L.Layer):
-  """Context Aggregation Module: x * sigmoid(BN(1x1(relu(BN(1x1(maxpool7x7(x))))))) - ONE fused kernel (cam_kernel)."""
+  """Context Aggregation Module: x * sigmoid(BN(1x1(relu(BN(1x1(maxpool7x7(x))))))) - ONE fused kernel (cam2_kernel)."""
 
   def __init__(self, path, in_channels, reduction_factor=16):
     super().__init__(path)

@@ -43,7 +43,7 @@ class TinyNet:
     opts = {"conv_impl": conv_impl, "use_graph": 0}
     if keep:
       opts["keep_tensors"] = 1
-    for kv in os.environ.get("PCLS_TEST_OPTS", "").split(","):  # e.g. tc_base_offset=0 (A/B experiments)
+    for kv in os.environ.get("PCLS_TEST_OPTS", "").split(","):  # e.g. fuse_pool=0 (A/B experiments)
       if "=" in kv:
         opts[kv.split("=")[0]] = int(kv.split("=")[1])
     net = g.build_net(self.logits, 2, 0, _lib.PCLS_F16, B, opts)
@@ -252,11 +252,9 @@ def test_residual_and_skip_adds(impl):
   _check_layer(ys, got, p, "c2", "b2", act="leaky", residuals=[ys, ya], what="block 3x3 + residual + skip")
 
 
-@pytest.mark.parametrize("px", [2, 1])
 @pytest.mark.parametrize("C,W", [(64, 70), (128, 33)])
-def test_cam_and_pool(C, W, px, monkeypatch):
-  """Both CAM kernels: two pixels per thread (the default) and one (option cam_px = 1)."""
-  monkeypatch.setenv("PCLS_TEST_OPTS", "cam_px=%d" % px)
+def test_cam_and_pool(C, W):
+  """The CAM kernel (two pixels per thread) and the max-pool behind it."""
   rng = np.random.default_rng(C)
   B, H = 2, 11
   t = TinyNet(H, W)

@@ -202,7 +202,7 @@ def test_projection_darknet53_pipeline_full_scans():
 
 @pytest.mark.parametrize("C,W,B", [(64, 1024, 32), (128, 512, 32)])
 def test_cam_and_pool_at_benchmark_shapes(C, W, B):
-  """cam_kernel / maxpool3x3_s2_kernel at the benchmark's shapes and batch (the row-segment count on blockIdx.z / .y
+  """cam2_kernel / maxpool3x3_s2_kernel at the benchmark's shapes and batch (the row-segment count on blockIdx.z / .y
   follows from the batch): CAM(64) at W = 1024 and CAM(128) at W = 512, H = 64, batch 32; frames 0 and B-1 vs the oracle."""
   from pclsegmentation_b200.nets import layers as L
   from tests.test_gpu_nets import TinyNet, _check_cam, _input, _nchw, _nhwc, _rand_vars, _tp
