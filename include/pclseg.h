@@ -221,6 +221,8 @@ void pcls_net_destroy(pcls_net* net);
  * is_logits = 1 declares the float32 logits tensor [B,H,width,channels]. */
 int pcls_net_tensor(pcls_net* net, int width, int channels, int is_logits);
 
+/* Adds a convolution.  Into a 16-bit (non-logits) tensor, out_channel_offset and cout must be multiples of 8, like the
+ * channel count of every 16-bit tensor: outputs are written as whole 8-channel vectors.  Otherwise PCLS_ERR_INVALID. */
 int pcls_net_conv(pcls_net* net, const pcls_conv_desc* desc);
 
 /* tf.nn.max_pool2d(ksize=3, strides=[1,2], padding='SAME') (SqueezeSegV2.py:295,301,305). */

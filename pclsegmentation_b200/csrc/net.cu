@@ -95,6 +95,8 @@ int Net::add_conv(const pcls_conv_desc& d) {
                d.out_channel_offset + d.cout, to.channels);
   PCLS_REQUIRE((d.out_is_logits != 0) == to.logits, "pcls_net_conv: out_is_logits does not match the output tensor");
   PCLS_REQUIRE(to.logits || d.out_channel_offset % 8 == 0, "pcls_net_conv: channel offset must be a multiple of 8");
+  // the 16-bit epilogues store whole 8-channel (16-byte) vectors: a slice that ends inside one would be left unwritten
+  PCLS_REQUIRE(to.logits || d.cout % 8 == 0, "pcls_net_conv: cout %d must be a multiple of 8", d.cout);
   int wout = ti.width;
   if (L.p.mode == MODE_3x3_S2) wout = (ti.width + 1) / 2;
   if (L.p.mode == MODE_DECONV) wout = ti.width * 2;
