@@ -102,6 +102,38 @@ int pcls_project_resolve_net_input(const float* points, const int64_t* offsets, 
                                    const uint64_t* keys, const double* h_mean5, const double* h_std5, int precision,
                                    void* input8, uint8_t* mask, int32_t* proj_idx, pcls_stream stream);
 
+/* Per-point labels from the range-image predictions (no reference call site: the reference stops at [H,W]
+ * predictions, inference.py:78).  A k-NN vote in a search x search window of the range image, neighbours ranked by
+ * range difference (the post-processing published with RangeNet++), so that a point that lost its pixel to a nearer
+ * point does not simply take that point's label.
+ *   preds        [B,H,W] i32   the forward's predictions, each in [0, num_classes)
+ *   keys         [B,H,W] u64   winner keys left by pcls_project_scatter (either variant; ~0 = empty pixel)
+ *   offsets      [B+1]  i64;  proj_x, proj_y [total] i32, unproj_range [total] f32 from the same scatter
+ *   search       odd window size 1..9; 1 = plain back-projection (the label of the point's own pixel)
+ *   k            1 <= k <= min(search*search, 32)
+ *   h_window_weights  host f32 [search*search] (row-major, centre at search*search/2), finite and >= 0, or NULL = all 1
+ *   cutoff       neighbours with weighted distance > cutoff do not vote; <= 0 = no cutoff
+ *   ignore_class votes for this class are not counted; -1 = none
+ *   pixel_scratch [B,H,W] u64 caller-provided when search > 1 (may be NULL when search == 1)
+ *   point_labels [total] i32 out.  num_classes <= 32, 0 <= none_index < num_classes.
+ * Rules (all deterministic): a dropped point (proj_x < 0) gets none_index.  Point i of scan b at pixel (r, c) with range
+ * rho; window entry j = (dy+p)*search + (dx+p), p = (search-1)/2.  An entry outside the image (no column wrap-around) or
+ * on an empty pixel is invalid.  A valid entry's range rho_j is unproj_range[offsets[b] + (key & 0xffffffff)] (the
+ * centre entry uses rho itself) and its label preds[b, r+dy, c+dx].  d_j = |rho_j - rho| * w_j in float32 (separate
+ * roundings).  The k valid entries with the smallest d_j are selected (ties: lower j; all of them if fewer than k); an
+ * entry votes if d_j <= cutoff (or cutoff <= 0) and its label is not ignore_class.  The label is the class with the most
+ * votes, ties to the lowest class; with no votes, the centre pixel's prediction. */
+int pcls_point_labels(const int32_t* preds, const uint64_t* keys, const int64_t* offsets, int B, int H, int W,
+                      int64_t total_points, const int32_t* proj_x, const int32_t* proj_y, const float* unproj_range,
+                      int num_classes, int none_index, int search, int k, const float* h_window_weights,
+                      float cutoff, int ignore_class, uint64_t* pixel_scratch, int32_t* point_labels,
+                      pcls_stream stream);
+
+/* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
+ * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
+int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,
+                    pcls_stream stream);
+
 /* =====================================================================================
  * Segmentation head, input stage, confusion matrix
  * ===================================================================================== */

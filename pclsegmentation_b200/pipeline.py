@@ -1,7 +1,9 @@
 """Device-resident pipelines over the C-ABI kernels:
 
 * ``ScanSegmenter``  raw scans -> spherical projection -> network forward -> labels (BASELINE config 4: the converter's
-  per-scan loop dataset_convert/semantic_kitti.py:152-179 fused with inference.py:44-78; range images never leave HBM)
+  per-scan loop dataset_convert/semantic_kitti.py:152-179 fused with inference.py:44-78; range images never leave HBM),
+  optionally one label per point (pcls_point_labels: back-projection or the k-NN vote of ``KNN``)
+* ``ScanEvaluator``  point-wise evaluation on raw scans: scans -> point labels -> confusion update per point
 * ``Evaluator``      the eval.py hot loop (eval.py:45-50): forward -> head -> confusion update per batch on this rank's
   shard of the frames, one all-reduce of the int64 matrix at the end, then IoU / recall / precision / mIoU.
 """
@@ -18,6 +20,27 @@ from .sharding import Communicator, shard_range
 from .utils.util import confusion_matrix_to_iou_recall_precision
 
 
+class KNN:
+  """Parameters of the k-NN vote that turns range-image predictions into per-point labels (pcls_point_labels).  The
+  defaults are the post-processing settings published with RangeNet++ (window 5, k 5, sigma 1, cutoff 1 m, the
+  unlabeled class ignored); ``ignore_class="none"`` resolves to the config's "None" class, an int is taken as is (-1 =
+  count every class).  The window weights are 1 - g / sum(g), g = exp(-(dx^2 + dy^2) / (2 sigma^2)), computed in float64
+  and rounded once to float32."""
+
+  def __init__(self, search=5, k=5, sigma=1.0, cutoff=1.0, ignore_class="none"):
+    self.search, self.k, self.sigma, self.cutoff, self.ignore_class = int(search), int(k), float(sigma), float(cutoff), \
+        ignore_class
+
+  def weights(self):
+    p = (self.search - 1) // 2
+    dy, dx = np.mgrid[-p:p + 1, -p:p + 1].astype(np.float64)
+    g = np.exp(-(dx * dx + dy * dy) / (2.0 * self.sigma ** 2))
+    return (1.0 - g / g.sum()).reshape(-1).astype(np.float32)
+
+  def ignore_index(self, mc):
+    return mc.CLASSES.index("None") if self.ignore_class == "none" else int(self.ignore_class)
+
+
 class ScanSegmenter:
   def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None):
     mc = model.mc
@@ -25,30 +48,43 @@ class ScanSegmenter:
     self.projector = SphericalProjector(mc.ZENITH_LEVEL, mc.AZIMUTH_LEVEL, fov_up, fov_down, label_lut=label_lut)
 
   def segment_device(self, points, offsets, labels=None, want_probabilities=False, out=None, want_image=False,
-                     want_logits=False):
+                     want_logits=False, want_point_labels=False, knn=None):
     """points [total,4] float32 CUDA (x,y,z,remission), offsets [B+1] int64 CUDA -> dict(predictions, proj_idx,
-    probabilities?, logits?, image?) - keys and activations stay on the device.
+    probabilities?, logits?, image?, point_labels?) - keys and activations stay on the device.
 
     Default (no image, no labels wanted): the resolve pass writes the NORMALISED 16-bit network input and the mask
     straight into the net's own buffers (pcls_project_resolve_net_input): no float32 [B,H,W,6] range image is written
     and read back, and the forward runs without its input kernel.  With want_image / labels the range image is
-    materialised (the converters' output) and the forward reads it."""
+    materialised (the converters' output) and the forward reads it.
+
+    want_point_labels: also one label per point, ``point_labels`` [total] int32 CUDA (pcls_point_labels on the same
+    stream after the forward): with ``knn=None`` each point takes its pixel's prediction, with a ``KNN`` the k-NN vote
+    decides; points the projection dropped get the "None" class."""
     B = int(offsets.numel()) - 1
     if want_image or labels is not None or B > self._staged_capacity(B):
-      proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0)
+      proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0, want_point_outputs=want_point_labels)
       res = self.model.forward_device(proj["image"], None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD,
                                       want_probabilities=want_probabilities, want_logits=want_logits, out=out)
       res.update(image=proj["image"], proj_idx=proj["proj_idx"])
+      if want_point_labels:
+        res["point_labels"] = self._point_labels(res["predictions"], proj["keys"], offsets, proj["proj_x"],
+                                                 proj["proj_y"], proj["unproj_range"], knn)
       return res
     lib = _lib.load()
     H, W = self.projector.H, self.projector.W
     inp, msk, _ = self.model.input_buffers(B)
     keys = torch.empty((B, H, W), dtype=torch.int64, device=points.device)
     idx = torch.empty((B, H, W), dtype=torch.int32, device=points.device)
+    px = py = ur = None
+    if want_point_labels:
+      total = int(points.shape[0])
+      px = torch.empty(total, dtype=torch.int32, device=points.device)
+      py = torch.empty(total, dtype=torch.int32, device=points.device)
+      ur = torch.empty(total, dtype=torch.float32, device=points.device)
     s = stream_handle()
     _lib.check(lib.pcls_project_scatter(ptr(points), None, ptr(offsets), B, int(points.shape[0]), H, W,
-                                        float(self.projector.fov_up), float(self.projector.fov_down), ptr(keys), None, None,
-                                        None, s), "pcls_project_scatter")
+                                        float(self.projector.fov_up), float(self.projector.fov_down), ptr(keys), ptr(px),
+                                        ptr(py), ptr(ur), s), "pcls_project_scatter")
     mean = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_MEAN, np.float64).reshape(-1))
     std = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_STD, np.float64).reshape(-1))
     _lib.check(lib.pcls_project_resolve_net_input(ptr(points), ptr(offsets), B, H, W, ptr(keys), mean, std,
@@ -56,7 +92,26 @@ class ScanSegmenter:
                "pcls_project_resolve_net_input")
     res = self.model.forward_staged(B, want_probabilities=want_probabilities, want_logits=want_logits, out=out)
     res.update(proj_idx=idx)
+    if want_point_labels:
+      res["point_labels"] = self._point_labels(res["predictions"], keys, offsets, px, py, ur, knn)
     return res
+
+  def _point_labels(self, preds, keys, offsets, px, py, ur, knn):
+    B, H, W = preds.shape
+    total = int(px.numel())
+    out = torch.empty(total, dtype=torch.int32, device=preds.device)
+    search, k, w, cutoff, ignore, scratch = 1, 1, None, 0.0, -1, None
+    if knn is not None:
+      search, k, cutoff, ignore = knn.search, knn.k, knn.cutoff, knn.ignore_index(self.mc)
+      wt = knn.weights()
+      w = (ctypes.c_float * wt.size)(*wt.tolist())
+      if search > 1:
+        scratch = torch.empty((B, H, W), dtype=torch.int64, device=preds.device)
+    _lib.check(_lib.load().pcls_point_labels(ptr(preds), ptr(keys), ptr(offsets), B, H, W, total, ptr(px), ptr(py),
+                                             ptr(ur), self.mc.NUM_CLASS, self.mc.CLASSES.index("None"), search, k, w,
+                                             float(cutoff), ignore, ptr(scratch), ptr(out), stream_handle()),
+               "pcls_point_labels")
+    return out
 
   def _staged_capacity(self, B):
     return self.model.input_buffers(B)[2]
@@ -74,8 +129,15 @@ class ScanSegmenter:
     return self.segment_device(pts, offsets, labels=lab, **kw)
 
   def point_labels(self, res, points_per_scan):
-    """Back-projects the per-pixel predictions to the points (each point takes the label of its pixel)."""
-    raise NotImplementedError("per-point label back-projection is not part of the reference path")
+    """The ``point_labels`` of a ``segment_device(..., want_point_labels=True)`` result as one int32 numpy array per
+    scan (lengths ``points_per_scan``)."""
+    if "point_labels" not in res:
+      raise ValueError("the result holds no point labels: segment with want_point_labels=True")
+    lab = res["point_labels"].cpu().numpy()
+    sizes = [int(n) for n in points_per_scan]
+    if sum(sizes) != lab.shape[0]:
+      raise ValueError("points_per_scan sums to %d, the result has %d point labels" % (sum(sizes), lab.shape[0]))
+    return np.split(lab, np.cumsum(sizes)[:-1])
 
 
 class Evaluator:
@@ -112,6 +174,44 @@ class Evaluator:
     iou, recall, precision = confusion_matrix_to_iou_recall_precision(cm)
     return dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
                 miou=float(self.miou_tracker.result()))
+
+
+class ScanEvaluator:
+  """Point-wise evaluation on raw scans (single GPU): per batch projection -> forward -> per-point labels (``knn``:
+  a ``KNN`` or None for the plain back-projection) -> ground truth ``label_lut[word & 0xFFFF]`` (pcls_map_labels; the raw
+  semantic id without a LUT) -> confusion update over the points.  ``finish()`` gives the report of
+  ``Evaluator.finish``."""
+
+  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None):
+    self.seg = ScanSegmenter(model, fov_up, fov_down)
+    self.mc, self.knn = model.mc, knn
+    self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
+    self.lut = None
+    if label_lut is not None:
+      self.lut = torch.as_tensor(np.asarray(label_lut, dtype=np.int32)).to(self.seg.projector._dev)
+
+  def update(self, batch):
+    """batch: the dict ``dataset_convert.ScanBatchLoader.load`` returns, with labels.  Returns the segment_device result
+    (``point_labels`` included) and the per-point ground truth ``gt`` [total] int32 CUDA."""
+    if batch.get("labels") is None:
+      raise ValueError("point-wise evaluation needs the label files")
+    res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn)
+    n = int(batch["points"].shape[0])
+    gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
+    lut = self.lut
+    _lib.check(_lib.load().pcls_map_labels(ptr(batch["labels"]), n, ptr(lut), int(lut.numel()) if lut is not None else 0,
+                                           ptr(gt), stream_handle()), "pcls_map_labels")
+    self.miou_tracker.update_state(gt, res["point_labels"])
+    res["gt"] = gt
+    return res
+
+  def finish(self):
+    """The report of ``Evaluator.finish`` plus ``dropped``: points whose ground truth is not a class id (a raw semantic
+    id with no LUT, e.g. KITTI's 10 / 40 / 252); they are not in the matrix."""
+    cm = self.miou_tracker.total_cm
+    iou, recall, precision = confusion_matrix_to_iou_recall_precision(cm)
+    return dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
+                miou=float(self.miou_tracker.result()), dropped=self.miou_tracker.dropped)
 
 
 def shard_files(files, comm=None):
