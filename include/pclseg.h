@@ -280,7 +280,10 @@ int pcls_net_finalize(pcls_net* net, int logits_tensor, int num_classes, int non
  *            reference input (inference.py:56-62), channel 5 = mask.  channels == 5 or 6 with
  *            h_mean5/h_std5 given: RAW x,y,z,i,d(,label) - the input stage (inference.py:50-62) is
  *            fused into the load (mask = depth > 0).
- *   mask     [B,H,W] u8 (the reference's lidar_mask) or NULL = derive (channel 5 != 0, or depth > 0 for raw input)
+ *   mask     [B,H,W] u8 (the reference's lidar_mask) or NULL = derive: channel 5 != +-0 after its rounding to the
+ *            storage type (so a float32 channel 5 that rounds to a 16-bit zero is an empty pixel, NaN a valid one), or
+ *            depth > 0 for raw input.  For raw input a given mask sets only which pixels are valid (the head's
+ *            none_index); tensor 0's channel 5 and the zeroed channels still follow depth > 0.
  *   logits   [B,H,W,NC] f32 or NULL;  probs [B,H,W,NC] f32 or NULL;  preds [B,H,W] i32 (required)
  * B <= max_batch. */
 int pcls_net_forward(pcls_net* net, const float* lidar, int channels, const uint8_t* mask,
@@ -291,7 +294,7 @@ int pcls_net_forward(pcls_net* net, const float* lidar, int channels, const uint
  * in the net's storage type (IEEE half for PCLS_F16, bfloat16 for PCLS_BF16), [B,H,W,6] (5 channels + mask channel) or
  * [B,H,W,8] (tensor 0's own layout, channels 6-7 ignored).  The host ships 12 / 16 bytes per pixel instead of 24; the
  * results are bit-identical to pcls_net_forward on the float32 input these values were rounded from.
- *   mask  [B,H,W] u8 or NULL = derive (channel 5 != 0). */
+ *   mask  [B,H,W] u8 or NULL = derive (channel 5 != +-0; NaN is valid). */
 int pcls_net_forward_in16(pcls_net* net, const void* lidar16, int channels, const uint8_t* mask, int B,
                           float* logits, float* probs, int32_t* preds, pcls_stream stream);
 

@@ -161,7 +161,10 @@ net_input_kernel(const float* __restrict__ lidar, int channels, const uint8_t* _
       if (mask_in) m = mask_in[p] != 0;
     } else {    // already normalised 6-channel reference input; channel 5 is the mask
       f[5] = __ldg(s + 5);
-      m = mask_in ? (mask_in[p] != 0) : (f[5] != 0.0f);
+      // a derived mask follows channel 5 as tensor 0 stores it (16 bits, != +-0), like net_input16_kernel: a float32
+      // value that rounds to a 16-bit zero (1e-8 in fp16) is an empty pixel in both, and NaN a valid one
+      const T m5 = from_f32<T>(f[5]);
+      m = mask_in ? (mask_in[p] != 0) : (*reinterpret_cast<const uint16_t*>(&m5) & 0x7FFFu) != 0;
     }
     f[6] = 0.0f; f[7] = 0.0f;
     reinterpret_cast<int4*>(out8)[p] = pack8<T>(f);

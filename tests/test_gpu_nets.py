@@ -143,27 +143,6 @@ def _check_layer(x_dev, y_dev, p, conv, bn=None, strides=(1, 1), act=None, trans
   return worst
 
 
-def _check_cam(x_dev, y_dev, p, name, what=""):
-  """CAM (nets/SqueezeSegV2.py:66-70) at its own output, float64 on the device's own 16-bit input, with the error the
-  kernel's arithmetic allows: the 7x7 max is exact; squeeze / excitation weights and the hidden vector are fp16
-  (2^-11 each), the gate's slope is <= 1/4, the gated output is rounded to fp16 once."""
-  k1, b1 = _fold64(p, name + "/squeeze", name + "/squeeze_bn")
-  k2, b2 = _fold64(p, name + "/excitation", name + "/excitation_bn")
-  x = _nchw(x_dev).double()
-  pool = O.max_pool_same(x, 7, (1, 1))
-  pre = O.conv2d_same(pool, k1, b1)
-  s = torch.relu(pre)
-  e = O.conv2d_same(s, k2, b2)
-  y = x * torch.sigmoid(e)
-  ds = U16 * (1.5 * O.conv2d_same(pool.abs(), k1.abs(), b1.abs()) + s)
-  de = O.conv2d_same(ds, k2.abs()) + U16 * 1.5 * O.conv2d_same(s, k2.abs(), b2.abs())
-  bound = x.abs() * 0.25 * de + U16 * y.abs() + 1e-6
-  d = (_nchw(y_dev).double() - y).abs()
-  worst = float((d / bound).max())
-  assert worst <= 1.0, "%s: CAM error %.3g x the error model (max abs err %.3e)" % (what, worst, float(d.max()))
-  return worst
-
-
 @pytest.mark.parametrize("impl", IMPLS)
 @pytest.mark.parametrize("H,W,c1,c2", [(5, 48, 32, 48), (3, 27, 16, 64), (8, 256, 64, 128), (2, 130, 128, 32)])
 def test_conv_flavours_in_isolation(impl, H, W, c1, c2):
@@ -250,25 +229,6 @@ def test_residual_and_skip_adds(impl):
   _check_layer(xin, ya, p, "c0", "b0", act="leaky", what="conv1")
   _check_layer(ya, ys, p, "c1", "b1", act="leaky", what="block 1x1")
   _check_layer(ys, got, p, "c2", "b2", act="leaky", residuals=[ys, ya], what="block 3x3 + residual + skip")
-
-
-@pytest.mark.parametrize("C,W", [(64, 70), (128, 33)])
-def test_cam_and_pool(C, W):
-  """The CAM kernel (two pixels per thread) and the max-pool behind it."""
-  rng = np.random.default_rng(C)
-  B, H = 2, 11
-  t = TinyNet(H, W)
-  g = t.g
-  a = L.relu(L.BatchNormalization("b0")(L.Conv2D("c0", C, 3)(g.input)))
-  cam = g.cam(a, "cam", C // 16)
-  pooled = L.max_pool2d(cam)
-  _rand_vars(g, rng)
-  x = _input(rng, B, H, W)
-  p = _tp(g)
-  got = t.run(pooled, B, x, 1, keep=[a, cam])
-  ya, ycam = t.kept
-  _check_cam(ya, ycam, p, "cam", "C %d W %d" % (C, W))
-  assert np.array_equal(got, _nhwc(O.max_pool_same(_nchw(ycam), 3, (1, 2))))   # the max-pool is exact on its own input
 
 
 @pytest.mark.parametrize("C,S,W,H", [(64, 16, 256, 3), (64, 16, 70, 5), (128, 16, 33, 4), (256, 32, 14, 3), (128, 16, 15, 2)])

@@ -199,30 +199,3 @@ def test_projection_darknet53_pipeline_full_scans():
   assert err <= LOGIT_TOL, err
   assert agree >= 0.9985, agree      # Darknet53, random-init weights: see the note above CASES (measured 99.88 - 99.91 %)
 
-
-@pytest.mark.parametrize("C,W,B", [(64, 1024, 32), (128, 512, 32)])
-def test_cam_and_pool_at_benchmark_shapes(C, W, B):
-  """cam2_kernel / maxpool3x3_s2_kernel at the benchmark's shapes and batch (the row-segment count on blockIdx.z / .y
-  follows from the batch): CAM(64) at W = 1024 and CAM(128) at W = 512, H = 64, batch 32; frames 0 and B-1 vs the oracle."""
-  from pclsegmentation_b200.nets import layers as L
-  from tests.test_gpu_nets import TinyNet, _check_cam, _input, _nchw, _nhwc, _rand_vars, _tp
-  rng = np.random.default_rng(C + W)
-  H = 64
-  t = TinyNet(H, 2 * W)
-  g = t.g
-  a = L.relu(L.BatchNormalization("b0")(L.Conv2D("c0", C, 3, strides=[1, 2])(g.input)))
-  cam = g.cam(a, "cam", C // 16)
-  pooled = L.max_pool2d(cam)
-  _rand_vars(g, rng)
-  x = _input(rng, B, H, 2 * W)
-  p = _tp(g)
-  fr = [0, B - 1]
-  got = t.run(pooled, B, x, 0, keep=[a, cam])
-  ya, ycam = t.kept[0][fr], t.kept[1][fr]
-  _check_cam(ya, ycam, p, "cam", "C %d W %d B %d" % (C, W, B))
-  # the pool is exact on the device's own CAM output
-  assert np.array_equal(got[fr], _nhwc(O.max_pool_same(_nchw(ycam), 3, (1, 2))))
-  # and the chain agrees with the oracle's chain to a few fp16 roundings (conv c0 output, gate, product)
-  xa = torch.relu(O.batch_norm(O._conv(_nchw(x[fr]), p, "c0", (1, 2)), p, "b0"))
-  ref_cam = _nhwc(O.cam(xa, p, "cam"))
-  assert np.abs(ycam - ref_cam).max() <= 4e-3 * max(1.0, float(np.abs(ref_cam).max()))
