@@ -134,6 +134,26 @@ int pcls_point_labels(const int32_t* preds, const uint64_t* keys, const int64_t*
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,
                     pcls_stream stream);
 
+/* Per-frame statistics of range images [B,H,W,channels] (x, y, z, remission, range[, label]): the moments a config's
+ * INPUT_MEAN / INPUT_STD come from, channel ranges, occupancy and class counts (the reference computes them offline with
+ * numpy, preprocessing/inspect_training_data.py; the rules below are this project's, bit parity with its RunningStd is
+ * not claimed).
+ *   frames       dtype 0 = float32, 1 = float64 (the converters' .npy files, read without narrowing)
+ *   channels     5 or 6;  h_shift5 host doubles (s_c) or NULL (= 0), finite
+ *   frame_sums   [B,5,4] f64 OUT, per frame and channel: sum(d), sum(d*d), min(x), max(x), d = x - s_c,
+ *                over the frame's VALID pixels (valid = range channel > 0 on the stored value; NaN is invalid).  A NaN
+ *                value at a valid pixel enters the sums but not min / max.  A frame with no valid pixel gets sums of 0,
+ *                min = +inf, max = -inf.  The summation order depends only on H, W and channels: a frame's row is the
+ *                same bits whatever B is and wherever the frame sits in the batch.
+ *   frame_valid  [B] i64 OUT: valid pixels per frame
+ *   row_valid [H], col_valid [W], class_pixels [num_classes], dropped [1]: i64, ACCUMULATED, each may be NULL;
+ *                class_pixels counts the label channel at valid pixels, truncated toward zero like pcls_input_stage's
+ *                (int32_t) cast; a label that is not finite or not in [0, num_classes) increments *dropped
+ *                (class_pixels / dropped need channels == 6 and 1 <= num_classes <= 32).  H, W <= 16384. */
+int pcls_dataset_stats(const void* frames, int dtype, int channels, int B, int H, int W, const double* h_shift5,
+                       int num_classes, double* frame_sums, int64_t* frame_valid, int64_t* row_valid,
+                       int64_t* col_valid, int64_t* class_pixels, int64_t* dropped, pcls_stream stream);
+
 /* =====================================================================================
  * Segmentation head, input stage, confusion matrix
  * ===================================================================================== */

@@ -45,6 +45,8 @@ SIGNATURES = {
                                 c_int, c_int, c_int, c_int, POINTER(c_float), c_float, c_int, c_void_p, c_void_p,
                                 c_void_p]),
   "pcls_map_labels": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
+  "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
+                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
   "pcls_net_input_buffers": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int)]),
   "pcls_head": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
   "pcls_cast_f64_f32": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
