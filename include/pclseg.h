@@ -129,6 +129,38 @@ int pcls_point_labels(const int32_t* preds, const uint64_t* keys, const int64_t*
                       float cutoff, int ignore_class, uint64_t* pixel_scratch, int32_t* point_labels,
                       pcls_stream stream);
 
+/* Instance ids for thing-class points (no reference call site: the reference reads instance ids, SemLaserScan.set_label
+ * inst = label >> 16, but never produces them): connected components in the range image.  The rules are this project's;
+ * bit parity with any published clustering code is not claimed.
+ *   points       [total,4] f32 (16-byte aligned), keys [B,H,W] u64, offsets, proj_x, proj_y: pcls_project_scatter's
+ *                (either variant: the key's low word is the winner's local index)
+ *   point_labels [total] i32 L, e.g. from pcls_point_labels;  thing_mask: bit c set = class c is a thing class
+ *                (1 <= num_classes <= 32, no bit at or above num_classes; labels outside [0, num_classes) are never things)
+ *   scratch      caller-provided, 16-byte aligned, pcls_point_instances_scratch_bytes(B, H, W) bytes
+ *   instances    [total] i32 out;  instance_counts [B] i32 out: the number of ids in each scan
+ * Rules, per scan b:
+ *   1. A node is a pixel (r, c) whose winner point i (offsets[b] + low word of the key) has L[i] in the thing set.
+ *   2. Nodes u and v are joined when |r_u - r_v| <= ry; the column distance is <= rx (modulo W with wrap = 1, because a
+ *      360-degree scan's columns 0 and W-1 are neighbours; no wrap-around with wrap = 0); L is equal at the two nodes; and
+ *      d^2 <= tau^2, d^2 = (dx*dx + dy*dy) + dz*dz in float32 with separate roundings over the two winners' x, y, z,
+ *      tau^2 = fl32(tau * tau).
+ *   3. Components are the connected components of that graph.
+ *   4. A node's winner belongs to the node's component.  A non-winner point j whose pixel is a node belongs to that
+ *      component when L[j] equals the winner's label and d^2(j, winner) <= tau^2.  Every other point (stuff classes,
+ *      dropped points with proj_x < 0, occluded points that fail the test) belongs to no component.
+ *   5. A component's size is the number of points that belong to it.  Components with size >= min_points are numbered
+ *      1, 2, ... per scan in increasing order of their smallest pixel index r*W + c; every other point gets 0.
+ *   6. 0 <= ry <= 4, 0 <= rx <= 8, ry + rx > 0, 2 rx < W when wrapping, tau finite and > 0, min_points >= 1,
+ *      B*H*W < 2^31; otherwise PCLS_ERR_INVALID.
+ * The output is fully determined: the same bits on every run, whatever order the atomics land in.
+ * pcls_point_instances_scratch_bytes returns the bytes (24 per pixel), or PCLS_ERR_INVALID for bad sizes. */
+int64_t pcls_point_instances_scratch_bytes(int B, int H, int W);
+int pcls_point_instances(const float* points, const uint64_t* keys, const int64_t* offsets, int B, int H, int W,
+                         int64_t total_points, const int32_t* proj_x, const int32_t* proj_y,
+                         const int32_t* point_labels, int num_classes, uint32_t thing_mask, int ry, int rx, int wrap,
+                         float tau, int min_points, void* scratch, int32_t* instances, int32_t* instance_counts,
+                         pcls_stream stream);
+
 /* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
  * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,

@@ -44,6 +44,10 @@ SIGNATURES = {
   "pcls_point_labels": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p,
                                 c_int, c_int, c_int, c_int, POINTER(c_float), c_float, c_int, c_void_p, c_void_p,
                                 c_void_p]),
+  "pcls_point_instances_scratch_bytes": (c_int64, [c_int, c_int, c_int]),
+  "pcls_point_instances": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p,
+                                   c_void_p, c_int, c_uint32, c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p,
+                                   c_void_p, c_void_p]),
   "pcls_map_labels": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
   "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -93,3 +93,82 @@ class MeanIoU:
     self._cmw = None
 
   reset_state = reset_states
+
+
+class PanopticQuality:
+  """Panoptic quality over thing classes (Kirillov et al., "Panoptic Segmentation", CVPR 2019), point-wise per scan, on
+  the host (numpy; the caller hands over only the points that can be in a segment).  The rules are this project's; parity
+  with semantic-kitti-api's evaluation script is not claimed.
+
+  Per scan (``update``):
+  * points whose ground-truth class is ``ignore_class`` (the config's "None") are removed first;
+  * a ground-truth segment is the set of points of a thing class with equal (class, instance id), instance id > 0; one
+    with fewer than ``min_gt_points`` points is ignored: it counts as neither TP nor FN;
+  * a predicted segment is the set of points of a thing class with equal (class, instance id), instance id > 0;
+  * a predicted and a ground-truth segment of the same class match when their IoU is > 0.5 (strictly); a match with a
+    counted ground-truth segment is a TP, an unmatched counted ground-truth segment a FN, an unmatched predicted segment
+    a FP unless more than half of its points lie in ignored ground-truth segments of its class.
+  ``result()``: per thing class PQ = sum(IoU of TPs) / (TP + FP / 2 + FN / 2), SQ = sum(IoU) / TP (0 without TPs),
+  RQ = TP / (TP + FP / 2 + FN / 2), and their means over the classes with at least one counted segment."""
+
+  def __init__(self, num_classes, thing_classes, ignore_class=None, min_gt_points=50):
+    self.num_classes = int(num_classes)
+    self.thing_classes = sorted(int(c) for c in thing_classes)
+    self.ignore_class = -1 if ignore_class is None else int(ignore_class)
+    self.min_gt_points = int(min_gt_points)
+    self._thing = np.zeros(self.num_classes + 1, bool)      # the last entry: any id outside [0, num_classes)
+    self._thing[self.thing_classes] = True
+    self.reset_states()
+
+  def reset_states(self):
+    self.tp = np.zeros(self.num_classes, np.int64)
+    self.fp = np.zeros(self.num_classes, np.int64)
+    self.fn = np.zeros(self.num_classes, np.int64)
+    self.iou_sum = np.zeros(self.num_classes, np.float64)
+
+  def _segments(self, cls, inst):
+    ok = self._thing[np.where((cls >= 0) & (cls < self.num_classes), cls, self.num_classes)] & (inst > 0)
+    key = cls * (1 << 32) + inst
+    seg = np.full(cls.shape[0], -1, np.int64)
+    uniq, inv, size = np.unique(key[ok], return_inverse=True, return_counts=True)
+    seg[ok] = inv.reshape(-1)
+    return seg, uniq >> 32, size
+
+  def update(self, gt_class, gt_inst, pred_class, pred_inst):
+    """One scan: per point the ground-truth class and instance id, the predicted class and instance id (any integer
+    arrays of one length)."""
+    gc, gi, pc, pi = (np.asarray(a, np.int64).reshape(-1) for a in (gt_class, gt_inst, pred_class, pred_inst))
+    keep = gc != self.ignore_class
+    gc, gi, pc, pi = gc[keep], gi[keep], pc[keep], pi[keep]
+    gseg, gcls, gsize = self._segments(gc, gi)
+    pseg, pcls, psize = self._segments(pc, pi)
+    both = (gseg >= 0) & (pseg >= 0) & (gc == pc)
+    pair, inter = np.unique(gseg[both] * max(psize.size, 1) + pseg[both], return_counts=True)
+    g, p = pair // max(psize.size, 1), pair % max(psize.size, 1)
+    iou = inter / (gsize[g] + psize[p] - inter).astype(np.float64)
+    counted = gsize >= self.min_gt_points
+    tp = (iou > 0.5) & counted[g]
+    matched_g = np.zeros(gsize.size, bool)
+    matched_g[g[tp]] = True
+    matched_p = np.zeros(psize.size, bool)
+    matched_p[p[tp]] = True
+    in_ignored = np.bincount(p[~counted[g]], weights=inter[~counted[g]], minlength=psize.size)
+    fp = ~matched_p & ~(in_ignored > 0.5 * psize)
+    np.add.at(self.tp, gcls[g[tp]], 1)
+    np.add.at(self.iou_sum, gcls[g[tp]], iou[tp])
+    np.add.at(self.fn, gcls[counted & ~matched_g], 1)
+    np.add.at(self.fp, pcls[fp], 1)
+
+  def result(self):
+    """dict(classes, pq, sq, rq, tp, fp, fn: per thing class, counted: which have a counted segment, pq_mean, sq_mean,
+    rq_mean over the counted classes, 0 if none)."""
+    c = np.asarray(self.thing_classes, np.int64)
+    tp, fp, fn, s = self.tp[c], self.fp[c], self.fn[c], self.iou_sum[c]
+    den = tp + 0.5 * fp + 0.5 * fn
+    counted = den > 0
+    pq = np.divide(s, den, out=np.zeros(c.size), where=counted)
+    rq = np.divide(tp.astype(np.float64), den, out=np.zeros(c.size), where=counted)
+    sq = np.divide(s, tp.astype(np.float64), out=np.zeros(c.size), where=tp > 0)
+    mean = (lambda v: float(v[counted].mean()) if counted.any() else 0.0)
+    return dict(classes=c, pq=pq, sq=sq, rq=rq, tp=tp, fp=fp, fn=fn, counted=counted, pq_mean=mean(pq),
+                sq_mean=mean(sq), rq_mean=mean(rq))

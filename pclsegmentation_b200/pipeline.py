@@ -2,8 +2,10 @@
 
 * ``ScanSegmenter``  raw scans -> spherical projection -> network forward -> labels (BASELINE config 4: the converter's
   per-scan loop dataset_convert/semantic_kitti.py:152-179 fused with inference.py:44-78; range images never leave HBM),
-  optionally one label per point (pcls_point_labels: back-projection or the k-NN vote of ``KNN``)
-* ``ScanEvaluator``  point-wise evaluation on raw scans: scans -> point labels -> confusion update per point
+  optionally one label per point (pcls_point_labels: back-projection or the k-NN vote of ``KNN``) and an instance id
+  per thing-class point (pcls_point_instances: connected components of ``Clustering``)
+* ``ScanEvaluator``  point-wise evaluation on raw scans: scans -> point labels -> confusion update per point, and
+  panoptic quality (``metrics.PanopticQuality``) when instances are asked for
 * ``Evaluator``      the eval.py hot loop (eval.py:45-50): forward -> head -> confusion update per batch on this rank's
   shard of the frames, one all-reduce of the int64 matrix at the end, then IoU / recall / precision / mIoU.
 """
@@ -15,7 +17,7 @@ import torch
 from . import _lib
 from .device import ptr, samples_to_device, stream_handle, to_device
 from .laserscan import SphericalProjector
-from .metrics import MeanIoU
+from .metrics import MeanIoU, PanopticQuality
 from .sharding import Communicator, shard_range
 from .utils.util import confusion_matrix_to_iou_recall_precision
 
@@ -41,6 +43,41 @@ class KNN:
     return mc.CLASSES.index("None") if self.ignore_class == "none" else int(self.ignore_class)
 
 
+# Thing classes by name, for ``Clustering(thing_classes=None)``: SemanticKITTI's eight, and the ika / nuScenes configs'
+# road users.
+THING_CLASS_NAMES = ("car", "bicycle", "motorcycle", "truck", "other-vehicle", "person", "bicyclist", "motorcyclist",
+                     "Person", "Two-wheeler", "TwoWheeler", "Car", "Truck", "Bus")
+
+
+class Clustering:
+  """Parameters of the instance clustering of thing-class points (pcls_point_instances): pixels of the same thing
+  class within ``rows`` rows and ``cols`` columns of each other (a (2 rows + 1) x (2 cols + 1) window; columns wrap
+  around the 360-degree seam with ``wrap``) join when their points are at most ``tau`` metres apart; components with
+  fewer than ``min_points`` points get no id.  ``thing_classes`` is a list of class names or ids; None takes the
+  classes of ``THING_CLASS_NAMES`` that the config has.  The defaults (0.5 m, a 3 x 5 window, 10 points) are a
+  starting point: they have not been tuned against real scans."""
+
+  def __init__(self, tau=0.5, rows=1, cols=2, min_points=10, wrap=True, thing_classes=None):
+    self.tau, self.rows, self.cols, self.min_points, self.wrap = float(tau), int(rows), int(cols), int(min_points), \
+        bool(wrap)
+    self.thing_classes = thing_classes
+
+  def thing_ids(self, mc):
+    """The thing classes as sorted class ids of config ``mc``."""
+    if self.thing_classes is None:
+      ids = [i for i, n in enumerate(mc.CLASSES) if n in THING_CLASS_NAMES]
+      if not ids:
+        raise ValueError("no thing class of %s is in the config's classes; pass thing_classes" % (THING_CLASS_NAMES,))
+      return ids
+    ids = sorted({mc.CLASSES.index(c) if isinstance(c, str) else int(c) for c in self.thing_classes})
+    if ids and not 0 <= ids[0] <= ids[-1] < mc.NUM_CLASS:
+      raise ValueError("thing class ids %s are not all in [0, %d)" % (ids, mc.NUM_CLASS))
+    return ids
+
+  def thing_mask(self, mc):
+    return sum(1 << i for i in self.thing_ids(mc))
+
+
 class ScanSegmenter:
   def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None):
     mc = model.mc
@@ -48,7 +85,7 @@ class ScanSegmenter:
     self.projector = SphericalProjector(mc.ZENITH_LEVEL, mc.AZIMUTH_LEVEL, fov_up, fov_down, label_lut=label_lut)
 
   def segment_device(self, points, offsets, labels=None, want_probabilities=False, out=None, want_image=False,
-                     want_logits=False, want_point_labels=False, knn=None):
+                     want_logits=False, want_point_labels=False, knn=None, instances=None):
     """points [total,4] float32 CUDA (x,y,z,remission), offsets [B+1] int64 CUDA -> dict(predictions, proj_idx,
     probabilities?, logits?, image?, point_labels?) - keys and activations stay on the device.
 
@@ -59,7 +96,13 @@ class ScanSegmenter:
 
     want_point_labels: also one label per point, ``point_labels`` [total] int32 CUDA (pcls_point_labels on the same
     stream after the forward): with ``knn=None`` each point takes its pixel's prediction, with a ``KNN`` the k-NN vote
-    decides; points the projection dropped get the "None" class."""
+    decides; points the projection dropped get the "None" class.
+
+    instances: a ``Clustering`` - also ``instances`` [total] int32 (0 = no instance, ids 1, 2, ... per scan) and
+    ``instance_counts`` [B] int32 CUDA (pcls_point_instances on the same stream after the point labels); needs
+    want_point_labels."""
+    if instances is not None and not want_point_labels:
+      raise ValueError("instances need the point labels: segment with want_point_labels=True")
     B = int(offsets.numel()) - 1
     if want_image or labels is not None or B > self._staged_capacity(B):
       proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0, want_point_outputs=want_point_labels)
@@ -69,6 +112,9 @@ class ScanSegmenter:
       if want_point_labels:
         res["point_labels"] = self._point_labels(res["predictions"], proj["keys"], offsets, proj["proj_x"],
                                                  proj["proj_y"], proj["unproj_range"], knn)
+        if instances is not None:
+          res.update(self._instances(points, proj["keys"], offsets, proj["proj_x"], proj["proj_y"],
+                                     res["point_labels"], instances))
       return res
     lib = _lib.load()
     H, W = self.projector.H, self.projector.W
@@ -94,6 +140,8 @@ class ScanSegmenter:
     res.update(proj_idx=idx)
     if want_point_labels:
       res["point_labels"] = self._point_labels(res["predictions"], keys, offsets, px, py, ur, knn)
+      if instances is not None:
+        res.update(self._instances(points, keys, offsets, px, py, res["point_labels"], instances))
     return res
 
   def _point_labels(self, preds, keys, offsets, px, py, ur, knn):
@@ -112,6 +160,22 @@ class ScanSegmenter:
                                              float(cutoff), ignore, ptr(scratch), ptr(out), stream_handle()),
                "pcls_point_labels")
     return out
+
+  def _instances(self, points, keys, offsets, px, py, labels, clustering):
+    B, H, W = keys.shape
+    total = int(px.numel())
+    dev = keys.device
+    lib = _lib.load()
+    nbytes = _lib.check(lib.pcls_point_instances_scratch_bytes(B, H, W), "pcls_point_instances_scratch_bytes")
+    scratch = torch.empty(max(nbytes // 4, 4), dtype=torch.float32, device=dev)   # allocations are 256-byte aligned
+    inst = torch.empty(total, dtype=torch.int32, device=dev)
+    counts = torch.empty(B, dtype=torch.int32, device=dev)
+    _lib.check(lib.pcls_point_instances(ptr(points), ptr(keys), ptr(offsets), B, H, W, total, ptr(px), ptr(py),
+                                        ptr(labels), self.mc.NUM_CLASS, clustering.thing_mask(self.mc),
+                                        clustering.rows, clustering.cols, int(clustering.wrap), clustering.tau,
+                                        clustering.min_points, ptr(scratch), ptr(inst), ptr(counts), stream_handle()),
+               "pcls_point_instances")
+    return dict(instances=inst, instance_counts=counts)
 
   def _staged_capacity(self, B):
     return self.model.input_buffers(B)[2]
@@ -138,6 +202,22 @@ class ScanSegmenter:
     if sum(sizes) != lab.shape[0]:
       raise ValueError("points_per_scan sums to %d, the result has %d point labels" % (sum(sizes), lab.shape[0]))
     return np.split(lab, np.cumsum(sizes)[:-1])
+
+  def label_words(self, res, points_per_scan, inv_lut=None):
+    """SemanticKITTI ``.label`` words of a result, one uint32 numpy array per scan: ``(instance << 16) | sem`` with sem
+    = ``inv_lut[label]`` (e.g. the yaml's learning_map_inv as a LUT) or the class id, instance 0 when the result holds
+    no ``instances``.  Raises if an id does not fit in 16 bits."""
+    sems = self.point_labels(res, points_per_scan)
+    words = [(inv_lut[s] if inv_lut is not None else s).astype(np.uint32) for s in sems]
+    if any(int(w.max(initial=0)) > 0xFFFF for w in words):
+      raise ValueError("a semantic id does not fit in the lower 16 bits of a label word")
+    if "instances" not in res:
+      return words
+    inst = res["instances"].cpu().numpy()
+    if int(inst.max(initial=0)) > 0xFFFF:
+      raise ValueError("instance id %d does not fit in the upper 16 bits of a label word" % int(inst.max()))
+    parts = np.split(inst.astype(np.uint32), np.cumsum([int(n) for n in points_per_scan])[:-1])
+    return [(i << np.uint32(16)) | w for i, w in zip(parts, words)]
 
 
 class Evaluator:
@@ -180,12 +260,17 @@ class ScanEvaluator:
   """Point-wise evaluation on raw scans (single GPU): per batch projection -> forward -> per-point labels (``knn``:
   a ``KNN`` or None for the plain back-projection) -> ground truth ``label_lut[word & 0xFFFF]`` (pcls_map_labels; the raw
   semantic id without a LUT) -> confusion update over the points.  ``finish()`` gives the report of
-  ``Evaluator.finish``."""
+  ``Evaluator.finish``.  With ``instances`` (a ``Clustering``) each batch also gets instance ids and feeds a
+  ``PanopticQuality`` whose ground-truth instance id is the upper half of the label word (``word >> 16``); only the
+  points in a predicted or ground-truth thing segment come back to the host."""
 
-  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None):
+  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None):
     self.seg = ScanSegmenter(model, fov_up, fov_down)
-    self.mc, self.knn = model.mc, knn
+    self.mc, self.knn, self.instances = model.mc, knn, instances
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
+    self.pq = None
+    if instances is not None:
+      self.pq = PanopticQuality(self.mc.NUM_CLASS, instances.thing_ids(self.mc), self.mc.CLASSES.index("None"))
     self.lut = None
     if label_lut is not None:
       self.lut = torch.as_tensor(np.asarray(label_lut, dtype=np.int32)).to(self.seg.projector._dev)
@@ -195,7 +280,8 @@ class ScanEvaluator:
     (``point_labels`` included) and the per-point ground truth ``gt`` [total] int32 CUDA."""
     if batch.get("labels") is None:
       raise ValueError("point-wise evaluation needs the label files")
-    res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn)
+    res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn,
+                                  instances=self.instances)
     n = int(batch["points"].shape[0])
     gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
     lut = self.lut
@@ -203,15 +289,38 @@ class ScanEvaluator:
                                            ptr(gt), stream_handle()), "pcls_map_labels")
     self.miou_tracker.update_state(gt, res["point_labels"])
     res["gt"] = gt
+    if self.pq is not None:
+      self._update_pq(batch, gt, res)
     return res
+
+  def _update_pq(self, batch, gt, res):
+    """Feeds ``self.pq`` scan by scan with the points that can be in a segment: a predicted instance, or a ground-truth
+    thing point with an instance id; points of the "None" class are left out (the metric removes them anyway)."""
+    dev = gt.device
+    gt_inst = (batch["labels"] >> 16) & 0xFFFF
+    thing = torch.zeros(self.mc.NUM_CLASS + 1, dtype=torch.bool, device=dev)
+    thing[torch.as_tensor(self.pq.thing_classes, dtype=torch.long, device=dev)] = True
+    gcls = torch.where((gt >= 0) & (gt < self.mc.NUM_CLASS), gt, self.mc.NUM_CLASS).long()
+    keep = (gt != self.pq.ignore_class) & ((res["instances"] > 0) | (thing[gcls] & (gt_inst > 0)))
+    sizes = torch.as_tensor(batch["sizes"], dtype=torch.long, device=dev)
+    scan = torch.repeat_interleave(torch.arange(len(batch["sizes"]), device=dev), sizes)
+    cols = [t[keep].cpu().numpy() for t in (scan, gt, gt_inst, res["point_labels"], res["instances"])]
+    bounds = np.searchsorted(cols[0], np.arange(len(batch["sizes"]) + 1))
+    for b in range(len(batch["sizes"])):
+      sl = slice(bounds[b], bounds[b + 1])
+      self.pq.update(cols[1][sl], cols[2][sl], cols[3][sl], cols[4][sl])
 
   def finish(self):
     """The report of ``Evaluator.finish`` plus ``dropped``: points whose ground truth is not a class id (a raw semantic
-    id with no LUT, e.g. KITTI's 10 / 40 / 252); they are not in the matrix."""
+    id with no LUT, e.g. KITTI's 10 / 40 / 252); they are not in the matrix.  With instances, also ``panoptic``: the
+    ``PanopticQuality.result()`` report."""
     cm = self.miou_tracker.total_cm
     iou, recall, precision = confusion_matrix_to_iou_recall_precision(cm)
-    return dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
-                miou=float(self.miou_tracker.result()), dropped=self.miou_tracker.dropped)
+    rep = dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
+               miou=float(self.miou_tracker.result()), dropped=self.miou_tracker.dropped)
+    if self.pq is not None:
+      rep["panoptic"] = self.pq.result()
+    return rep
 
 
 def shard_files(files, comm=None):

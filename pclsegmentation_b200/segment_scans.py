@@ -10,6 +10,12 @@ published with RangeNet++) or, with --no_knn, from the point's own pixel.  With 
 back through the yaml's ``learning_map_inv`` (what a SemanticKITTI submission needs) and the ground truth through its
 ``learning_map``; without it the class ids are written and the ground truth is taken as raw ids.  With --labels the
 point-wise IoU / recall / precision / mIoU report is printed in eval.py's format.
+
+With --instances every thing-class point also gets an instance id (``pipeline.Clustering``: connected components in
+the range image, tuned by --cluster_tau / --cluster_rows / --cluster_cols / --min_points / --no_wrap), written to the
+upper 16 bits of its word as in SemanticKITTI's panoptic labels.  With --labels in KITTI format the panoptic quality
+report (PQ / SQ / RQ per thing class) follows the mIoU report; nuScenes lidarseg files carry no instance ids, so there
+it is skipped.
 """
 import argparse
 import glob
@@ -21,7 +27,7 @@ import numpy as np
 def segment_scans(arg):
   from .dataset_convert import KITTI, ScanBatchLoader, learning_map_lut
   from .inference import load_model_weights
-  from .pipeline import KNN, ScanEvaluator
+  from .pipeline import KNN, Clustering, ScanEvaluator
   from .utils.args_loader import load_model_config
 
   config, model = load_model_config(arg.model or "squeezesegv2", arg.config)
@@ -39,7 +45,11 @@ def segment_scans(arg):
       ym = yaml.safe_load(f)
     lut = learning_map_lut(ym["learning_map"])
     inv = learning_map_lut(ym["learning_map_inv"]).astype(np.uint32)
-  ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN())
+  clustering = None
+  if arg.instances:
+    clustering = Clustering(tau=arg.cluster_tau, rows=arg.cluster_rows, cols=arg.cluster_cols,
+                            min_points=arg.min_points, wrap=not arg.no_wrap)
+  ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering)
   os.makedirs(arg.output_dir, exist_ok=True)
   loader = ScanBatchLoader(arg.format)
   for i in range(0, len(scans), arg.batch):
@@ -48,7 +58,12 @@ def segment_scans(arg):
     if labels is not None:
       res = ev.update(data)
     else:
-      res = ev.seg.segment_device(data["points"], data["offsets"], want_point_labels=True, knn=ev.knn)
+      res = ev.seg.segment_device(data["points"], data["offsets"], want_point_labels=True, knn=ev.knn,
+                                  instances=clustering)
+    if clustering is not None:
+      for f, words in zip(files, ev.seg.label_words(res, data["sizes"], inv)):
+        words.tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
+      continue
     for f, lab in zip(files, ev.seg.point_labels(res, data["sizes"])):
       words = inv[lab] if inv is not None else lab.astype(np.uint32)
       words.astype(np.uint32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
@@ -67,7 +82,21 @@ def segment_scans(arg):
     print("WARNING: %d of %d points have a ground-truth id that is not a class id (0 .. %d) and are not scored%s"
           % (rep["dropped"], int(rep["confusion_matrix"].sum()) + rep["dropped"], config.NUM_CLASS - 1,
              "" if arg.learning_map else "; pass --learning_map to map raw label ids to classes"))
+  if clustering is not None and not kitti:
+    print("no panoptic report: nuScenes lidarseg label files carry no instance ids")
+  elif clustering is not None:
+    print_panoptic(rep["panoptic"], config.CLASSES)
   return rep
+
+
+def print_panoptic(pan, class_names):
+  """The PQ / SQ / RQ report of ``PanopticQuality.result()``, per thing class then the mean."""
+  print("PANOPTIC (thing classes, point-wise)")
+  for i, c in enumerate(pan["classes"]):
+    print("%s PQ: %s SQ: %s RQ: %s (TP %d FP %d FN %d)%s" % (class_names[c].upper(), pan["pq"][i], pan["sq"][i],
+                                                            pan["rq"][i], pan["tp"][i], pan["fp"][i], pan["fn"][i],
+                                                            "" if pan["counted"][i] else " no segment"))
+  print("PQ: {} SQ: {} RQ: {} ".format(pan["pq_mean"], pan["sq_mean"], pan["rq_mean"]))
 
 
 def main(argv=None):
@@ -83,6 +112,12 @@ def main(argv=None):
   ap.add_argument("--no_knn", action="store_true", help="each point takes its own pixel's label (no k-NN vote)")
   ap.add_argument("--labels", default=None, help="glob of .label (KITTI) / lidarseg .bin (nuScenes) files, same order: "
                                                  "print the point-wise report")
+  ap.add_argument("--instances", action="store_true", help="also an instance id per thing-class point (upper 16 bits)")
+  ap.add_argument("--cluster_tau", type=float, default=0.5, help="metres: neighbouring points closer than this join")
+  ap.add_argument("--cluster_rows", type=int, default=1, help="window half-height in rows (0..4)")
+  ap.add_argument("--cluster_cols", type=int, default=2, help="window half-width in columns (0..8)")
+  ap.add_argument("--min_points", type=int, default=10, help="instances with fewer points get id 0")
+  ap.add_argument("--no_wrap", action="store_true", help="columns 0 and W-1 are not neighbours")
   ap.add_argument("--learning_map", default=None, help="yaml with `learning_map` / `learning_map_inv` (semantic-kitti.yaml)")
   return segment_scans(ap.parse_args(argv))
 
