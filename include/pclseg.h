@@ -161,6 +161,42 @@ int pcls_point_instances(const float* points, const uint64_t* keys, const int64_
                          float tau, int min_points, void* scratch, int32_t* instances, int32_t* instance_counts,
                          pcls_stream stream);
 
+/* Test-time augmentation (no reference call site: the configs train with RANDOM_FLIPPING and SHIFT_LEFT_RIGHT, the
+ * reference infers on one view).  The rules are this project's; parity with the reference's training-time flip / shift
+ * code is not claimed.
+ *   A view is (flip, shift), flip in {0, 1}, 0 <= shift < W: a permutation of the columns of a raw range image plus a
+ *   rigid transform of its points.  For source pixel (h, w):
+ *     mirror (flip = 1): column w -> W-1-w and y -> -y (the scan mirrored across the x axis: yaw = -atan2(y, x) puts
+ *       column p at W - p, up to points exactly on a column boundary);
+ *     roll by shift: column w -> (w + shift) mod W, and (x, y) rotated about z by alpha = -2 pi shift / W:
+ *       x' = c x - s y, y' = s x + c y with c = h_cos[t], s = h_sin[t] (the sensor turned by `shift` columns; the
+ *       column grows with yaw).  c and s are computed on the host in float64; for shift a multiple of W/4 they are exactly
+ *       0 and +-1, so the half turn is x -> -x, y -> -y.  With shift = 0 the points are not rotated at all.
+ *     The mirror comes first, then the roll.  z, remission and range are unchanged; the mask is range > 0.
+ *   Frame order is view-major: view t of frame b is frame t*B + b.
+ * pcls_tta_views: raw [B,H,W,channels] f32 (channels 5 or 6; the label channel is ignored) -> for every view the
+ *   network input `input8` [n_views*B,H,W,8] 16-bit (precision PCLS_F16 | PCLS_BF16) and `mask` [n_views*B,H,W] u8, e.g.
+ *   the net's own buffers (pcls_net_input_buffers).  Per view pixel: the rotation in float64 from the float32 inputs
+ *   with separate roundings (c*x and s*y rounded, then their difference / sum), then the input stage of
+ *   pcls_net_forward's raw path, (float)((v - mean) / std) in float64 rounded to float32 and then to 16 bits; empty
+ *   pixels are zeros, channel 5 is the mask, channels 6-7 are zero.  View (0, 0) is bit-identical to the tensor 0 that
+ *   pcls_net_forward makes of raw input and to pcls_project_resolve_net_input's.
+ * pcls_tta_merge: probs [n_views*B,H,W,num_classes] f32 (the forward over the views), mask [n_views*B,H,W] u8 (the views'
+ *   masks) -> per output pixel (b, h, w) of the source image, with q_t the pixel of view t that (b, h, w) maps to:
+ *   acc = probs[q_0]; acc = acc + probs[q_t] for t = 1 .. n_views-1 in float32 (round to nearest); mean = acc / n_views
+ *   (T = 1 returns probs[q_0] unchanged); out_preds [B,H,W] i32 = argmax of the means (first index on ties, the head's
+ *   rule), none_index where mask[q_0] == 0; out_probs [B,H,W,num_classes] f32 = the means, or NULL.
+ * Both calls check before any launch: 1 <= n_views <= PCLS_TTA_MAX_VIEWS, flips 0 / 1, shifts in [0, W), no view twice,
+ * finite h_cos / h_sin, channels 5 / 6, 1 <= num_classes <= 32, 0 <= none_index < num_classes, and the pointers the call
+ * needs; otherwise PCLS_ERR_INVALID. */
+#define PCLS_TTA_MAX_VIEWS 8
+int pcls_tta_views(const float* raw, int channels, int B, int H, int W, const double* h_mean5, const double* h_std5,
+                   int n_views, const int* h_flip, const int* h_shift, const double* h_cos, const double* h_sin,
+                   int precision, void* input8, uint8_t* mask, pcls_stream stream);
+int pcls_tta_merge(const float* probs, const uint8_t* mask, int B, int H, int W, int num_classes, int none_index,
+                   int n_views, const int* h_flip, const int* h_shift, float* out_probs, int32_t* out_preds,
+                   pcls_stream stream);
+
 /* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
  * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,

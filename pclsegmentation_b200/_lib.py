@@ -48,6 +48,11 @@ SIGNATURES = {
   "pcls_point_instances": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p,
                                    c_void_p, c_int, c_uint32, c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
+  "pcls_tta_views": (c_int, [c_void_p, c_int, c_int, c_int, c_int, POINTER(c_double), POINTER(c_double), c_int,
+                             POINTER(c_int), POINTER(c_int), POINTER(c_double), POINTER(c_double), c_int, c_void_p,
+                             c_void_p, c_void_p]),
+  "pcls_tta_merge": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int),
+                             POINTER(c_int), c_void_p, c_void_p, c_void_p]),
   "pcls_map_labels": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
   "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -16,6 +16,7 @@ import numpy as np
 
 from .inference import load_model_weights
 from .pipeline import Evaluator, shard_files
+from .tta import add_tta_flags, from_args
 from .utils.args_loader import load_model_config
 
 
@@ -35,7 +36,7 @@ def evaluation(arg):
   load_model_weights(model, arg, verbose=rank == 0)
 
   files = shard_files(glob.glob(os.path.join(arg.data_path, arg.image_set, "*.npy")), comm)
-  ev = Evaluator(model, comm)
+  ev = Evaluator(model, comm, tta=from_args(arg.tta, arg.tta_shifts))
   if rank == 0:
     print("Performing Evaluation")
   for i in range(0, len(files), arg.batch):
@@ -69,6 +70,7 @@ def main(argv=None):
                            '`darknet53`, `darknet21`, `darknet53kitti`')
   parser.add_argument('-b', '--batch', type=int, default=8, help='frames per forward call (the reference uses 1)')
   parser.add_argument('--random_init', action='store_true', help='run without --path_to_model on Keras-default weights')
+  add_tta_flags(parser)
   return evaluation(parser.parse_args(argv))
 
 

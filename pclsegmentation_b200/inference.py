@@ -16,6 +16,7 @@ import os
 import numpy as np
 
 from .device import samples_to_device
+from .tta import add_tta_flags, forward_tta, from_args
 from .utils.args_loader import load_model_config
 from .utils.util import normalize
 
@@ -45,12 +46,16 @@ def inference(arg):
   if not os.path.exists(arg.output_dir):
     os.makedirs(arg.output_dir)
   none = config.CLASSES.index("None")
+  tta = from_args(arg.tta, arg.tta_shifts)
   files = sorted(glob.iglob(arg.input_path))
   for i in range(0, len(files), arg.batch):
     chunk = files[i:i + arg.batch]
     samples = np.stack([np.load(f) for f in chunk])          # float64 on disk: uploaded as is, narrowed on the device
-    res = model.forward_device(samples_to_device(samples), None, mean=config.INPUT_MEAN, std=config.INPUT_STD,
-                               want_probabilities=False)
+    if tta is not None:
+      res = forward_tta(model, samples_to_device(samples), tta)
+    else:
+      res = model.forward_device(samples_to_device(samples), None, mean=config.INPUT_MEAN, std=config.INPUT_STD,
+                                 want_probabilities=False)
     predictions = res["predictions"].cpu().numpy()
     for f, sample, pred in zip(chunk, samples, predictions):
       print("Process: {0}".format(f))
@@ -83,6 +88,7 @@ def main(argv=None):
   parser.add_argument('-b', '--batch', type=int, default=8, help='frames per forward call')
   parser.add_argument('--no_plots', action='store_true', help='only write pred_*.npy')
   parser.add_argument('--random_init', action='store_true', help='run without --path_to_model on Keras-default weights')
+  add_tta_flags(parser)
   inference(parser.parse_args(argv))
 
 

@@ -3,7 +3,8 @@
 * ``ScanSegmenter``  raw scans -> spherical projection -> network forward -> labels (BASELINE config 4: the converter's
   per-scan loop dataset_convert/semantic_kitti.py:152-179 fused with inference.py:44-78; range images never leave HBM),
   optionally one label per point (pcls_point_labels: back-projection or the k-NN vote of ``KNN``) and an instance id
-  per thing-class point (pcls_point_instances: connected components of ``Clustering``)
+  per thing-class point (pcls_point_instances: connected components of ``Clustering``); with a ``tta.TTA`` the forward
+  runs over mirrored / rotated views and their merged predictions feed the rest
 * ``ScanEvaluator``  point-wise evaluation on raw scans: scans -> point labels -> confusion update per point, and
   panoptic quality (``metrics.PanopticQuality``) when instances are asked for
 * ``Evaluator``      the eval.py hot loop (eval.py:45-50): forward -> head -> confusion update per batch on this rank's
@@ -19,6 +20,7 @@ from .device import ptr, samples_to_device, stream_handle, to_device
 from .laserscan import SphericalProjector
 from .metrics import MeanIoU, PanopticQuality
 from .sharding import Communicator, shard_range
+from .tta import forward_tta
 from .utils.util import confusion_matrix_to_iou_recall_precision
 
 
@@ -85,7 +87,7 @@ class ScanSegmenter:
     self.projector = SphericalProjector(mc.ZENITH_LEVEL, mc.AZIMUTH_LEVEL, fov_up, fov_down, label_lut=label_lut)
 
   def segment_device(self, points, offsets, labels=None, want_probabilities=False, out=None, want_image=False,
-                     want_logits=False, want_point_labels=False, knn=None, instances=None):
+                     want_logits=False, want_point_labels=False, knn=None, instances=None, tta=None):
     """points [total,4] float32 CUDA (x,y,z,remission), offsets [B+1] int64 CUDA -> dict(predictions, proj_idx,
     probabilities?, logits?, image?, point_labels?) - keys and activations stay on the device.
 
@@ -100,14 +102,23 @@ class ScanSegmenter:
 
     instances: a ``Clustering`` - also ``instances`` [total] int32 (0 = no instance, ids 1, 2, ... per scan) and
     ``instance_counts`` [B] int32 CUDA (pcls_point_instances on the same stream after the point labels); needs
-    want_point_labels."""
+    want_point_labels.
+
+    tta: a ``tta.TTA`` - the range image is materialised and goes through ``tta.forward_tta``; the merged predictions
+    (and probabilities) take the place of the forward's, and the point labels / instances are computed from them as
+    they are.  Logits are not merged, so want_logits is refused with it."""
     if instances is not None and not want_point_labels:
       raise ValueError("instances need the point labels: segment with want_point_labels=True")
+    if tta is not None and want_logits:
+      raise ValueError("test-time augmentation merges probabilities, not logits: segment without want_logits")
     B = int(offsets.numel()) - 1
-    if want_image or labels is not None or B > self._staged_capacity(B):
+    if tta is not None or want_image or labels is not None or B > self._staged_capacity(B):
       proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0, want_point_outputs=want_point_labels)
-      res = self.model.forward_device(proj["image"], None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD,
-                                      want_probabilities=want_probabilities, want_logits=want_logits, out=out)
+      if tta is not None:
+        res = forward_tta(self.model, proj["image"], tta, want_probabilities=want_probabilities, out=out)
+      else:
+        res = self.model.forward_device(proj["image"], None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD,
+                                        want_probabilities=want_probabilities, want_logits=want_logits, out=out)
       res.update(image=proj["image"], proj_idx=proj["proj_idx"])
       if want_point_labels:
         res["point_labels"] = self._point_labels(res["predictions"], proj["keys"], offsets, proj["proj_x"],
@@ -221,11 +232,12 @@ class ScanSegmenter:
 
 
 class Evaluator:
-  """eval.py:33-58 on one rank; ``comm`` sums the confusion matrix over ranks (sharding.Communicator) or is None."""
+  """eval.py:33-58 on one rank; ``comm`` sums the confusion matrix over ranks (sharding.Communicator) or is None.
+  ``tta``: a ``tta.TTA`` - the predictions are merged over its views (``tta.forward_tta``)."""
 
-  def __init__(self, model, comm=None):
+  def __init__(self, model, comm=None, tta=None):
     self.model, self.mc = model, model.mc
-    self.comm = comm
+    self.comm, self.tta = comm, tta
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self._none = self.mc.CLASSES.index("None")
     self._mean = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_MEAN).reshape(-1))
@@ -239,7 +251,10 @@ class Evaluator:
     B, H, W, C = x.shape
     if C != 6:
       raise ValueError("evaluation samples need 6 channels (x,y,z,intensity,depth,label)")
-    res = self.model.forward_device(x, None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD, want_probabilities=False)
+    if self.tta is not None:
+      res = forward_tta(self.model, x, self.tta)
+    else:
+      res = self.model.forward_device(x, None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD, want_probabilities=False)
     label = torch.empty((B, H, W), dtype=torch.int32, device=x.device)
     _lib.check(_lib.load().pcls_input_stage(ptr(x), 6, B * H * W, self._mean, self._std, self._none, None, None,
                                             ptr(label), None, 0, None, stream_handle()), "pcls_input_stage")
@@ -262,11 +277,12 @@ class ScanEvaluator:
   semantic id without a LUT) -> confusion update over the points.  ``finish()`` gives the report of
   ``Evaluator.finish``.  With ``instances`` (a ``Clustering``) each batch also gets instance ids and feeds a
   ``PanopticQuality`` whose ground-truth instance id is the upper half of the label word (``word >> 16``); only the
-  points in a predicted or ground-truth thing segment come back to the host."""
+  points in a predicted or ground-truth thing segment come back to the host.  ``tta``: a ``tta.TTA`` for the forward
+  (``ScanSegmenter.segment_device(tta=)``)."""
 
-  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None):
+  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None, tta=None):
     self.seg = ScanSegmenter(model, fov_up, fov_down)
-    self.mc, self.knn, self.instances = model.mc, knn, instances
+    self.mc, self.knn, self.instances, self.tta = model.mc, knn, instances, tta
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self.pq = None
     if instances is not None:
@@ -281,7 +297,7 @@ class ScanEvaluator:
     if batch.get("labels") is None:
       raise ValueError("point-wise evaluation needs the label files")
     res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn,
-                                  instances=self.instances)
+                                  instances=self.instances, tta=self.tta)
     n = int(batch["points"].shape[0])
     gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
     lut = self.lut

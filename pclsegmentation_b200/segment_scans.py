@@ -16,6 +16,9 @@ the range image, tuned by --cluster_tau / --cluster_rows / --cluster_cols / --mi
 upper 16 bits of its word as in SemanticKITTI's panoptic labels.  With --labels in KITTI format the panoptic quality
 report (PQ / SQ / RQ per thing class) follows the mIoU report; nuScenes lidarseg files carry no instance ids, so there
 it is skipped.
+
+With --tta (the mirror image) and / or --tta_shifts (rolls by that many columns, e.g. 0,1024) the forward runs over
+those views of each scan's range image and their averaged probabilities decide the pixel labels (``tta.TTA``).
 """
 import argparse
 import glob
@@ -28,6 +31,7 @@ def segment_scans(arg):
   from .dataset_convert import KITTI, ScanBatchLoader, learning_map_lut
   from .inference import load_model_weights
   from .pipeline import KNN, Clustering, ScanEvaluator
+  from .tta import from_args
   from .utils.args_loader import load_model_config
 
   config, model = load_model_config(arg.model or "squeezesegv2", arg.config)
@@ -49,7 +53,9 @@ def segment_scans(arg):
   if arg.instances:
     clustering = Clustering(tau=arg.cluster_tau, rows=arg.cluster_rows, cols=arg.cluster_cols,
                             min_points=arg.min_points, wrap=not arg.no_wrap)
-  ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering)
+  tta = from_args(arg.tta, arg.tta_shifts)
+  ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering,
+                     tta=tta)
   os.makedirs(arg.output_dir, exist_ok=True)
   loader = ScanBatchLoader(arg.format)
   for i in range(0, len(scans), arg.batch):
@@ -59,7 +65,7 @@ def segment_scans(arg):
       res = ev.update(data)
     else:
       res = ev.seg.segment_device(data["points"], data["offsets"], want_point_labels=True, knn=ev.knn,
-                                  instances=clustering)
+                                  instances=clustering, tta=tta)
     if clustering is not None:
       for f, words in zip(files, ev.seg.label_words(res, data["sizes"], inv)):
         words.tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
@@ -119,6 +125,8 @@ def main(argv=None):
   ap.add_argument("--min_points", type=int, default=10, help="instances with fewer points get id 0")
   ap.add_argument("--no_wrap", action="store_true", help="columns 0 and W-1 are not neighbours")
   ap.add_argument("--learning_map", default=None, help="yaml with `learning_map` / `learning_map_inv` (semantic-kitti.yaml)")
+  from .tta import add_tta_flags
+  add_tta_flags(ap)
   return segment_scans(ap.parse_args(argv))
 
 
