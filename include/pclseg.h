@@ -197,6 +197,44 @@ int pcls_tta_merge(const float* probs, const uint8_t* mask, int B, int H, int W,
                    int n_views, const int* h_flip, const int* h_shift, float* out_probs, int32_t* out_preds,
                    pcls_stream stream);
 
+/* Calibrated confidence (no reference call site: the reference reduces the softmax to an argmax).  Post-hoc temperature
+ * scaling (Guo et al., "On Calibration of Modern Neural Networks", ICML 2017): one scalar T, probabilities softmax(z / T).
+ * The argmax does not depend on T.  The host passes a = 1/T, computed in float64 and rounded once to float32.
+ * All four calls check every argument before any launch (1 <= num_classes <= 32, the pointers the call needs; otherwise
+ * PCLS_ERR_INVALID with a pcls_last_error message); n == 0 is a no-op.
+ * pcls_confidence: exactly one of logits / probs [n,NC] f32 is non-NULL; a finite and > 0, and a == 1 in probs mode.
+ *   Logits mode: v_c = z_c * a rounded to float32, then the head's softmax (pcls_head's arithmetic: at a = 1 out_probs is
+ *   bit-identical to pcls_head's probabilities; the fused conv_head path uses ex2.approx and is not).  Probs mode: p = probs.
+ *   out_conf [n] f32 = max_c p_c; out_entropy [n] f32 = (-sum_c p_c * logf(p_c)) over the classes with p_c > 0, summed in
+ *   class order in float32 (products and sums rounded one at a time), divided by logf(NC); 0 when NC = 1.  Where
+ *   mask[i] == 0 (mask [n] u8, NULL = all valid) conf and entropy are 0.  out_probs [n,NC] f32 is written for every pixel,
+ *   as the head does.  Each output may be NULL, at least one must be given.
+ * pcls_temperature_nll: the NLL of softmax(z * a_t) for n_temps (1..64) inverse temperatures h_inv_temps (host f32, each
+ *   finite and > 0) in one pass over logits [n,NC] f32.  A pixel counts when 0 <= label < NC and label != ignore_index
+ *   (label [n] i32).  Per counted pixel and t, in float32 with separate roundings: s_c = z_c * a_t, m = max_c s_c,
+ *   e = sum_c expf(s_c - m) in class order, term = (logf(e) + m) - s_label.  nll_acc [n_temps] f64 += term (float64 sums,
+ *   order unspecified), counted [1] i64 += 1 per counted pixel; both accumulated in place.
+ * pcls_reliability_update: the reliability histogram of n_bins (1..64) equal bins of [0, 1].  An element counts when
+ *   0 <= label < NC, label != ignore_index and 0 <= pred < NC (conf [n] f32, pred / label [n] i32).  Its bin is
+ *   b = min((int)(conf * (float)n_bins), n_bins - 1) with the product rounded to float32 (clamped at 0 below);
+ *   bin_count[b] (i64) += 1, bin_correct[b] (i64) += (pred == label), bin_conf[b] (f64) += conf, accumulated in place.
+ *   The host computes ECE = sum_b |bin_correct_b - bin_conf_b| / N, MCE over the non-empty bins, accuracy and mean
+ *   confidence from these sums.
+ * pcls_point_confidence: per point i of scan b (offsets [B+1] i64, proj_x / proj_y [total] i32 of pcls_project_scatter,
+ *   point_labels [total] i32, probs [B,H,W,NC] f32): out_conf[i] = probs[b, proj_y[i], proj_x[i], point_labels[i]], the
+ *   probability the point's own pixel gives the label the point got; 0 for a dropped point (proj_x < 0) or a label
+ *   outside [0, NC).  An exact gather. */
+int pcls_confidence(const float* logits, const float* probs, const uint8_t* mask, int64_t n, int num_classes,
+                    float inv_temperature, float* out_probs, float* out_conf, float* out_entropy, pcls_stream stream);
+int pcls_temperature_nll(const float* logits, const int32_t* label, int64_t n, int num_classes, int ignore_index,
+                         int n_temps, const float* h_inv_temps, double* nll_acc, int64_t* counted, pcls_stream stream);
+int pcls_reliability_update(const float* conf, const int32_t* pred, const int32_t* label, int64_t n, int num_classes,
+                            int ignore_index, int n_bins, int64_t* bin_count, int64_t* bin_correct, double* bin_conf,
+                            pcls_stream stream);
+int pcls_point_confidence(const float* probs, const int64_t* offsets, int B, int H, int W, int64_t total,
+                          const int32_t* proj_x, const int32_t* proj_y, const int32_t* point_labels, int num_classes,
+                          float* out_conf, pcls_stream stream);
+
 /* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
  * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,

@@ -53,7 +53,15 @@ SIGNATURES = {
                              c_void_p, c_void_p]),
   "pcls_tta_merge": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int),
                              POINTER(c_int), c_void_p, c_void_p, c_void_p]),
-  "pcls_map_labels": (c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
+  "pcls_confidence": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_float, c_void_p, c_void_p, c_void_p,
+                              c_void_p]),
+  "pcls_temperature_nll": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, POINTER(c_float), c_void_p,
+                                   c_void_p, c_void_p]),
+  "pcls_reliability_update": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p,
+                                      c_void_p, c_void_p]),
+  "pcls_point_confidence": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p,
+                                    c_int, c_void_p, c_void_p]),
+  "pcls_map_labels":(c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
   "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
   "pcls_net_input_buffers": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int)]),

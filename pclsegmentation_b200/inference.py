@@ -15,6 +15,7 @@ import os
 
 import numpy as np
 
+from .calibration import add_temperature_flag, confidence, raw_mask
 from .device import samples_to_device
 from .tta import add_tta_flags, forward_tta, from_args
 from .utils.args_loader import load_model_config
@@ -47,20 +48,30 @@ def inference(arg):
     os.makedirs(arg.output_dir)
   none = config.CLASSES.index("None")
   tta = from_args(arg.tta, arg.tta_shifts)
+  if arg.confidence and tta is not None and arg.temperature != 1.0:
+    raise SystemExit("--tta merges probabilities, not logits: --confidence with --tta needs --temperature 1")
   files = sorted(glob.iglob(arg.input_path))
   for i in range(0, len(files), arg.batch):
     chunk = files[i:i + arg.batch]
     samples = np.stack([np.load(f) for f in chunk])          # float64 on disk: uploaded as is, narrowed on the device
+    x = samples_to_device(samples)
     if tta is not None:
-      res = forward_tta(model, samples_to_device(samples), tta)
+      res = forward_tta(model, x, tta, want_probabilities=arg.confidence)
     else:
-      res = model.forward_device(samples_to_device(samples), None, mean=config.INPUT_MEAN, std=config.INPUT_STD,
-                                 want_probabilities=False)
+      res = model.forward_device(x, None, mean=config.INPUT_MEAN, std=config.INPUT_STD, want_probabilities=False,
+                                 want_logits=arg.confidence)
+    conf = None
+    if arg.confidence:
+      src = dict(probs=res["probabilities"]) if tta is not None else dict(logits=res["logits"])
+      conf = confidence(config.NUM_CLASS, mask=raw_mask(x, config), temperature=arg.temperature,
+                        **src)["confidence"].cpu().numpy()
     predictions = res["predictions"].cpu().numpy()
-    for f, sample, pred in zip(chunk, samples, predictions):
+    for k, (f, sample, pred) in enumerate(zip(chunk, samples, predictions)):
       print("Process: {0}".format(f))
       file_name = os.path.splitext(os.path.basename(f))[0]
       np.save(os.path.join(arg.output_dir, 'pred_' + file_name + '.npy'), pred)
+      if conf is not None:
+        np.save(os.path.join(arg.output_dir, 'conf_' + file_name + '.npy'), conf[k])
       if arg.no_plots:
         continue
       from PIL import Image
@@ -89,6 +100,9 @@ def main(argv=None):
   parser.add_argument('--no_plots', action='store_true', help='only write pred_*.npy')
   parser.add_argument('--random_init', action='store_true', help='run without --path_to_model on Keras-default weights')
   add_tta_flags(parser)
+  parser.add_argument('--confidence', action='store_true',
+                      help='also write conf_<name>.npy: float32 [H,W] max softmax(logits / T) per pixel, 0 at empty pixels')
+  add_temperature_flag(parser)
   inference(parser.parse_args(argv))
 
 

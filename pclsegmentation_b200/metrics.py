@@ -95,6 +95,77 @@ class MeanIoU:
   reset_state = reset_states
 
 
+class Reliability:
+  """Reliability of confidences (Guo et al., ICML 2017): ``n_bins`` equal bins of [0, 1], per bin the number of counted
+  elements, how many of them are correct and the sum of their confidences, accumulated on the GPU
+  (pcls_reliability_update: int64 / int64 / float64, a shared-memory histogram per block).  An element counts when its
+  label and prediction are class ids in [0, num_classes) and the label is not ``ignore_index``.  Pixels and points go
+  through the same kernel."""
+
+  def __init__(self, n_bins, num_classes):
+    self.n_bins, self.num_classes = int(n_bins), int(num_classes)
+    if not 1 <= self.n_bins <= 64:
+      raise ValueError("n_bins must be in [1, 64], got %d" % self.n_bins)
+    self.count = self.correct = self.conf = None
+
+  def _ensure(self, dev=None):
+    if self.count is None:
+      dev = dev if dev is not None else require_cuda()
+      self.count = torch.zeros(self.n_bins, dtype=torch.int64, device=dev)
+      self.correct = torch.zeros(self.n_bins, dtype=torch.int64, device=dev)
+      self.conf = torch.zeros(self.n_bins, dtype=torch.float64, device=dev)
+
+  def update_state(self, conf, pred, label, ignore_index=-1):
+    """conf float32, pred / label int32: CUDA tensors (or arrays) of one size."""
+    self._ensure()
+    c = to_device(conf, torch.float32).reshape(-1)
+    p = to_device(pred, torch.int32).reshape(-1)
+    y = to_device(label, torch.int32).reshape(-1)
+    if not c.numel() == p.numel() == y.numel():
+      raise ValueError("conf / pred / label sizes differ: %d, %d, %d" % (c.numel(), p.numel(), y.numel()))
+    _lib.check(_lib.load().pcls_reliability_update(ptr(c), ptr(p), ptr(y), c.numel(), self.num_classes, int(ignore_index),
+                                                   self.n_bins, ptr(self.count), ptr(self.correct), ptr(self.conf),
+                                                   stream_handle()), "pcls_reliability_update")
+
+  def allreduce(self, comm):
+    """Sums the bins over the ranks of ``comm`` (torch.distributed, off the hot path)."""
+    self._ensure()
+    comm.allreduce_sums([self.count, self.correct, self.conf])
+
+  def reset_states(self):
+    if self.count is not None:
+      self.count.zero_()
+      self.correct.zero_()
+      self.conf.zero_()
+
+  def result(self):
+    """dict(ece, mce, accuracy, mean_confidence, count (N), and per bin: bin_lo, bin_hi, bin_count, bin_accuracy,
+    bin_confidence (0 for an empty bin)).  ECE = sum_b |correct_b - conf_b| / N; MCE = max over the non-empty bins of
+    |accuracy_b - confidence_b|; all 0 when nothing was counted."""
+    if self.count is None:
+      cnt, cor, cs = np.zeros(self.n_bins, np.int64), np.zeros(self.n_bins, np.int64), np.zeros(self.n_bins)
+    else:
+      cnt, cor, cs = self.count.cpu().numpy(), self.correct.cpu().numpy(), self.conf.cpu().numpy()
+    return reliability_scores(cnt, cor, cs)
+
+
+def reliability_scores(count, correct, conf_sum):
+  """The scores of ``Reliability.result`` from the three per-bin sums (host, float64)."""
+  count = np.asarray(count, np.int64)
+  correct = np.asarray(correct, np.int64)
+  conf_sum = np.asarray(conf_sum, np.float64)
+  nb = count.size
+  n = int(count.sum())
+  full = count > 0
+  acc_b = np.divide(correct, count, out=np.zeros(nb), where=full)
+  conf_b = np.divide(conf_sum, count, out=np.zeros(nb), where=full)
+  edges = np.arange(nb + 1) / nb
+  return dict(ece=float(np.abs(correct - conf_sum).sum() / n) if n else 0.0,
+              mce=float(np.abs(acc_b - conf_b)[full].max()) if n else 0.0,
+              accuracy=float(correct.sum() / n) if n else 0.0, mean_confidence=float(conf_sum.sum() / n) if n else 0.0,
+              count=n, bin_lo=edges[:-1], bin_hi=edges[1:], bin_count=count, bin_accuracy=acc_b, bin_confidence=conf_b)
+
+
 class PanopticQuality:
   """Panoptic quality over thing classes (Kirillov et al., "Panoptic Segmentation", CVPR 2019), point-wise per scan, on
   the host (numpy; the caller hands over only the points that can be in a segment).  The rules are this project's; parity

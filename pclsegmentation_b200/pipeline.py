@@ -6,9 +6,11 @@
   per thing-class point (pcls_point_instances: connected components of ``Clustering``); with a ``tta.TTA`` the forward
   runs over mirrored / rotated views and their merged predictions feed the rest
 * ``ScanEvaluator``  point-wise evaluation on raw scans: scans -> point labels -> confusion update per point, and
-  panoptic quality (``metrics.PanopticQuality``) when instances are asked for
+  panoptic quality (``metrics.PanopticQuality``) when instances are asked for, and the reliability of the per-point
+  confidences with a ``calibration.Calibration``
 * ``Evaluator``      the eval.py hot loop (eval.py:45-50): forward -> head -> confusion update per batch on this rank's
-  shard of the frames, one all-reduce of the int64 matrix at the end, then IoU / recall / precision / mIoU.
+  shard of the frames, one all-reduce of the int64 matrix at the end, then IoU / recall / precision / mIoU; with a
+  ``calibration.Calibration`` also the reliability of the confidences (ECE / MCE) and the NLL of a temperature grid.
 """
 import ctypes
 
@@ -16,9 +18,10 @@ import numpy as np
 import torch
 
 from . import _lib
+from .calibration import TemperatureNLL, check_tta, confidence as pixel_confidence, raw_mask
 from .device import ptr, samples_to_device, stream_handle, to_device
 from .laserscan import SphericalProjector
-from .metrics import MeanIoU, PanopticQuality
+from .metrics import MeanIoU, PanopticQuality, Reliability
 from .sharding import Communicator, shard_range
 from .tta import forward_tta
 from .utils.util import confusion_matrix_to_iou_recall_precision
@@ -87,7 +90,7 @@ class ScanSegmenter:
     self.projector = SphericalProjector(mc.ZENITH_LEVEL, mc.AZIMUTH_LEVEL, fov_up, fov_down, label_lut=label_lut)
 
   def segment_device(self, points, offsets, labels=None, want_probabilities=False, out=None, want_image=False,
-                     want_logits=False, want_point_labels=False, knn=None, instances=None, tta=None):
+                     want_logits=False, want_point_labels=False, knn=None, instances=None, tta=None, confidence=None):
     """points [total,4] float32 CUDA (x,y,z,remission), offsets [B+1] int64 CUDA -> dict(predictions, proj_idx,
     probabilities?, logits?, image?, point_labels?) - keys and activations stay on the device.
 
@@ -106,19 +109,33 @@ class ScanSegmenter:
 
     tta: a ``tta.TTA`` - the range image is materialised and goes through ``tta.forward_tta``; the merged predictions
     (and probabilities) take the place of the forward's, and the point labels / instances are computed from them as
-    they are.  Logits are not merged, so want_logits is refused with it."""
+    they are.  Logits are not merged, so want_logits is refused with it.
+
+    confidence: a temperature T - also ``confidence`` [B,H,W] float32 (max softmax(logits / T) per pixel, 0 at empty
+    pixels; pcls_confidence) and ``point_confidence`` [total] float32 (the probability at T that the point's own pixel
+    gives the point's label; pcls_point_confidence); needs want_point_labels.  At T = 1 the forward's probabilities are
+    used as they are; with a TTA only T = 1 is available (the merged probabilities)."""
     if instances is not None and not want_point_labels:
       raise ValueError("instances need the point labels: segment with want_point_labels=True")
     if tta is not None and want_logits:
       raise ValueError("test-time augmentation merges probabilities, not logits: segment without want_logits")
+    if confidence is not None:
+      if not want_point_labels:
+        raise ValueError("confidence needs the point labels: segment with want_point_labels=True")
+      if tta is not None and float(confidence) != 1.0:
+        raise ValueError("test-time augmentation merges probabilities, not logits: confidence with TTA is only "
+                         "available at temperature 1")
+    tempered = confidence is not None and float(confidence) != 1.0
+    fwd_probs = want_probabilities or (confidence is not None and not tempered)
+    fwd_logits = want_logits or tempered
     B = int(offsets.numel()) - 1
     if tta is not None or want_image or labels is not None or B > self._staged_capacity(B):
       proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0, want_point_outputs=want_point_labels)
       if tta is not None:
-        res = forward_tta(self.model, proj["image"], tta, want_probabilities=want_probabilities, out=out)
+        res = forward_tta(self.model, proj["image"], tta, want_probabilities=fwd_probs, out=out)
       else:
         res = self.model.forward_device(proj["image"], None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD,
-                                        want_probabilities=want_probabilities, want_logits=want_logits, out=out)
+                                        want_probabilities=fwd_probs, want_logits=fwd_logits, out=out)
       res.update(image=proj["image"], proj_idx=proj["proj_idx"])
       if want_point_labels:
         res["point_labels"] = self._point_labels(res["predictions"], proj["keys"], offsets, proj["proj_x"],
@@ -126,6 +143,9 @@ class ScanSegmenter:
         if instances is not None:
           res.update(self._instances(points, proj["keys"], offsets, proj["proj_x"], proj["proj_y"],
                                      res["point_labels"], instances))
+        if confidence is not None:
+          res.update(self._confidence(res, raw_mask(proj["image"], self.mc), offsets, proj["proj_x"], proj["proj_y"],
+                                      float(confidence), want_probabilities, want_logits))
       return res
     lib = _lib.load()
     H, W = self.projector.H, self.projector.W
@@ -147,13 +167,38 @@ class ScanSegmenter:
     _lib.check(lib.pcls_project_resolve_net_input(ptr(points), ptr(offsets), B, H, W, ptr(keys), mean, std,
                                                   self.model.precision, inp, msk, ptr(idx), s),
                "pcls_project_resolve_net_input")
-    res = self.model.forward_staged(B, want_probabilities=want_probabilities, want_logits=want_logits, out=out)
+    res = self.model.forward_staged(B, want_probabilities=fwd_probs, want_logits=fwd_logits, out=out)
     res.update(proj_idx=idx)
     if want_point_labels:
       res["point_labels"] = self._point_labels(res["predictions"], keys, offsets, px, py, ur, knn)
       if instances is not None:
         res.update(self._instances(points, keys, offsets, px, py, res["point_labels"], instances))
+      if confidence is not None:
+        # the net's own mask buffer holds this batch's mask (range > 0) until the next forward
+        res.update(self._confidence(res, msk, offsets, px, py, float(confidence), want_probabilities, want_logits))
     return res
+
+  def _confidence(self, res, mask, offsets, px, py, T, want_probabilities, want_logits):
+    """Pixel confidence at temperature T and the per-point confidence of the point labels; drops the probabilities /
+    logits the caller did not ask for."""
+    nc = self.mc.NUM_CLASS
+    if T != 1.0:
+      c = pixel_confidence(nc, logits=res["logits"], mask=mask, temperature=T, want_probs=True)
+      probs = c["probabilities"]
+    else:
+      probs = res["probabilities"]
+      c = pixel_confidence(nc, probs=probs, mask=mask)
+    B, H, W = res["predictions"].shape
+    total = int(px.numel())
+    pc = torch.empty(total, dtype=torch.float32, device=probs.device)
+    _lib.check(_lib.load().pcls_point_confidence(ptr(probs), ptr(offsets), B, H, W, total, ptr(px), ptr(py),
+                                                 ptr(res["point_labels"]), nc, ptr(pc), stream_handle()),
+               "pcls_point_confidence")
+    if not want_probabilities:
+      res.pop("probabilities", None)
+    if not want_logits:
+      res.pop("logits", None)
+    return dict(confidence=c["confidence"], point_confidence=pc)
 
   def _point_labels(self, preds, keys, offsets, px, py, ur, knn):
     B, H, W = preds.shape
@@ -233,13 +278,24 @@ class ScanSegmenter:
 
 class Evaluator:
   """eval.py:33-58 on one rank; ``comm`` sums the confusion matrix over ranks (sharding.Communicator) or is None.
-  ``tta``: a ``tta.TTA`` - the predictions are merged over its views (``tta.forward_tta``)."""
+  ``tta``: a ``tta.TTA`` - the predictions are merged over its views (``tta.forward_tta``).
+  ``calibration``: a ``calibration.Calibration`` - the forward also returns its logits; the confidence at the
+  calibration's temperature (pcls_confidence) is binned against the head's predictions and the fixed-up labels, the
+  "None" class ignored (``metrics.Reliability``), and the NLL at T = 1, at the temperature and, with ``fit``, on the
+  grid is accumulated (``calibration.TemperatureNLL``).  With a TTA the merged probabilities give the confidence, so
+  only T = 1 without a fit is available."""
 
-  def __init__(self, model, comm=None, tta=None):
+  def __init__(self, model, comm=None, tta=None, calibration=None):
+    check_tta(calibration, tta)
     self.model, self.mc = model, model.mc
-    self.comm, self.tta = comm, tta
+    self.comm, self.tta, self.calibration = comm, tta, calibration
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self._none = self.mc.CLASSES.index("None")
+    self.reliability = self.nll = None
+    if calibration is not None:
+      self.reliability = Reliability(calibration.n_bins, self.mc.NUM_CLASS)
+      if tta is None:
+        self.nll = TemperatureNLL(calibration, self.mc.NUM_CLASS, self._none)
     self._mean = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_MEAN).reshape(-1))
     self._std = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_STD).reshape(-1))
 
@@ -251,14 +307,25 @@ class Evaluator:
     B, H, W, C = x.shape
     if C != 6:
       raise ValueError("evaluation samples need 6 channels (x,y,z,intensity,depth,label)")
+    cal = self.calibration is not None
     if self.tta is not None:
-      res = forward_tta(self.model, x, self.tta)
+      res = forward_tta(self.model, x, self.tta, want_probabilities=cal)
     else:
-      res = self.model.forward_device(x, None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD, want_probabilities=False)
+      res = self.model.forward_device(x, None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD, want_probabilities=False,
+                                      want_logits=cal)
     label = torch.empty((B, H, W), dtype=torch.int32, device=x.device)
     _lib.check(_lib.load().pcls_input_stage(ptr(x), 6, B * H * W, self._mean, self._std, self._none, None, None,
                                             ptr(label), None, 0, None, stream_handle()), "pcls_input_stage")
     self.miou_tracker.update_state(label, res["predictions"])
+    if cal:
+      nc = self.mc.NUM_CLASS
+      if self.tta is not None:
+        conf = pixel_confidence(nc, probs=res["probabilities"])["confidence"]
+      else:
+        conf = pixel_confidence(nc, logits=res["logits"], temperature=self.calibration.temperature)["confidence"]
+        self.nll.update(res["logits"], label)
+      # masked pixels carry the "None" label after the fix-up, so they are not binned
+      self.reliability.update_state(conf, res["predictions"], label, self._none)
     return (res["predictions"], label) if return_label else res["predictions"]
 
   def finish(self):
@@ -267,8 +334,22 @@ class Evaluator:
       self.miou_tracker.allreduce(self.comm)
     cm = self.miou_tracker.total_cm
     iou, recall, precision = confusion_matrix_to_iou_recall_precision(cm)
-    return dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
-                miou=float(self.miou_tracker.result()))
+    rep = dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
+               miou=float(self.miou_tracker.result()))
+    if self.calibration is not None:
+      rep["calibration"] = _calibration_report(self.calibration, self.reliability, self.nll, self.comm)
+    return rep
+
+
+def _calibration_report(calibration, reliability, nll, comm):
+  """dict(temperature, n_bins, reliability: ``Reliability.result()``, nll: ``TemperatureNLL.result()`` or None), the
+  sums all-reduced first when ``comm`` is given."""
+  if comm is not None:
+    reliability.allreduce(comm)
+    if nll is not None:
+      nll.allreduce(comm)
+  return dict(temperature=calibration.temperature, n_bins=calibration.n_bins, reliability=reliability.result(),
+              nll=nll.result() if nll is not None else None)
 
 
 class ScanEvaluator:
@@ -278,11 +359,19 @@ class ScanEvaluator:
   ``Evaluator.finish``.  With ``instances`` (a ``Clustering``) each batch also gets instance ids and feeds a
   ``PanopticQuality`` whose ground-truth instance id is the upper half of the label word (``word >> 16``); only the
   points in a predicted or ground-truth thing segment come back to the host.  ``tta``: a ``tta.TTA`` for the forward
-  (``ScanSegmenter.segment_device(tta=)``)."""
+  (``ScanSegmenter.segment_device(tta=)``).  ``calibration``: a ``calibration.Calibration`` without ``fit`` (the
+  temperature is fitted on pixels, with ``Evaluator``) - each point's confidence at its temperature
+  (``segment_device(confidence=)``) is binned against its label and the ground truth, the "None" class ignored."""
 
-  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None, tta=None):
+  def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None, tta=None,
+               calibration=None):
+    check_tta(calibration, tta)
+    if calibration is not None and calibration.fit:
+      raise ValueError("the temperature is fitted on pixels (Evaluator); point-wise evaluation takes a fixed temperature")
     self.seg = ScanSegmenter(model, fov_up, fov_down)
     self.mc, self.knn, self.instances, self.tta = model.mc, knn, instances, tta
+    self.calibration = calibration
+    self.reliability = Reliability(calibration.n_bins, self.mc.NUM_CLASS) if calibration is not None else None
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self.pq = None
     if instances is not None:
@@ -297,13 +386,16 @@ class ScanEvaluator:
     if batch.get("labels") is None:
       raise ValueError("point-wise evaluation needs the label files")
     res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn,
-                                  instances=self.instances, tta=self.tta)
+                                  instances=self.instances, tta=self.tta,
+                                  confidence=self.calibration.temperature if self.calibration is not None else None)
     n = int(batch["points"].shape[0])
     gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
     lut = self.lut
     _lib.check(_lib.load().pcls_map_labels(ptr(batch["labels"]), n, ptr(lut), int(lut.numel()) if lut is not None else 0,
                                            ptr(gt), stream_handle()), "pcls_map_labels")
     self.miou_tracker.update_state(gt, res["point_labels"])
+    if self.reliability is not None:
+      self.reliability.update_state(res["point_confidence"], res["point_labels"], gt, self.mc.CLASSES.index("None"))
     res["gt"] = gt
     if self.pq is not None:
       self._update_pq(batch, gt, res)
@@ -336,6 +428,8 @@ class ScanEvaluator:
                miou=float(self.miou_tracker.result()), dropped=self.miou_tracker.dropped)
     if self.pq is not None:
       rep["panoptic"] = self.pq.result()
+    if self.calibration is not None:
+      rep["calibration"] = _calibration_report(self.calibration, self.reliability, None, None)
     return rep
 
 

@@ -19,6 +19,11 @@ it is skipped.
 
 With --tta (the mirror image) and / or --tta_shifts (rolls by that many columns, e.g. 0,1024) the forward runs over
 those views of each scan's range image and their averaged probabilities decide the pixel labels (``tta.TTA``).
+
+With --confidence each point's confidence is written next to its ``.label`` file as ``<name>.conf`` (raw float32, one
+per point): the probability at --temperature T that the point's own pixel gives the point's label (0 for a point the
+projection dropped).  With --labels the point-wise reliability report (ECE, MCE, per-bin table) follows the other
+reports.
 """
 import argparse
 import glob
@@ -30,6 +35,7 @@ import numpy as np
 def segment_scans(arg):
   from .dataset_convert import KITTI, ScanBatchLoader, learning_map_lut
   from .inference import load_model_weights
+  from .calibration import Calibration
   from .pipeline import KNN, Clustering, ScanEvaluator
   from .tta import from_args
   from .utils.args_loader import load_model_config
@@ -54,8 +60,12 @@ def segment_scans(arg):
     clustering = Clustering(tau=arg.cluster_tau, rows=arg.cluster_rows, cols=arg.cluster_cols,
                             min_points=arg.min_points, wrap=not arg.no_wrap)
   tta = from_args(arg.tta, arg.tta_shifts)
-  ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering,
-                     tta=tta)
+  cal = Calibration(temperature=arg.temperature, n_bins=arg.bins) if arg.confidence else None
+  try:
+    ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering,
+                       tta=tta, calibration=cal)
+  except ValueError as e:
+    raise SystemExit(str(e))
   os.makedirs(arg.output_dir, exist_ok=True)
   loader = ScanBatchLoader(arg.format)
   for i in range(0, len(scans), arg.batch):
@@ -65,7 +75,11 @@ def segment_scans(arg):
       res = ev.update(data)
     else:
       res = ev.seg.segment_device(data["points"], data["offsets"], want_point_labels=True, knn=ev.knn,
-                                  instances=clustering, tta=tta)
+                                  instances=clustering, tta=tta, confidence=cal.temperature if cal else None)
+    if cal is not None:
+      pc = res["point_confidence"].cpu().numpy()
+      for f, c in zip(files, np.split(pc, np.cumsum(data["sizes"])[:-1])):
+        c.astype(np.float32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".conf"))
     if clustering is not None:
       for f, words in zip(files, ev.seg.label_words(res, data["sizes"], inv)):
         words.tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
@@ -92,6 +106,9 @@ def segment_scans(arg):
     print("no panoptic report: nuScenes lidarseg label files carry no instance ids")
   elif clustering is not None:
     print_panoptic(rep["panoptic"], config.CLASSES)
+  if cal is not None:
+    from .eval import print_reliability
+    print_reliability(rep["calibration"]["reliability"], cal.temperature, "points")
   return rep
 
 
@@ -127,6 +144,10 @@ def main(argv=None):
   ap.add_argument("--learning_map", default=None, help="yaml with `learning_map` / `learning_map_inv` (semantic-kitti.yaml)")
   from .tta import add_tta_flags
   add_tta_flags(ap)
+  from .calibration import add_temperature_flag
+  ap.add_argument("--confidence", action="store_true", help="also write <name>.conf: float32 confidence per point")
+  add_temperature_flag(ap)
+  ap.add_argument("--bins", type=int, default=15, help="reliability bins of the --labels report (1..64)")
   return segment_scans(ap.parse_args(argv))
 
 

@@ -82,6 +82,13 @@ class Communicator:
       dist.all_reduce(metric._cmw, op=dist.ReduceOp.SUM)
     dist.all_reduce(metric._dropped, op=dist.ReduceOp.SUM)
 
+  def allreduce_sums(self, tensors):
+    """In-place sum of each tensor over all ranks with ``torch.distributed`` (small accumulators, off the hot path)."""
+    if self.world_size == 1:
+      return
+    for t in tensors:
+      dist.all_reduce(t, op=dist.ReduceOp.SUM)
+
   def close(self):
     if self._comm is not None:
       _lib.load().pcls_comm_destroy(self._comm)
