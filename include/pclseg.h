@@ -235,6 +235,48 @@ int pcls_point_confidence(const float* probs, const int64_t* offsets, int B, int
                           const int32_t* proj_x, const int32_t* proj_y, const int32_t* point_labels, int num_classes,
                           float* out_conf, pcls_stream stream);
 
+/* Monte-Carlo dropout (Gal & Ghahramani, ICML 2016; Kendall et al., Bayesian SegNet, 2015): T forward passes of a
+ * stochastic net whose Dropout layers are active; the mean probabilities, the predictive entropy and the mutual
+ * information between prediction and weights.  No reference call site: the reference's Dropout layers act in training only.
+ * Dropout site: one Dropout call of the model, numbered in trace order (SqueezeSegV2: site 0 = fire13 + conv1_skip, 64
+ * channels at full width; Darknet: sites 0-4 = the outputs of enc1 .. enc5, site 5 = the input of head).  A site modifies
+ * its tensor IN PLACE: every later reader sees the dropped tensor.
+ * Mask: element e = (h * W_t + w) * C + c of frame f's tensor (C a multiple of 8), pass t (0 <= t < 65536), site k
+ *   (0 <= k < 65536), f the GLOBAL frame id = frame_base + the frame's index in the forward call (micro-batch passes
+ *   counted).  Philox4x32-10 (Salmon et al., SC 2011) with counter (g, k | t << 16, lo32(f), hi32(f)), g = e / 8, and key
+ *   (lo32(seed), hi32(seed)); output word i (0..3) gives u (16 bits) to two elements: its low half to element 8g + 2i,
+ *   its high half to element 8g + 2i + 1.  thr = floor(rate * 65536 + 0.5) in float64 (0 <= rate, thr < 65536, else
+ *   PCLS_ERR_INVALID); the element is kept iff u >= thr, and then becomes round16_rn(fl32(x) * scale) with
+ *   scale = (float)(65536.0 / (65536 - thr)) (computed in float64, rounded once, the product rounded to float32); a
+ *   dropped element becomes the bit pattern 0.  At rate 0 the tensor is bit-for-bit unchanged.  The mask of a frame
+ *   depends only on (seed, global frame id, pass, site): not on the batch, the micro batch, graph replay or the number of
+ *   GPUs.  Parity with TensorFlow's dropout RNG is not claimed.
+ * pcls_net_dropout (before pcls_net_finalize): appends the in-place dropout of activation `tensor` as site `site` at
+ *   `rate` to the op list.  Refused (PCLS_ERR_INVALID): the network input or a logits tensor, a tensor no earlier op
+ *   writes, channels not a multiple of 8 or a pixel stride other than the channel count (the 48 -> 64 padded tensors), a
+ *   site used twice, an invalid rate; pcls_net_finalize refuses a site tensor the planner fuses away.  The op is listed
+ *   by pcls_net_num_ops / pcls_net_op_info / pcls_net_profile_ops like any other.
+ * pcls_net_set_dropout: writes the net's device-side (seed, frame_base, pass) with a one-thread kernel on `stream`,
+ *   outside the forward's CUDA graph: the dropout kernels read it, so one captured graph serves every pass and batch.
+ *   Needs a finalized net with at least one dropout op and 0 <= pass < 65536.  The state starts as (0, 0, 0).
+ * pcls_mc_accumulate: probs [n,NC] f32 of pass `pass`; h_t = the normalised entropy of probs as pcls_confidence computes
+ *   it.  pass 0: acc_probs [n,NC] f32 = probs, acc_entropy [n] f64 = (double)h_0; pass > 0: acc_probs = fl32(acc_probs +
+ *   probs) (round to nearest), acc_entropy += (double)h_t.  Passes are accumulated in the order of the calls.
+ * pcls_mc_finalize over n_passes = T (1 .. 65536): mean = acc_probs / T (__fdiv_rn; T = 1 leaves acc_probs unchanged);
+ *   out_preds [n] i32 = argmax of mean (first index on ties, the head's rule), none_index where mask == 0 (mask [n] u8,
+ *   NULL = all valid); out_conf [n] f32 = max mean; out_entropy [n] f32 = H, the normalised entropy of mean by the same
+ *   rule as h_t; out_mi [n] f32 = max(0, fl32(H - EH)) with EH = (float)(acc_entropy / T); conf / H / MI are 0 where
+ *   mask == 0; out_probs [n,NC] f32 = mean, written for every pixel as the head does.  Each output may be NULL, at least
+ *   one must be given.  At rate 0 with T = 1 or 2, mean and preds are the plain forward's bits and MI is 0; from T = 3
+ *   on the running float32 sum rounds (3p is not exact), so the mean is within a few ulp of the plain probabilities.
+ * Both calls check every argument before any launch (1 <= num_classes <= 32, 0 <= none_index < num_classes, the pointers
+ * the call needs); n == 0 is a no-op.  pcls_net_dropout / pcls_net_set_dropout are declared with the net below. */
+int pcls_mc_accumulate(const float* probs, int64_t n, int num_classes, int pass, float* acc_probs, double* acc_entropy,
+                       pcls_stream stream);
+int pcls_mc_finalize(const float* acc_probs, const double* acc_entropy, const uint8_t* mask, int64_t n, int num_classes,
+                     int none_index, int n_passes, float* out_probs, int32_t* out_preds, float* out_conf,
+                     float* out_entropy, float* out_mi, pcls_stream stream);
+
 /* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
  * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,
@@ -468,6 +510,10 @@ int64_t pcls_net_workspace_bytes(const pcls_net* net);
  *                needs a library built with PCLS_NVCC_FLAGS=-DPCLS_TC_DEBUG=1
  * Any other name fails with PCLS_ERR_INVALID. */
 int pcls_net_set_option(pcls_net* net, const char* name, int value);
+
+/* MC dropout ops of a stochastic net (the rules are stated with pcls_mc_accumulate above). */
+int pcls_net_dropout(pcls_net* net, int tensor, int site, double rate);
+int pcls_net_set_dropout(pcls_net* net, uint64_t seed, uint64_t frame_base, int pass, pcls_stream stream);
 
 #ifdef __cplusplus
 }

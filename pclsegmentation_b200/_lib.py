@@ -61,6 +61,11 @@ SIGNATURES = {
                                       c_void_p, c_void_p]),
   "pcls_point_confidence": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p,
                                     c_int, c_void_p, c_void_p]),
+  "pcls_net_dropout": (c_int, [c_void_p, c_int, c_int, c_double]),
+  "pcls_net_set_dropout": (c_int, [c_void_p, c_uint64, c_uint64, c_int, c_void_p]),
+  "pcls_mc_accumulate": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+  "pcls_mc_finalize": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                               c_void_p, c_void_p, c_void_p]),
   "pcls_map_labels":(c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
   "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

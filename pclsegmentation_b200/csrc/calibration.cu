@@ -63,13 +63,7 @@ confidence_kernel(const float* __restrict__ src, bool is_logits, const uint8_t* 
       for (int c = 0; c < CAL_MAX_NC; ++c) if (c == best) top = v[c];   // no dynamic index: v stays in registers
       const bool valid = mask == nullptr || mask[p0 + lane] != 0;
       if (out_conf != nullptr) out_conf[p0 + lane] = valid ? top : 0.0f;
-      if (out_entropy != nullptr) {
-        float h = 0.0f;
-#pragma unroll
-        for (int c = 0; c < CAL_MAX_NC; ++c)
-          if (c < nc && v[c] > 0.0f) h = __fadd_rn(h, __fmul_rn(v[c], logf(v[c])));
-        out_entropy[p0 + lane] = valid && nc > 1 ? __fdiv_rn(-h, log_nc) : 0.0f;
-      }
+      if (out_entropy != nullptr) out_entropy[p0 + lane] = valid ? normalised_entropy<CAL_MAX_NC>(v, nc, log_nc) : 0.0f;
       if (out_probs != nullptr && is_logits) {
 #pragma unroll
         for (int c = 0; c < CAL_MAX_NC; ++c) if (c < nc) t[lane * pitch + c] = v[c];

@@ -311,6 +311,37 @@ int Net::add_cam(const pcls_cam_desc& d) {
   return PCLS_OK;
 }
 
+// MC dropout site: the tensor must already be written (a site modifies it in place; every later reader sees the dropped
+// values), 16-bit with a dense pixel stride, channels a multiple of 8 (one 16-byte vector = 8 elements = one Philox call).
+int Net::add_dropout(int t, int site, double rate) {
+  PCLS_REQUIRE(!finalized, "pcls_net_dropout: net already finalized");
+  PCLS_REQUIRE(t >= 1 && t < (int)tensors.size(), "pcls_net_dropout: bad tensor id %d (the network input is not a site)", t);
+  const TensorInfo& ti = tensors[t];
+  PCLS_REQUIRE(!ti.logits, "pcls_net_dropout: tensor %d is a logits tensor", t);
+  PCLS_REQUIRE(ti.channels % 8 == 0 && ti.stride == ti.channels,
+               "pcls_net_dropout: tensor %d has %d channels with pixel stride %d (needs a multiple of 8, stride == channels)",
+               t, ti.channels, ti.stride);
+  PCLS_REQUIRE((int64_t)H * ti.width * ti.channels / 8 < (1ll << 31), "pcls_net_dropout: tensor %d is too large", t);
+  bool written = false;
+  std::vector<int> rd, wr;
+  for (const OpRef& op : ops) {
+    op_tensors(op, rd, wr);
+    for (int w : wr) written = written || w == t;
+  }
+  PCLS_REQUIRE(written, "pcls_net_dropout: tensor %d is not written by any op before this one", t);
+  PCLS_REQUIRE(site >= 0 && site < 65536, "pcls_net_dropout: site %d not in [0,65536)", site);
+  for (const auto& D : dropouts) PCLS_REQUIRE(D.site != site, "pcls_net_dropout: site %d is used twice", site);
+  PCLS_REQUIRE(std::isfinite(rate) && rate >= 0.0, "pcls_net_dropout: rate %g must be finite and >= 0", rate);
+  const double thr = std::floor(rate * 65536.0 + 0.5);
+  PCLS_REQUIRE(thr < 65536.0, "pcls_net_dropout: rate %g drops every element (round(rate * 65536) = %.0f)", rate, thr);
+  DropoutLayer D;
+  D.tensor = t; D.site = site; D.thr = (uint32_t)thr;
+  D.scale = (float)(65536.0 / (65536.0 - thr));
+  dropouts.push_back(D);
+  ops.push_back({OP_DROPOUT, (int)dropouts.size() - 1});
+  return PCLS_OK;
+}
+
 void Net::op_tensors(const OpRef& op, std::vector<int>& reads, std::vector<int>& writes) const {
   reads.clear(); writes.clear();
   if (op.type == OP_CONV) {
@@ -325,6 +356,8 @@ void Net::op_tensors(const OpRef& op, std::vector<int>& reads, std::vector<int>&
     writes.push_back(L.out);
   } else if (op.type == OP_POOL) {
     reads.push_back(pools[op.index].in); writes.push_back(pools[op.index].out);
+  } else if (op.type == OP_DROPOUT) {
+    reads.push_back(dropouts[op.index].tensor); writes.push_back(dropouts[op.index].tensor);
   } else {
     reads.push_back(cams[op.index].in); writes.push_back(cams[op.index].out);
   }
@@ -411,6 +444,14 @@ int Net::finalize(int logits_tensor_, int num_classes_, int none_index_) {
       E.skip_src = ops[i].index;
       P.skip_into = ops[reader].index;
     }
+  // a dropout op reads its tensor, so no fusion above takes it away; checked all the same, a fused tensor is never written
+  for (const auto& D : dropouts) {
+    bool fused = false;
+    for (const auto& L : convs)
+      fused = fused || ((L.skip_into >= 0 || (conv_impl == 0 && L.fused_into_up >= 0)) && L.out == D.tensor);
+    for (const auto& P : pools) fused = fused || (P.fused_conv >= 0 && P.out == D.tensor);
+    PCLS_REQUIRE(!fused, "pcls_net_finalize: dropout site %d: tensor %d is fused away by the planner", D.site, D.tensor);
+  }
   // liveness: first write .. last read (op order); the logits tensor lives to the end (head reads it)
   std::vector<int> reads, writes;
   for (auto& t : tensors) { t.first = -1; t.last = -1; }
@@ -512,6 +553,10 @@ int Net::finalize(int logits_tensor_, int num_classes_, int none_index_) {
     L.p.w1 = base; L.p.w2 = base + L.C * L.R; L.p.b1 = L.p.w2 + L.R * L.C; L.p.b2 = L.p.b1 + L.R;
     off += align_up(L.h.size() * 4, 256);
   }
+  if (!dropouts.empty()) {
+    PCLS_CHECK_CUDA(cudaMalloc(&drop_state, sizeof(DropState)));
+    PCLS_CHECK_CUDA(cudaMemset(drop_state, 0, sizeof(DropState)));
+  }
   int rc = tc_prepare();
   if (rc != PCLS_OK) return rc;
   finalized = true;
@@ -526,7 +571,7 @@ void* Net::tensor_ptr(int t, int frames) const {
 
 template <typename T>
 int Net::run_pass(const float* lidar, int channels, const uint8_t* mask, bool raw, const double* mean5,
-                  const double* std5, int nb, float* logits, float* probs, int32_t* preds, cudaStream_t s,
+                  const double* std5, int b0, int nb, float* logits, float* probs, int32_t* preds, cudaStream_t s,
                   cudaEvent_t* ev) {
   const int64_t n_pixels = (int64_t)nb * H * W;
   pdl_early_now = (pdl_mode && n_pixels <= pdl_early_px) ? 1 : 0;   // small passes: latency mode (common.cuh)
@@ -586,6 +631,11 @@ int Net::run_pass(const float* lidar, int channels, const uint8_t* mask, bool ra
         }
       }
       else rc = launch_conv_direct<T>(p, nb, s);
+    } else if (op.type == OP_DROPOUT) {
+      const DropoutLayer& D = dropouts[op.index];
+      const TensorInfo& ti = tensors[D.tensor];
+      const int64_t vpf = (int64_t)H * ti.width * ti.channels / 8;
+      rc = launch_dropout<T>(tensor_ptr(D.tensor, nb), vpf * nb, vpf, D.site, D.thr, D.scale, drop_state, b0, s);
     } else if (op.type == OP_POOL) {
       const PoolLayer& L = pools[op.index];
       if (conv_impl == 0 && L.fused_conv >= 0) continue;   // pooled on the fly by the 1x1 conv behind it
@@ -628,8 +678,8 @@ int Net::run_all(const float* lidar, int channels, const uint8_t* mask, bool raw
     float* lg = logits ? logits + (size_t)b0 * px * num_classes : nullptr;
     float* pr = probs ? probs + (size_t)b0 * px * num_classes : nullptr;
     int32_t* pd = preds + (size_t)b0 * px;
-    int rc = (precision == PCLS_F16) ? run_pass<__half>(l, channels, m, raw, mean5, std5, nb, lg, pr, pd, s, ev)
-                                     : run_pass<__nv_bfloat16>(l, channels, m, raw, mean5, std5, nb, lg, pr, pd, s, ev);
+    int rc = (precision == PCLS_F16) ? run_pass<__half>(l, channels, m, raw, mean5, std5, b0, nb, lg, pr, pd, s, ev)
+                                     : run_pass<__nv_bfloat16>(l, channels, m, raw, mean5, std5, b0, nb, lg, pr, pd, s, ev);
     if (rc) return rc;
   }
   return PCLS_OK;
@@ -799,6 +849,11 @@ int Net::op_info(int i, char* name, int* family, int64_t* flops, int64_t* bytes)
              ((int64_t)Q.cin_logical * Q.cout_logical + (int64_t)p.ntaps * cin * cout) * 2;
         fam = 0;
       }
+    } else if (op.type == OP_DROPOUT) {
+      const DropoutLayer& D = dropouts[op.index];
+      const TensorInfo& ti = tensors[D.tensor];
+      snprintf(buf, sizeof(buf), "dropout_s%d_c%d_w%d", D.site, ti.channels, ti.width);
+      by = (int64_t)H * ti.width * ti.channels * 2 * 2;   // read and written in place
     } else if (op.type == OP_POOL) {
       const PoolLayer& L = pools[op.index];
       const bool fused = conv_impl == 0 && L.fused_conv >= 0;
@@ -835,6 +890,7 @@ Net::~Net() {
   if (cap_stream) cudaStreamDestroy(cap_stream);
   if (arena) cudaFree(arena);
   if (weights) cudaFree(weights);
+  if (drop_state) cudaFree(drop_state);
   tc_release();
 }
 
@@ -881,6 +937,19 @@ extern "C" int pcls_net_maxpool3x3_s2(pcls_net* net, int in_tensor, int out_tens
 extern "C" int pcls_net_cam(pcls_net* net, const pcls_cam_desc* desc) {
   PCLS_REQUIRE(net != nullptr && desc != nullptr, "pcls_net_cam: NULL argument");
   return reinterpret_cast<Net*>(net)->add_cam(*desc);
+}
+
+extern "C" int pcls_net_dropout(pcls_net* net, int tensor, int site, double rate) {
+  PCLS_REQUIRE(net != nullptr, "pcls_net_dropout: NULL net");
+  return reinterpret_cast<Net*>(net)->add_dropout(tensor, site, rate);
+}
+
+extern "C" int pcls_net_set_dropout(pcls_net* net, uint64_t seed, uint64_t frame_base, int pass, pcls_stream stream) {
+  Net* n = reinterpret_cast<Net*>(net);
+  PCLS_REQUIRE(n != nullptr && n->finalized, "pcls_net_set_dropout: net is NULL or not finalized");
+  PCLS_REQUIRE(n->drop_state != nullptr, "pcls_net_set_dropout: the net has no dropout op (pcls_net_dropout)");
+  PCLS_REQUIRE(pass >= 0 && pass < 65536, "pcls_net_set_dropout: pass %d not in [0,65536)", pass);
+  return launch_set_dropout(n->drop_state, seed, frame_base, (unsigned)pass, (cudaStream_t)stream);
 }
 
 extern "C" int pcls_net_finalize(pcls_net* net, int logits_tensor, int num_classes, int none_index) {

@@ -50,7 +50,10 @@ struct CamLayer {
   CamParams p;
 };
 
-enum OpType { OP_CONV = 0, OP_POOL = 1, OP_CAM = 2 };
+// In-place MC dropout of one tensor (mc_dropout.cu); only in a net built with pcls_net_dropout.
+struct DropoutLayer { int tensor, site; uint32_t thr; float scale; };
+
+enum OpType { OP_CONV = 0, OP_POOL = 1, OP_CAM = 2, OP_DROPOUT = 3 };
 struct OpRef { int type, index; };
 
 constexpr int kIn16 = 0x100;   // OR-ed into `channels` inside the library: the input is 16-bit (pcls_net_forward_in16)
@@ -68,6 +71,7 @@ struct Net {
   std::vector<ConvLayer> convs;
   std::vector<PoolLayer> pools;
   std::vector<CamLayer> cams;
+  std::vector<DropoutLayer> dropouts;
   std::vector<OpRef> ops;
   bool finalized = false;
   int logits_tensor = -1, num_classes = 0, none_index = 0;
@@ -93,6 +97,7 @@ struct Net {
   uint64_t graph_clock = 0;
   int graph_misses = 0;       // consecutive forwards whose argument set was not in the graph cache
   cudaStream_t cap_stream = nullptr;
+  DropState* drop_state = nullptr;   // (seed, frame_base, pass) of the dropout ops, written by pcls_net_set_dropout
 
   ~Net();
   int add_tensor(int width, int channels, bool logits);
@@ -102,12 +107,13 @@ struct Net {
   void build_deconv_row3(ConvLayer& L);
   int add_pool(int in, int out);
   int add_cam(const pcls_cam_desc& d);
+  int add_dropout(int tensor, int site, double rate);
   void op_tensors(const OpRef& op, std::vector<int>& reads, std::vector<int>& writes) const;
   int finalize(int logits_tensor, int num_classes, int none_index);
   void* tensor_ptr(int t, int frames) const;
   template <typename T>
   int run_pass(const float* lidar, int channels, const uint8_t* mask, bool raw, const double* mean5, const double* std5,
-               int nb, float* logits, float* probs, int32_t* preds, cudaStream_t s, cudaEvent_t* ev);
+               int b0, int nb, float* logits, float* probs, int32_t* preds, cudaStream_t s, cudaEvent_t* ev);
   int run_all(const float* lidar, int channels, const uint8_t* mask, bool raw, const double* mean5, const double* std5,
               int B, float* logits, float* probs, int32_t* preds, cudaStream_t s, cudaEvent_t* ev);
   void drop_graphs();

@@ -107,6 +107,26 @@ __device__ __forceinline__ int softmax_argmax(float (&v)[MAXNC], int nc) {
   return best;
 }
 
+// Normalised entropy of probabilities v[0..nc): (-sum_c v_c * logf(v_c)) over the classes with v_c > 0, summed in class
+// order in float32 with every product and sum rounded on its own, divided by log_nc = logf(nc); 0 when nc = 1.  Shared by
+// pcls_confidence (calibration.cu) and the MC-dropout accumulate / finalize (mc_dropout.cu).
+template <int MAXNC>
+__device__ __forceinline__ float normalised_entropy(const float (&v)[MAXNC], int nc, float log_nc) {
+  float h = 0.0f;
+#pragma unroll
+  for (int c = 0; c < MAXNC; ++c)
+    if (c < nc && v[c] > 0.0f) h = __fadd_rn(h, __fmul_rn(v[c], logf(v[c])));
+  return nc > 1 ? __fdiv_rn(-h, log_nc) : 0.0f;
+}
+
+// MC dropout (mc_dropout.cu): one in-place dropout op of the forward; `state` is the net's device-side
+// (seed, frame_base, pass), written by pcls_net_set_dropout.  n_vec / vec_per_frame count 16-byte vectors.
+struct DropState { unsigned long long seed, frame_base; unsigned int pass; };
+template <typename T> int launch_dropout(void* data, int64_t n_vec, int64_t vec_per_frame, int site, uint32_t thr,
+                                         float scale, const DropState* state, int b0, cudaStream_t s);
+int launch_set_dropout(DropState* state, unsigned long long seed, unsigned long long frame_base, unsigned pass,
+                       cudaStream_t s);
+
 // 16-bit <-> float helpers
 template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }

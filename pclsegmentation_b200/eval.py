@@ -22,6 +22,7 @@ import numpy as np
 
 from .inference import load_model_weights
 from .calibration import Calibration, add_temperature_flag
+from .mc_dropout import add_mc_flags, from_args as mc_from_args
 from .pipeline import Evaluator, shard_files
 from .tta import add_tta_flags, from_args
 from .utils.args_loader import load_model_config
@@ -30,7 +31,7 @@ from .utils.args_loader import load_model_config
 def evaluation(arg):
   import torch
   import torch.distributed as dist
-  from .sharding import Communicator, env_rank
+  from .sharding import Communicator, env_rank, shard_range
   rank, local_rank, world = env_rank()
   torch.cuda.set_device(local_rank)
   comm = None
@@ -42,13 +43,18 @@ def evaluation(arg):
   config.DATA_AUGMENTATION = False
   load_model_weights(model, arg, verbose=rank == 0)
 
-  files = shard_files(glob.glob(os.path.join(arg.data_path, arg.image_set, "*.npy")), comm)
+  all_files = glob.glob(os.path.join(arg.data_path, arg.image_set, "*.npy"))
+  files = shard_files(all_files, comm)
   tta = from_args(arg.tta, arg.tta_shifts)
+  mcd = mc_from_args(arg)
+  if mcd is not None and comm is not None:
+    # the rank's first frame keeps its single-GPU global id: the same masks, so the same integer histograms
+    mcd.next_frame = shard_range(len(all_files), comm.rank, comm.world_size)[0]
   cal = None
   if arg.calibration or arg.fit_temperature or arg.calibration_json:
     cal = Calibration(temperature=arg.temperature, n_bins=arg.bins, fit=arg.fit_temperature)
   try:
-    ev = Evaluator(model, comm, tta=tta, calibration=cal)
+    ev = Evaluator(model, comm, tta=tta, calibration=cal, mc_dropout=mcd)
   except ValueError as e:
     raise SystemExit(str(e))
   if rank == 0:
@@ -70,6 +76,8 @@ def evaluation(arg):
       print("Precision: " + str(rep["precision"][i]))
       print("")
     print("MIoU: {} ".format(rep["miou"]))
+    if mcd is not None:
+      print_mc_report(rep["mc_dropout"], "pixels")
   if cal is not None:
     calib = rep["calibration"]
     if rank == 0:
@@ -97,6 +105,17 @@ def evaluation(arg):
     comm.close()
     dist.destroy_process_group()
   return rep
+
+
+def print_mc_report(m, what):
+  """The MC-dropout report: T, rate, seed, the AUROC of H and MI for detecting errors, ECE / MCE of the mean."""
+  u, r = m["uncertainty"], m["reliability"]
+  print("MC DROPOUT T = %d, rate = %g, seed = %d (%d %s, %d errors)" % (m["passes"], m["rate"], m["seed"], u["count"],
+                                                                        what, u["errors"]))
+  print("AUROC(H):        %.6f" % u["auroc_entropy"])
+  print("AUROC(MI):       %.6f" % u["auroc_mi"])
+  print("ECE (mean conf): %.6f" % r["ece"])
+  print("MCE (mean conf): %.6f" % r["mce"])
 
 
 def print_reliability(r, temperature, what):
@@ -138,6 +157,7 @@ def main(argv=None):
   parser.add_argument('-b', '--batch', type=int, default=8, help='frames per forward call (the reference uses 1)')
   parser.add_argument('--random_init', action='store_true', help='run without --path_to_model on Keras-default weights')
   add_tta_flags(parser)
+  add_mc_flags(parser)
   parser.add_argument('--calibration', action='store_true',
                       help='print the reliability of the confidences (ECE, MCE, per-bin table) at --temperature')
   parser.add_argument('--fit_temperature', action='store_true',

@@ -14,9 +14,11 @@ import glob
 import os
 
 import numpy as np
+import torch
 
 from .calibration import add_temperature_flag, confidence, raw_mask
 from .device import samples_to_device
+from .mc_dropout import add_mc_flags, check_exclusive, forward_mc, from_args as mc_from_args
 from .tta import add_tta_flags, forward_tta, from_args
 from .utils.args_loader import load_model_config
 from .utils.util import normalize
@@ -50,18 +52,32 @@ def inference(arg):
   tta = from_args(arg.tta, arg.tta_shifts)
   if arg.confidence and tta is not None and arg.temperature != 1.0:
     raise SystemExit("--tta merges probabilities, not logits: --confidence with --tta needs --temperature 1")
+  mcd = mc_from_args(arg)
+  if mcd is not None:
+    if arg.confidence and arg.temperature != 1.0:
+      raise SystemExit("MC dropout cannot be combined with a softmax temperature: --confidence needs --temperature 1")
+    try:
+      check_exclusive(mcd, tta)
+    except ValueError as e:
+      raise SystemExit(str(e))
   files = sorted(glob.iglob(arg.input_path))
   for i in range(0, len(files), arg.batch):
     chunk = files[i:i + arg.batch]
     samples = np.stack([np.load(f) for f in chunk])          # float64 on disk: uploaded as is, narrowed on the device
     x = samples_to_device(samples)
-    if tta is not None:
+    unc = None
+    if mcd is not None:
+      res = forward_mc(model, x, mcd)
+      unc = torch.stack([res["entropy"], res["mutual_information"]], dim=-1).cpu().numpy()   # [B,H,W,2]: H, MI
+    elif tta is not None:
       res = forward_tta(model, x, tta, want_probabilities=arg.confidence)
     else:
       res = model.forward_device(x, None, mean=config.INPUT_MEAN, std=config.INPUT_STD, want_probabilities=False,
                                  want_logits=arg.confidence)
     conf = None
-    if arg.confidence:
+    if arg.confidence and mcd is not None:
+      conf = res["confidence"].cpu().numpy()
+    elif arg.confidence:
       src = dict(probs=res["probabilities"]) if tta is not None else dict(logits=res["logits"])
       conf = confidence(config.NUM_CLASS, mask=raw_mask(x, config), temperature=arg.temperature,
                         **src)["confidence"].cpu().numpy()
@@ -72,6 +88,8 @@ def inference(arg):
       np.save(os.path.join(arg.output_dir, 'pred_' + file_name + '.npy'), pred)
       if conf is not None:
         np.save(os.path.join(arg.output_dir, 'conf_' + file_name + '.npy'), conf[k])
+      if unc is not None:
+        np.save(os.path.join(arg.output_dir, 'unc_' + file_name + '.npy'), unc[k])
       if arg.no_plots:
         continue
       from PIL import Image
@@ -100,6 +118,7 @@ def main(argv=None):
   parser.add_argument('--no_plots', action='store_true', help='only write pred_*.npy')
   parser.add_argument('--random_init', action='store_true', help='run without --path_to_model on Keras-default weights')
   add_tta_flags(parser)
+  add_mc_flags(parser)
   parser.add_argument('--confidence', action='store_true',
                       help='also write conf_<name>.npy: float32 [H,W] max softmax(logits / T) per pixel, 0 at empty pixels')
   add_temperature_flag(parser)

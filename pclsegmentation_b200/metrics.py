@@ -149,6 +149,51 @@ class Reliability:
     return reliability_scores(cnt, cor, cs)
 
 
+class UncertaintyAUROC:
+  """How well an uncertainty u in [0, 1] detects misclassified elements, as a binned AUROC: ``n_bins`` equal bins of u
+  hold the number of elements and of correct ones (pcls_reliability_update with u as the "confidence", so pixels and
+  points share the kernel and its counting rule).  AUROC = P(u_error > u_correct) over (error, correct) pairs, a pair in
+  the same bin counted 1/2; 0.5 when there are no errors or nothing correct.  Two uncertainties are tracked: the
+  normalised predictive entropy H and the normalised mutual information MI of MC dropout."""
+
+  def __init__(self, num_classes, n_bins=64):
+    self.entropy = Reliability(n_bins, num_classes)
+    self.mutual_information = Reliability(n_bins, num_classes)
+
+  def update_state(self, entropy, mutual_information, pred, label, ignore_index=-1):
+    self.entropy.update_state(entropy, pred, label, ignore_index)
+    self.mutual_information.update_state(mutual_information, pred, label, ignore_index)
+
+  def allreduce(self, comm):
+    self.entropy.allreduce(comm)
+    self.mutual_information.allreduce(comm)
+
+  def result(self):
+    """dict(auroc_entropy, auroc_mi, count, errors, and the integer bins: entropy_count / entropy_correct / mi_count /
+    mi_correct)."""
+    out = {}
+    for key, r in (("entropy", self.entropy), ("mi", self.mutual_information)):
+      r._ensure()
+      cnt, cor = r.count.cpu().numpy(), r.correct.cpu().numpy()
+      out["auroc_" + key] = binned_auroc(cnt, cor)
+      out[key + "_count"], out[key + "_correct"] = cnt, cor
+    out["count"] = int(out["entropy_count"].sum())
+    out["errors"] = int(out["entropy_count"].sum() - out["entropy_correct"].sum())
+    return out
+
+
+def binned_auroc(count, correct):
+  """AUROC of u for detecting errors from its histogram (per bin: elements, correct ones); see UncertaintyAUROC."""
+  count = np.asarray(count, np.float64)
+  correct = np.asarray(correct, np.float64)
+  err = count - correct
+  n_err, n_ok = err.sum(), correct.sum()
+  if n_err == 0 or n_ok == 0:
+    return 0.5
+  below_ok = np.concatenate([[0.0], np.cumsum(correct)[:-1]])
+  return float((err * (below_ok + 0.5 * correct)).sum() / (n_err * n_ok))
+
+
 def reliability_scores(count, correct, conf_sum):
   """The scores of ``Reliability.result`` from the three per-bin sums (host, float64)."""
   count = np.asarray(count, np.int64)

@@ -49,6 +49,7 @@ class PCLSegmentationNetwork:
     self._taps = {}          # name -> symbolic tensor, recorded by call() (per-layer parity tests, see read_tap)
     self._net = None
     self._net_batch = 0
+    self._mc_nets = {}       # dropout rate -> (stochastic pcls_net handle, its batch capacity); see mc_net
     self._pinned = {}
 
   # ---- the subclass provides call(); tracing it builds the op program and creates the variables ----
@@ -63,15 +64,17 @@ class PCLSegmentationNetwork:
     self._taps[name] = x
     return x
 
-  def read_tap(self, name, batch):
-    """float32 CUDA copy [batch,H,width,channels] of a tapped intermediate of the LAST forward.  Intermediates share a
-    liveness-planned arena, so this is only meaningful with set_option("keep_tensors", 1)."""
+  def read_tap(self, name, batch, net=None):
+    """float32 CUDA copy [batch,H,width,channels] of a tapped intermediate of the LAST forward (of ``net``, e.g. an
+    ``mc_net`` handle; default: the default net).  Intermediates share a liveness-planned arena, so this is only
+    meaningful with set_option("keep_tensors", 1)."""
     if not self.net_options.get("keep_tensors"):
       raise _lib.PclsError("read_tap needs set_option('keep_tensors', 1) before the forward")
     sym = self._taps[name]
     out = torch.empty((batch, self.ZENITH_LEVEL, sym.width, sym.channels), dtype=torch.float32,
                       device=torch.device("cuda", torch.cuda.current_device()))
-    _lib.check(_lib.load().pcls_net_read_tensor(self._net, sym.tid, batch, ptr(out), stream_handle()),
+    _lib.check(_lib.load().pcls_net_read_tensor(self._net if net is None else net, sym.tid, batch, ptr(out),
+                                                stream_handle()),
                "pcls_net_read_tensor")
     return out
 
@@ -156,6 +159,9 @@ class PCLSegmentationNetwork:
     if self._net is not None:
       _lib.load().pcls_net_destroy(self._net)
       self._net, self._net_batch = None, 0
+    for handle, _ in self._mc_nets.values():
+      _lib.load().pcls_net_destroy(handle)
+    self._mc_nets.clear()
 
   def __del__(self):
     try:
@@ -177,6 +183,23 @@ class PCLSegmentationNetwork:
                                         cap, self.net_options)
       self._net_batch = cap
     return self._net
+
+  def mc_net(self, rate, batch):
+    """The stochastic net of MC dropout (``mc_dropout.forward_mc``): the same program, variables and ``net_options``
+    as the default net plus one in-place dropout op per Dropout call of the model (``rate``: one float, or one per
+    site).  Built on first use and cached by rate; the default net is not touched."""
+    key = tuple(rate) if hasattr(rate, "__len__") else float(rate)
+    handle, cap = self._mc_nets.get(key, (None, 0))
+    if handle is None or batch > cap:
+      if handle is not None:
+        _lib.load().pcls_net_destroy(handle)
+        del self._mc_nets[key]
+      require_cuda()
+      cap = max(batch, 1)
+      handle = self._graph.build_net(self._logits_sym, self.NUM_CLASS, self.CLASSES.index("None"), self.precision, cap,
+                                     self.net_options, dropout_rate=rate)
+      self._mc_nets[key] = (handle, cap)
+    return handle
 
   def forward_device(self, lidar, mask=None, mean=None, std=None, want_probabilities=True, want_logits=False,
                      out=None):

@@ -45,6 +45,7 @@ class Graph:
     self.H, self.W = H, W
     self.variables = {}     # name -> np.float32 array (Keras layout)
     self.program = []       # ops in execution order
+    self.dropout_sites = []  # (sym, rate, op it follows) per Dropout call, in trace order (MC dropout sites)
     self.rng = np.random.default_rng(0)
     self.merge_expand = True  # fuse Fire expand1x1 || expand3x3 into one convolution (see concat)
     self.input = Sym(self, W, 8, is_input=True)
@@ -161,6 +162,16 @@ class Graph:
     bn = [cat(a["bn"] + s, b["bn"] + s) for s in ("/gamma", "/beta", "/moving_mean", "/moving_variance")] if a["bn"] else [None] * 4
     return [kernel, bias] + bn
 
+  def dropout(self, x, rate):
+    """Records a Dropout call as an MC dropout site and returns ``x``: the traced program does not change.  A net built
+    with a ``dropout_rate`` drops ``x`` in place right after the last op traced so far (the op object is recorded, not
+    its index, so that a later merge of program entries cannot move the site), and every later reader sees the dropped
+    tensor; nothing may be folded into its producer after this point."""
+    assert self.program and not x.is_input, "a dropout site must follow the op that writes its tensor"
+    self._consume(x)
+    self.dropout_sites.append((x, float(rate), self.program[-1]))
+    return x
+
   def max_pool_3x3_s2(self, x):
     self._consume(x)
     out = Sym(self, (x.width + 1) // 2, x.channels)
@@ -180,8 +191,19 @@ class Graph:
     return out
 
   # ---- lowering to the C ABI -----------------------------------------------------------------------
-  def build_net(self, logits, num_classes, none_index, precision, max_batch, options=None):
-    """Emits the traced program into a fresh pcls_net and finalizes it.  Returns the handle (c_void_p)."""
+  def build_net(self, logits, num_classes, none_index, precision, max_batch, options=None, dropout_rate=None):
+    """Emits the traced program into a fresh pcls_net and finalizes it.  Returns the handle (c_void_p).
+    ``dropout_rate``: None (the deterministic net), one rate for every site of ``dropout_sites``, or a sequence with one
+    rate per site; each site becomes a pcls_net_dropout op (site = its index) right after the op it follows."""
+    rates = None
+    if dropout_rate is not None:
+      rates = [float(r) for r in dropout_rate] if hasattr(dropout_rate, "__len__") else \
+          [float(dropout_rate)] * len(self.dropout_sites)
+      if len(rates) != len(self.dropout_sites):
+        raise ValueError("%d dropout rates for %d sites" % (len(rates), len(self.dropout_sites)))
+      lost = [k for k, (_, _, after) in enumerate(self.dropout_sites) if not any(op is after for op in self.program)]
+      if lost:
+        raise ValueError("dropout sites %s follow ops that are no longer in the program" % lost)
     lib = _lib.load()
     handle = ctypes.c_void_p()
     _lib.check(lib.pcls_net_create(ctypes.byref(handle), self.H, self.W, precision, max_batch), "pcls_net_create")
@@ -215,7 +237,14 @@ class Graph:
         s.tid = None
       self.input.tid = 0
       logits.logits = True
-      for op in self.program:
+
+      def emit_dropouts(prev):
+        for k, (sym, _, after) in enumerate(self.dropout_sites):
+          if rates is not None and after is prev:
+            _lib.check(lib.pcls_net_dropout(handle, tid(sym), k, rates[k]), "pcls_net_dropout(site %d)" % k)
+
+      for i, op in enumerate(self.program):
+        emit_dropouts(self.program[i - 1] if i else None)
         if op["op"] == "conv":
           d = _lib.ConvDesc()
           d.kind, d.kh, d.kw, d.stride_w, d.cin, d.cout = op["kind"], op["kh"], op["kw"], op["stride_w"], op["cin"], op["cout"]
@@ -249,6 +278,7 @@ class Graph:
           d.h_ex_mean, d.h_ex_var = fptr(n + "/excitation_bn/moving_mean"), fptr(n + "/excitation_bn/moving_variance")
           d.in_tensor, d.out_tensor = tid(op["src"]), tid(op["dst"])
           _lib.check(lib.pcls_net_cam(handle, ctypes.byref(d)), "pcls_net_cam(%s)" % n)
+      emit_dropouts(self.program[-1])
       _lib.check(lib.pcls_net_finalize(handle, tid(logits), num_classes, none_index), "pcls_net_finalize")
     except Exception:
       lib.pcls_net_destroy(handle)
@@ -314,14 +344,15 @@ class LeakyReLU(Layer):
 
 
 class Dropout(Layer):
-  """Identity at inference (training=False everywhere on this path)."""
+  """Identity in the default net (training=False everywhere on this path).  Each call records an MC dropout site
+  (``Graph.dropout`` / ``Graph.dropout_sites``), used only by the stochastic net of ``mc_dropout``."""
 
   def __init__(self, rate):
     super().__init__(None)
     self.rate = rate
 
   def __call__(self, x, training=False):
-    return x
+    return x.graph.dropout(x, self.rate)
 
 
 def relu(x):

@@ -21,7 +21,8 @@ from . import _lib
 from .calibration import TemperatureNLL, check_tta, confidence as pixel_confidence, raw_mask
 from .device import ptr, samples_to_device, stream_handle, to_device
 from .laserscan import SphericalProjector
-from .metrics import MeanIoU, PanopticQuality, Reliability
+from .mc_dropout import check_exclusive, forward_mc
+from .metrics import MeanIoU, PanopticQuality, Reliability, UncertaintyAUROC
 from .sharding import Communicator, shard_range
 from .tta import forward_tta
 from .utils.util import confusion_matrix_to_iou_recall_precision
@@ -90,7 +91,8 @@ class ScanSegmenter:
     self.projector = SphericalProjector(mc.ZENITH_LEVEL, mc.AZIMUTH_LEVEL, fov_up, fov_down, label_lut=label_lut)
 
   def segment_device(self, points, offsets, labels=None, want_probabilities=False, out=None, want_image=False,
-                     want_logits=False, want_point_labels=False, knn=None, instances=None, tta=None, confidence=None):
+                     want_logits=False, want_point_labels=False, knn=None, instances=None, tta=None, confidence=None,
+                     mc_dropout=None):
     """points [total,4] float32 CUDA (x,y,z,remission), offsets [B+1] int64 CUDA -> dict(predictions, proj_idx,
     probabilities?, logits?, image?, point_labels?) - keys and activations stay on the device.
 
@@ -114,7 +116,19 @@ class ScanSegmenter:
     confidence: a temperature T - also ``confidence`` [B,H,W] float32 (max softmax(logits / T) per pixel, 0 at empty
     pixels; pcls_confidence) and ``point_confidence`` [total] float32 (the probability at T that the point's own pixel
     gives the point's label; pcls_point_confidence); needs want_point_labels.  At T = 1 the forward's probabilities are
-    used as they are; with a TTA only T = 1 is available (the merged probabilities)."""
+    used as they are; with a TTA only T = 1 is available (the merged probabilities).
+
+    mc_dropout: an ``mc_dropout.MCDropout`` - the range image is materialised and goes through
+    ``mc_dropout.forward_mc``; the MC mean's predictions (and probabilities) take the place of the forward's, and the
+    result also holds ``confidence`` / ``entropy`` / ``mutual_information`` [B,H,W] and, with want_point_labels,
+    ``point_mi`` / ``point_entropy`` [total] float32 (the value of the point's own pixel, 0 for a dropped point) and
+    ``point_confidence``: as with ``confidence=1``, the MC mean's probability of the label the point got.  Refused with a
+    TTA, logits or a temperature other than 1."""
+    if mc_dropout is not None and (tta is not None or want_logits or (confidence is not None and
+                                                                      float(confidence) != 1.0)):
+      raise ValueError("MC dropout cannot be combined with test-time augmentation, logits or a softmax temperature")
+    if mc_dropout is not None and want_point_labels:
+      confidence = 1.0     # one definition of the point confidence under MC: the mean's probability of the point's label
     if instances is not None and not want_point_labels:
       raise ValueError("instances need the point labels: segment with want_point_labels=True")
     if tta is not None and want_logits:
@@ -129,9 +143,14 @@ class ScanSegmenter:
     fwd_probs = want_probabilities or (confidence is not None and not tempered)
     fwd_logits = want_logits or tempered
     B = int(offsets.numel()) - 1
-    if tta is not None or want_image or labels is not None or B > self._staged_capacity(B):
+    if mc_dropout is not None or tta is not None or want_image or labels is not None or B > self._staged_capacity(B):
       proj = self.projector.project(points, offsets, labels=labels, empty_fill=0.0, want_point_outputs=want_point_labels)
-      if tta is not None:
+      if mc_dropout is not None:
+        res = forward_mc(self.model, proj["image"], mc_dropout, want_probabilities=fwd_probs, out=out)
+        if want_point_labels:
+          for k, name in (("mutual_information", "point_mi"), ("entropy", "point_entropy")):
+            res[name] = self._point_gather(res[k], offsets, proj["proj_x"], proj["proj_y"])
+      elif tta is not None:
         res = forward_tta(self.model, proj["image"], tta, want_probabilities=fwd_probs, out=out)
       else:
         res = self.model.forward_device(proj["image"], None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD,
@@ -199,6 +218,18 @@ class ScanSegmenter:
     if not want_logits:
       res.pop("logits", None)
     return dict(confidence=c["confidence"], point_confidence=pc)
+
+  def _point_gather(self, values, offsets, px, py):
+    """values [B,H,W] float32 -> [total] float32: each point's own pixel's value, 0 for a dropped point (the exact
+    gather of pcls_point_confidence with one class and every label 0)."""
+    B, H, W = values.shape
+    total = int(px.numel())
+    zero = torch.zeros(total, dtype=torch.int32, device=values.device)
+    out = torch.empty(total, dtype=torch.float32, device=values.device)
+    _lib.check(_lib.load().pcls_point_confidence(ptr(values.contiguous()), ptr(offsets), B, H, W, total, ptr(px),
+                                                 ptr(py), ptr(zero), 1, ptr(out), stream_handle()),
+               "pcls_point_confidence")
+    return out
 
   def _point_labels(self, preds, keys, offsets, px, py, ur, knn):
     B, H, W = preds.shape
@@ -283,18 +314,25 @@ class Evaluator:
   calibration's temperature (pcls_confidence) is binned against the head's predictions and the fixed-up labels, the
   "None" class ignored (``metrics.Reliability``), and the NLL at T = 1, at the temperature and, with ``fit``, on the
   grid is accumulated (``calibration.TemperatureNLL``).  With a TTA the merged probabilities give the confidence, so
-  only T = 1 without a fit is available."""
+  only T = 1 without a fit is available.
+  ``mc_dropout``: an ``mc_dropout.MCDropout`` - the predictions are the MC mean's (``mc_dropout.forward_mc``), and the
+  AUROC of H and of MI for detecting misclassified pixels (``metrics.UncertaintyAUROC``) and the reliability of the
+  mean's confidence are accumulated, the "None" class ignored; refused with a TTA or a temperature / fit."""
 
-  def __init__(self, model, comm=None, tta=None, calibration=None):
+  def __init__(self, model, comm=None, tta=None, calibration=None, mc_dropout=None):
     check_tta(calibration, tta)
+    check_exclusive(mc_dropout, tta, calibration)
     self.model, self.mc = model, model.mc
-    self.comm, self.tta, self.calibration = comm, tta, calibration
+    self.comm, self.tta, self.calibration, self.mc_dropout = comm, tta, calibration, mc_dropout
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self._none = self.mc.CLASSES.index("None")
-    self.reliability = self.nll = None
+    self.reliability = self.nll = self.auroc = self.mc_reliability = None
+    if mc_dropout is not None:
+      self.auroc = UncertaintyAUROC(self.mc.NUM_CLASS)
+      self.mc_reliability = Reliability(calibration.n_bins if calibration is not None else 15, self.mc.NUM_CLASS)
     if calibration is not None:
       self.reliability = Reliability(calibration.n_bins, self.mc.NUM_CLASS)
-      if tta is None:
+      if tta is None and mc_dropout is None:
         self.nll = TemperatureNLL(calibration, self.mc.NUM_CLASS, self._none)
     self._mean = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_MEAN).reshape(-1))
     self._std = (ctypes.c_double * 5)(*np.asarray(self.mc.INPUT_STD).reshape(-1))
@@ -308,7 +346,9 @@ class Evaluator:
     if C != 6:
       raise ValueError("evaluation samples need 6 channels (x,y,z,intensity,depth,label)")
     cal = self.calibration is not None
-    if self.tta is not None:
+    if self.mc_dropout is not None:
+      res = forward_mc(self.model, x, self.mc_dropout)
+    elif self.tta is not None:
       res = forward_tta(self.model, x, self.tta, want_probabilities=cal)
     else:
       res = self.model.forward_device(x, None, mean=self.mc.INPUT_MEAN, std=self.mc.INPUT_STD, want_probabilities=False,
@@ -317,7 +357,13 @@ class Evaluator:
     _lib.check(_lib.load().pcls_input_stage(ptr(x), 6, B * H * W, self._mean, self._std, self._none, None, None,
                                             ptr(label), None, 0, None, stream_handle()), "pcls_input_stage")
     self.miou_tracker.update_state(label, res["predictions"])
-    if cal:
+    if self.mc_dropout is not None:
+      # masked pixels carry the "None" label after the fix-up, so they are not binned
+      self.auroc.update_state(res["entropy"], res["mutual_information"], res["predictions"], label, self._none)
+      self.mc_reliability.update_state(res["confidence"], res["predictions"], label, self._none)
+      if cal:
+        self.reliability.update_state(res["confidence"], res["predictions"], label, self._none)
+    elif cal:
       nc = self.mc.NUM_CLASS
       if self.tta is not None:
         conf = pixel_confidence(nc, probs=res["probabilities"])["confidence"]
@@ -337,8 +383,21 @@ class Evaluator:
     rep = dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
                miou=float(self.miou_tracker.result()))
     if self.calibration is not None:
-      rep["calibration"] = _calibration_report(self.calibration, self.reliability, self.nll, self.comm)
+      nll = self.nll if self.mc_dropout is None else None
+      rep["calibration"] = _calibration_report(self.calibration, self.reliability, nll, self.comm)
+    if self.mc_dropout is not None:
+      rep["mc_dropout"] = _mc_report(self.mc_dropout, self.mc, self.auroc, self.mc_reliability, self.comm)
     return rep
+
+
+def _mc_report(mcd, mc, auroc, reliability, comm):
+  """dict(passes, rate, seed, uncertainty: ``UncertaintyAUROC.result()``, reliability: ``Reliability.result()`` of the
+  MC mean's confidence), the sums all-reduced first when ``comm`` is given."""
+  if comm is not None:
+    auroc.allreduce(comm)
+    reliability.allreduce(comm)
+  return dict(passes=mcd.passes, rate=mcd.rate_for(mc), seed=mcd.seed, uncertainty=auroc.result(),
+              reliability=reliability.result())
 
 
 def _calibration_report(calibration, reliability, nll, comm):
@@ -361,17 +420,24 @@ class ScanEvaluator:
   points in a predicted or ground-truth thing segment come back to the host.  ``tta``: a ``tta.TTA`` for the forward
   (``ScanSegmenter.segment_device(tta=)``).  ``calibration``: a ``calibration.Calibration`` without ``fit`` (the
   temperature is fitted on pixels, with ``Evaluator``) - each point's confidence at its temperature
-  (``segment_device(confidence=)``) is binned against its label and the ground truth, the "None" class ignored."""
+  (``segment_device(confidence=)``) is binned against its label and the ground truth, the "None" class ignored.
+  ``mc_dropout``: an ``mc_dropout.MCDropout`` - the point labels come from the MC mean, and the AUROC of each point's H
+  and MI (its own pixel's) for detecting misclassified points and the reliability of the MC confidence are accumulated."""
 
   def __init__(self, model, fov_up=3.0, fov_down=-25.0, label_lut=None, knn=None, instances=None, tta=None,
-               calibration=None):
+               calibration=None, mc_dropout=None):
     check_tta(calibration, tta)
+    check_exclusive(mc_dropout, tta, calibration)
     if calibration is not None and calibration.fit:
       raise ValueError("the temperature is fitted on pixels (Evaluator); point-wise evaluation takes a fixed temperature")
     self.seg = ScanSegmenter(model, fov_up, fov_down)
     self.mc, self.knn, self.instances, self.tta = model.mc, knn, instances, tta
-    self.calibration = calibration
+    self.calibration, self.mc_dropout = calibration, mc_dropout
     self.reliability = Reliability(calibration.n_bins, self.mc.NUM_CLASS) if calibration is not None else None
+    self.auroc = self.mc_reliability = None
+    if mc_dropout is not None:
+      self.auroc = UncertaintyAUROC(self.mc.NUM_CLASS)
+      self.mc_reliability = Reliability(calibration.n_bins if calibration is not None else 15, self.mc.NUM_CLASS)
     self.miou_tracker = MeanIoU(num_classes=self.mc.NUM_CLASS, name="MeanIoU")
     self.pq = None
     if instances is not None:
@@ -387,7 +453,8 @@ class ScanEvaluator:
       raise ValueError("point-wise evaluation needs the label files")
     res = self.seg.segment_device(batch["points"], batch["offsets"], want_point_labels=True, knn=self.knn,
                                   instances=self.instances, tta=self.tta,
-                                  confidence=self.calibration.temperature if self.calibration is not None else None)
+                                  confidence=self.calibration.temperature if self.calibration is not None else None,
+                                  mc_dropout=self.mc_dropout)
     n = int(batch["points"].shape[0])
     gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
     lut = self.lut
@@ -396,6 +463,10 @@ class ScanEvaluator:
     self.miou_tracker.update_state(gt, res["point_labels"])
     if self.reliability is not None:
       self.reliability.update_state(res["point_confidence"], res["point_labels"], gt, self.mc.CLASSES.index("None"))
+    if self.auroc is not None:
+      none = self.mc.CLASSES.index("None")
+      self.auroc.update_state(res["point_entropy"], res["point_mi"], res["point_labels"], gt, none)
+      self.mc_reliability.update_state(res["point_confidence"], res["point_labels"], gt, none)
     res["gt"] = gt
     if self.pq is not None:
       self._update_pq(batch, gt, res)
@@ -430,6 +501,8 @@ class ScanEvaluator:
       rep["panoptic"] = self.pq.result()
     if self.calibration is not None:
       rep["calibration"] = _calibration_report(self.calibration, self.reliability, None, None)
+    if self.mc_dropout is not None:
+      rep["mc_dropout"] = _mc_report(self.mc_dropout, self.mc, self.auroc, self.mc_reliability, None)
     return rep
 
 

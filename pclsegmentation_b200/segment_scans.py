@@ -38,6 +38,7 @@ def segment_scans(arg):
   from .calibration import Calibration
   from .pipeline import KNN, Clustering, ScanEvaluator
   from .tta import from_args
+  from .mc_dropout import from_args as mc_from_args
   from .utils.args_loader import load_model_config
 
   config, model = load_model_config(arg.model or "squeezesegv2", arg.config)
@@ -60,10 +61,11 @@ def segment_scans(arg):
     clustering = Clustering(tau=arg.cluster_tau, rows=arg.cluster_rows, cols=arg.cluster_cols,
                             min_points=arg.min_points, wrap=not arg.no_wrap)
   tta = from_args(arg.tta, arg.tta_shifts)
+  mcd = mc_from_args(arg)
   cal = Calibration(temperature=arg.temperature, n_bins=arg.bins) if arg.confidence else None
   try:
     ev = ScanEvaluator(model, fov_up, fov_down, label_lut=lut, knn=None if arg.no_knn else KNN(), instances=clustering,
-                       tta=tta, calibration=cal)
+                       tta=tta, calibration=cal, mc_dropout=mcd)
   except ValueError as e:
     raise SystemExit(str(e))
   os.makedirs(arg.output_dir, exist_ok=True)
@@ -75,11 +77,16 @@ def segment_scans(arg):
       res = ev.update(data)
     else:
       res = ev.seg.segment_device(data["points"], data["offsets"], want_point_labels=True, knn=ev.knn,
-                                  instances=clustering, tta=tta, confidence=cal.temperature if cal else None)
+                                  instances=clustering, tta=tta, confidence=cal.temperature if cal else None,
+                                  mc_dropout=mcd)
     if cal is not None:
       pc = res["point_confidence"].cpu().numpy()
       for f, c in zip(files, np.split(pc, np.cumsum(data["sizes"])[:-1])):
         c.astype(np.float32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".conf"))
+    if mcd is not None:
+      mi = res["point_mi"].cpu().numpy()
+      for f, u in zip(files, np.split(mi, np.cumsum(data["sizes"])[:-1])):
+        u.astype(np.float32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".unc"))
     if clustering is not None:
       for f, words in zip(files, ev.seg.label_words(res, data["sizes"], inv)):
         words.tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
@@ -109,6 +116,9 @@ def segment_scans(arg):
   if cal is not None:
     from .eval import print_reliability
     print_reliability(rep["calibration"]["reliability"], cal.temperature, "points")
+  if mcd is not None:
+    from .eval import print_mc_report
+    print_mc_report(rep["mc_dropout"], "points")
   return rep
 
 
@@ -144,6 +154,8 @@ def main(argv=None):
   ap.add_argument("--learning_map", default=None, help="yaml with `learning_map` / `learning_map_inv` (semantic-kitti.yaml)")
   from .tta import add_tta_flags
   add_tta_flags(ap)
+  from .mc_dropout import add_mc_flags
+  add_mc_flags(ap)
   from .calibration import add_temperature_flag
   ap.add_argument("--confidence", action="store_true", help="also write <name>.conf: float32 confidence per point")
   add_temperature_flag(ap)
