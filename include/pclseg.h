@@ -277,6 +277,47 @@ int pcls_mc_finalize(const float* acc_probs, const double* acc_entropy, const ui
                      int none_index, int n_passes, float* out_probs, int32_t* out_preds, float* out_conf,
                      float* out_entropy, float* out_mi, pcls_stream stream);
 
+/* Semantic map fusion (no reference call site: the reference labels each scan on its own).  The point labels of a
+ * pose-registered sequence are voted into a voxel hash map, and points are relabelled from it.  The rules are this
+ * project's; parity with SuMa++ or any other mapping code is not claimed.
+ * Voxel of a point: point i of scan b has float32 (x, y, z) from points [total,4] f32 (16-byte aligned) and offsets [B+1]
+ *   i64.  poses [B,12] f64 is a DEVICE array: the 3x4 row-major lidar-to-world transform (R | t) of each scan.  World
+ *   coordinate w_k = ((R_k0*x + R_k1*y) + R_k2*z) + t_k in float64, every product and sum rounded on its own (no FMA
+ *   contraction).  v_k = floor(w_k / s), s = voxel_size, IEEE float64 division.  A point has no voxel when a w_k is not
+ *   finite or a v_k is outside [-2^20, 2^20).  Key = ((vx + 2^20) << 42) | ((vy + 2^20) << 21) | (vz + 2^20) as u64,
+ *   always below 2^63, so ~0 marks an empty slot.
+ * Table: table_keys [capacity] u64 and table_counts [capacity, NC] u32, capacity a power of two, 1 <= NC <= 32.  An empty
+ *   table is all keys ~0 and all counts 0.  state [2] i64: state[0] = occupied slots; state[1] = points (or, when
+ *   growing, keys) that found no free slot within `capacity` probes - 0 while the load stays at most 1/2, there so that
+ *   misuse cannot hang a kernel.  The hash and the probe sequence are internal; slot placement depends on the order of
+ *   atomics, but the set of (key, counts), the query results and an export sorted by key are the same bits on every run.
+ * pcls_semantic_map_vote: a point votes when it has a voxel, 0 <= labels[i] < NC, labels[i] != ignore_class, and
+ *   r2 >= min_range^2 and (max_range <= 0 or r2 <= max_range^2), r2 = (x*x + y*y) + z*z in float64 with separate roundings
+ *   in the sensor frame, the squared limits computed in float64.  A vote inserts the key if it is new (state[0] += 1) and
+ *   then adds 1 to table_counts[slot, label].
+ * pcls_semantic_map_grow: initialises the new table itself (keys ~0, counts 0) and reinserts every occupied slot of the
+ *   old one with its row of counts; state[0] is unchanged.  new_capacity must be a power of two at least twice state[0]
+ *   (the host may pass a bound it holds instead of reading state[0]).  The tables must not overlap.
+ * pcls_semantic_map_query: per point, out_labels[i] = labels_in[i] when it is a class of keep_mask (bit c = class c);
+ *   otherwise, when its voxel is in the table with at least min_votes (>= 1) votes in total, the argmax of the voxel's
+ *   counts (ties to the lowest class); otherwise labels_in[i].  The range limits do not apply: a far point, or one the
+ *   projection dropped, takes the label of a voxel that nearer scans established.
+ * Every call checks before any launch: 1 <= NC <= 32; ignore_class -1 or in [0, NC); no keep_mask bit at or above NC;
+ * voxel_size finite and > 0; finite range limits with 0 <= min_range and (max_range <= 0 or max_range >= min_range);
+ * capacities powers of two; total < 2^31; the pointers the call needs.  Otherwise PCLS_ERR_INVALID.  Pose entries live
+ * on the device and are not checked here (semantic_map.SemanticMap checks them).  total == 0 is a no-op. */
+int pcls_semantic_map_vote(const float* points, const int64_t* offsets, int B, int64_t total, const double* poses,
+                           double voxel_size, double min_range, double max_range, const int32_t* labels,
+                           int num_classes, int ignore_class, uint64_t* table_keys, uint32_t* table_counts,
+                           int64_t capacity, int64_t* state, pcls_stream stream);
+int pcls_semantic_map_grow(const uint64_t* old_keys, const uint32_t* old_counts, int64_t old_capacity, int num_classes,
+                           uint64_t* new_keys, uint32_t* new_counts, int64_t new_capacity, int64_t* state,
+                           pcls_stream stream);
+int pcls_semantic_map_query(const float* points, const int64_t* offsets, int B, int64_t total, const double* poses,
+                            double voxel_size, const int32_t* labels_in, int num_classes, uint32_t keep_mask,
+                            int min_votes, const uint64_t* table_keys, const uint32_t* table_counts, int64_t capacity,
+                            int32_t* out_labels, pcls_stream stream);
+
 /* Per-point ground truth for point-wise evaluation: out[i] = lut[labels[i] & 0xFFFF], ids >= lut_len -> 0,
  * lut NULL -> the raw semantic id (the same rule pcls_project_resolve applies per pixel). */
 int pcls_map_labels(const uint32_t* labels, int64_t n, const int32_t* label_lut, int lut_len, int32_t* out,

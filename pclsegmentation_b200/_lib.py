@@ -66,6 +66,12 @@ SIGNATURES = {
   "pcls_mc_accumulate": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
   "pcls_mc_finalize": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                c_void_p, c_void_p, c_void_p]),
+  "pcls_semantic_map_vote": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_double, c_double, c_double,
+                                     c_void_p, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+  "pcls_semantic_map_grow": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p,
+                                     c_void_p]),
+  "pcls_semantic_map_query": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_double, c_void_p, c_int, c_uint32,
+                                      c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
   "pcls_map_labels":(c_int, [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_void_p]),
   "pcls_dataset_stats": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_double), c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -20,7 +20,7 @@ OBJ_DIR = os.path.join(HERE, "build%s" % _SUFFIX)
 # conv_tc.cu holds ~160 kernel instantiations: it is compiled once per part (-DPCLS_TC_PART=k, see the file) in parallel
 TC_PARTS = 13
 SOURCES = [("conv_tc.cu", k) for k in range(TC_PARTS)] + ["conv_head.cu", "net.cu", "nn_kernels.cu", "pool_conv.cu", "squeeze_upconv.cu",
-           "projection.cu", "point_labels.cu", "point_instances.cu", "tta.cu", "calibration.cu", "mc_dropout.cu", "dataset_stats.cu", "head.cu", "input_stage.cu", "confusion.cu", "validation.cu", "error.cu"]
+           "projection.cu", "point_labels.cu", "point_instances.cu", "tta.cu", "calibration.cu", "mc_dropout.cu", "semantic_map.cu", "dataset_stats.cu", "head.cu", "input_stage.cu", "confusion.cu", "validation.cu", "error.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr"]
 # development builds, e.g. PCLS_NVCC_FLAGS="-DPCLS_TC_DEBUG=1" (wait-cycle counters)

@@ -455,11 +455,7 @@ class ScanEvaluator:
                                   instances=self.instances, tta=self.tta,
                                   confidence=self.calibration.temperature if self.calibration is not None else None,
                                   mc_dropout=self.mc_dropout)
-    n = int(batch["points"].shape[0])
-    gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
-    lut = self.lut
-    _lib.check(_lib.load().pcls_map_labels(ptr(batch["labels"]), n, ptr(lut), int(lut.numel()) if lut is not None else 0,
-                                           ptr(gt), stream_handle()), "pcls_map_labels")
+    gt = self.ground_truth(batch)
     self.miou_tracker.update_state(gt, res["point_labels"])
     if self.reliability is not None:
       self.reliability.update_state(res["point_confidence"], res["point_labels"], gt, self.mc.CLASSES.index("None"))
@@ -471,6 +467,15 @@ class ScanEvaluator:
     if self.pq is not None:
       self._update_pq(batch, gt, res)
     return res
+
+  def ground_truth(self, batch):
+    """The per-point ground truth of a batch with labels: [total] int32 CUDA, ``label_lut[word & 0xFFFF]``."""
+    n = int(batch["points"].shape[0])
+    gt = torch.empty(n, dtype=torch.int32, device=batch["points"].device)
+    lut = self.lut
+    _lib.check(_lib.load().pcls_map_labels(ptr(batch["labels"]), n, ptr(lut), int(lut.numel()) if lut is not None else 0,
+                                           ptr(gt), stream_handle()), "pcls_map_labels")
+    return gt
 
   def _update_pq(self, batch, gt, res):
     """Feeds ``self.pq`` scan by scan with the points that can be in a segment: a predicted instance, or a ground-truth

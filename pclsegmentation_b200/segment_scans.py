@@ -24,6 +24,14 @@ With --confidence each point's confidence is written next to its ``.label`` file
 per point): the probability at --temperature T that the point's own pixel gives the point's label (0 for a point the
 projection dropped).  With --labels the point-wise reliability report (ECE, MCE, per-bin table) follows the other
 reports.
+
+With --map (KITTI layout; needs --poses and --calib) the sequence is fused through a semantic map
+(``semantic_map.SemanticMap``): pass 1 segments every batch as above and votes its point labels into a voxel map
+registered by the sequence's poses ("None" casts no vote); pass 2 relabels every scan from the map and writes the fused
+labels.  The pose of a scan is the integer stem of its file name (``000123.bin`` -> line 123 of poses.txt), so a glob
+over part of a sequence works.  --map_keep things (default) keeps the thing classes of ``pipeline.Clustering`` as the
+network labelled them, since moving objects would otherwise take the static votes under them.  --map_out writes the
+map (``SemanticMap.save``).  With --labels a second report, headed FUSED (semantic map), follows the per-scan one.
 """
 import argparse
 import glob
@@ -34,9 +42,21 @@ import numpy as np
 
 def segment_scans(arg):
   from .dataset_convert import KITTI, ScanBatchLoader, learning_map_lut
+  if arg.map:
+    if arg.instances or arg.confidence or arg.mc_dropout is not None:
+      raise SystemExit("--map cannot be combined with --instances, --confidence or --mc_dropout")
+    if arg.format != KITTI:
+      raise SystemExit("--map reads SemanticKITTI poses.txt / calib.txt; there is no nuScenes poses reader (the Python "
+                       "API, semantic_map.SemanticMap, takes any poses)")
+    if not arg.poses or not arg.calib:
+      raise SystemExit("--map needs --poses (poses.txt) and --calib (calib.txt) of the sequence")
+    if arg.map_min_votes < 1:
+      raise SystemExit("--map_min_votes must be >= 1")
   from .inference import load_model_weights
   from .calibration import Calibration
+  from .metrics import MeanIoU
   from .pipeline import KNN, Clustering, ScanEvaluator
+  from .semantic_map import SemanticMap, kitti_lidar_poses, scan_pose_index
   from .tta import from_args
   from .mc_dropout import from_args as mc_from_args
   from .utils.args_loader import load_model_config
@@ -68,6 +88,23 @@ def segment_scans(arg):
                        tta=tta, calibration=cal, mc_dropout=mcd)
   except ValueError as e:
     raise SystemExit(str(e))
+  smap = None
+  if arg.map:
+    poses = kitti_lidar_poses(arg.poses, arg.calib)
+    try:
+      pose_of = np.array([scan_pose_index(f, len(poses)) for f in scans], np.int64)
+      smap = SemanticMap(config.NUM_CLASS, voxel_size=arg.voxel_size, min_range=arg.map_min_range,
+                         max_range=arg.map_max_range, ignore_class=config.CLASSES.index("None"))
+    except ValueError as e:
+      raise SystemExit(str(e))
+    keep = Clustering().thing_ids(config) if arg.map_keep == "things" else ()
+    scan_labels = []      # pass 1's point labels per batch, uint8 on the host
+
+  def write_labels(files, labs):
+    for f, lab in zip(files, labs):
+      words = inv[lab] if inv is not None else lab.astype(np.uint32)
+      words.astype(np.uint32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
+
   os.makedirs(arg.output_dir, exist_ok=True)
   loader = ScanBatchLoader(arg.format)
   for i in range(0, len(scans), arg.batch):
@@ -91,20 +128,30 @@ def segment_scans(arg):
       for f, words in zip(files, ev.seg.label_words(res, data["sizes"], inv)):
         words.tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
       continue
-    for f, lab in zip(files, ev.seg.point_labels(res, data["sizes"])):
-      words = inv[lab] if inv is not None else lab.astype(np.uint32)
-      words.astype(np.uint32).tofile(os.path.join(arg.output_dir, os.path.splitext(os.path.basename(f))[0] + ".label"))
+    if smap is not None:
+      smap.vote(data["points"], data["offsets"], poses[pose_of[i:i + arg.batch]], res["point_labels"])
+      scan_labels.append(res["point_labels"].cpu().numpy().astype(np.uint8))
+      continue
+    write_labels(files, ev.seg.point_labels(res, data["sizes"]))
+  fused_iou = None
+  if smap is not None:
+    fused_iou = MeanIoU(num_classes=config.NUM_CLASS, name="MeanIoU") if labels is not None else None
+    for j, i in enumerate(range(0, len(scans), arg.batch)):
+      files = scans[i:i + arg.batch]
+      data = loader.load(files, labels[i:i + arg.batch] if labels is not None else None)
+      fused = smap.relabel(data["points"], data["offsets"], poses[pose_of[i:i + arg.batch]], scan_labels[j],
+                           keep_classes=keep, min_votes=arg.map_min_votes)
+      if fused_iou is not None:
+        fused_iou.update_state(ev.ground_truth(data), fused)
+      write_labels(files, np.split(fused.cpu().numpy(), np.cumsum(data["sizes"])[:-1]))
+    print("semantic map: %d voxels of %g m" % (smap.num_voxels, smap.voxel_size))
+    if arg.map_out:
+      smap.save(arg.map_out)
   print("labelled %d scans -> %s" % (len(scans), arg.output_dir))
   if labels is None:
     return None
   rep = ev.finish()
-  for c, cls in enumerate(config.CLASSES):
-    print(cls.upper())
-    print("IoU:       " + str(rep["iou"][c]))
-    print("Recall:    " + str(rep["recall"][c]))
-    print("Precision: " + str(rep["precision"][c]))
-    print("")
-  print("MIoU: {} ".format(rep["miou"]))
+  print_iou(rep, config.CLASSES)
   if rep["dropped"]:
     print("WARNING: %d of %d points have a ground-truth id that is not a class id (0 .. %d) and are not scored%s"
           % (rep["dropped"], int(rep["confusion_matrix"].sum()) + rep["dropped"], config.NUM_CLASS - 1,
@@ -119,7 +166,26 @@ def segment_scans(arg):
   if mcd is not None:
     from .eval import print_mc_report
     print_mc_report(rep["mc_dropout"], "points")
+  if fused_iou is not None:
+    from .utils.util import confusion_matrix_to_iou_recall_precision
+    cm = fused_iou.total_cm
+    iou, recall, precision = confusion_matrix_to_iou_recall_precision(cm)
+    rep["fused"] = dict(confusion_matrix=cm.cpu().numpy(), iou=iou, recall=recall, precision=precision,
+                        miou=float(fused_iou.result()))
+    print("FUSED (semantic map)")
+    print_iou(rep["fused"], config.CLASSES)
   return rep
+
+
+def print_iou(rep, class_names):
+  """The per-class IoU / recall / precision lines and the mIoU of a report, in eval.py's format."""
+  for c, cls in enumerate(class_names):
+    print(cls.upper())
+    print("IoU:       " + str(rep["iou"][c]))
+    print("Recall:    " + str(rep["recall"][c]))
+    print("Precision: " + str(rep["precision"][c]))
+    print("")
+  print("MIoU: {} ".format(rep["miou"]))
 
 
 def print_panoptic(pan, class_names):
@@ -160,6 +226,16 @@ def main(argv=None):
   ap.add_argument("--confidence", action="store_true", help="also write <name>.conf: float32 confidence per point")
   add_temperature_flag(ap)
   ap.add_argument("--bins", type=int, default=15, help="reliability bins of the --labels report (1..64)")
+  ap.add_argument("--map", action="store_true", help="fuse the sequence's labels through a semantic voxel map (2 passes)")
+  ap.add_argument("--poses", default=None, help="--map: the sequence's poses.txt (camera frame, 3x4 per line)")
+  ap.add_argument("--calib", default=None, help="--map: the sequence's calib.txt (its Tr: line)")
+  ap.add_argument("--voxel_size", type=float, default=0.2, help="--map: voxel edge in metres")
+  ap.add_argument("--map_min_range", type=float, default=0.0, help="--map: nearer points cast no vote (metres)")
+  ap.add_argument("--map_max_range", type=float, default=50.0, help="--map: farther points cast no vote; <= 0: no limit")
+  ap.add_argument("--map_min_votes", type=int, default=1, help="--map: a voxel with fewer votes relabels nothing")
+  ap.add_argument("--map_keep", choices=["things", "none"], default="things",
+                  help="--map: points labelled as these classes keep their label")
+  ap.add_argument("--map_out", default=None, help="--map: also write the map (.npz: voxels, counts, labels)")
   return segment_scans(ap.parse_args(argv))
 
 
