@@ -363,7 +363,12 @@ int pcls_head(const float* logits, const uint8_t* mask, int64_t n_pixels, int nu
  *   lidar   [n_pixels,6] f32 or NULL; mask [n_pixels] u8 or NULL; label [n_pixels] i32 or NULL
  *   h_cls_loss_weight  host doubles [num_classes] (mc.CLS_LOSS_WEIGHT) or NULL; weight [n_pixels] f32 or NULL: 0 where
  *           the label is not one of 0 .. num_classes-1 (the reference starts from np.zeros), num_classes <= 32
- *           (label and weight require channels == 6). */
+ *           (label and weight require channels == 6).
+ * Label rule at valid pixels (the label channel is a float): like parse_sample, the weight compares the FLOAT label with
+ * each class id, so weight = CLS_LOSS_WEIGHT[l] only if the label equals the integer l exactly (-0.0 counts as 0);
+ * fractional (2.5), NaN, +-inf, negative and >= num_classes labels get 0.  label = the float truncated toward zero,
+ * saturated to the int32 range, NaN -> 0 (numpy's astype leaves NaN / out-of-range to the host; integer labels in range
+ * are the same either way). */
 int pcls_input_stage(const float* sample, int channels, int64_t n_pixels, const double* h_mean5,
                      const double* h_std5, int none_index, float* lidar, uint8_t* mask,
                      int32_t* label, const double* h_cls_loss_weight, int num_classes, float* weight,

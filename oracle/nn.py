@@ -242,9 +242,25 @@ def input_stage(sample_hw6, mean, std, none_index):
     lidar = (lidar - np.asarray(mean, np.float64).reshape(1, 1, 5)) / np.asarray(std, np.float64).reshape(1, 1, 5)
     lidar[~mask] = 0.0
     lidar = np.append(lidar, np.expand_dims(mask, -1), axis=2)
-    label = sample[:, :, 5].copy()
-    label[~mask] = none_index
-    return lidar.astype(np.float32), mask, label.astype(np.int32)
+    return lidar.astype(np.float32), mask, label_to_int32(fixed_label(sample, none_index))
+
+
+def fixed_label(sample_hw6, none_index):
+    """data_loader.py:176-178: the float32 label channel with label[~mask] = none_index.  parse_sample keeps it float
+    until its return, so the class-weight map (class_weight_map) compares this float label, not the int32 cast."""
+    sample = np.asarray(sample_hw6).astype(np.float32)
+    label = sample[..., 5].copy()
+    label[~(sample[..., 4] > 0)] = none_index
+    return label
+
+
+def label_to_int32(label):
+    """label.astype('int32') (data_loader.py:187) with the rule pclseg.h states for pcls_input_stage: truncation toward
+    zero, saturated to the int32 range, NaN -> 0.  numpy's own cast leaves NaN and out-of-range values to the host
+    (INT_MIN on x86); on integer-valued labels in range both agree."""
+    x = np.asarray(label, dtype=np.float64)
+    x = np.where(np.isnan(x), 0.0, np.clip(np.trunc(x), -2.0 ** 31, 2.0 ** 31 - 1))
+    return x.astype(np.int32)
 
 
 def to_torch_params(params: dict, dtype=torch.float32):
@@ -273,7 +289,8 @@ def forward(arch: str, params: dict, lidar_bhw6, mask_bhw, none_index: int,
 
 def class_weight_map(label_hw, cls_loss_weight):
     """data_loader.py:181-185: weight = zeros(label.shape); weight[label == l] = CLS_LOSS_WEIGHT[l] for l in
-    range(NUM_CLASS); returned as float32 like parse_sample (:187)."""
+    range(NUM_CLASS); returned as float32 like parse_sample (:187).  label_hw is the FLOAT label of fixed_label, as
+    parse_sample compares it: 2.5, NaN and +-inf match no class (weight 0), -0.0 matches class 0."""
     weight = np.zeros(np.asarray(label_hw).shape)
     for l in range(len(cls_loss_weight)):
         weight[np.asarray(label_hw) == l] = cls_loss_weight[int(l)]

@@ -74,7 +74,7 @@ def test_input_stage_matches_oracle():
     assert np.array_equal(lidar[sl].cpu().numpy().reshape(64, 512, 6), l_ref)     # bit-exact (float64 normalise)
     assert np.array_equal(mask[sl].cpu().numpy().reshape(64, 512).astype(bool), m_ref)
     assert np.array_equal(label[sl].cpu().numpy().reshape(64, 512), lab_ref)
-    w_ref = O.class_weight_map(lab_ref, cls_w)                                     # data_loader.py:181-185
+    w_ref = O.class_weight_map(O.fixed_label(raw[b], 0), cls_w)                   # data_loader.py:181-185 (float label)
     assert np.array_equal(weight[sl].cpu().numpy().reshape(64, 512), w_ref)
   assert (weight.cpu().numpy().reshape(2, 64, 512)[0, :4, :8] == 0).all()
   # the DataLoader.parse_sample facade returns the same four arrays
